@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""Benchmark of the B200 Attention U-Net hot path (contract: see the task statement).
+"""Benchmark of the B200 Attention U-Net hot path.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference|reference-gpu]
+                  [--dump-outputs DIR]
 
 A "step" is one training step (forward, DiceBCELoss, backward, gradient all-reduce for N > 1,
 clip 1.0, AdamW) of AttentionUNet(1, 2, bilinear, 64) on a synthetic batch of B 1x512x512
@@ -29,6 +30,13 @@ launch under torchrun.  Rank 0 prints ONE JSON line.
               baseline/_ref (installed by baseline/install_reference.py; kind "reference"), its model, loss
               and the loop of scripts/train.py:132-143, same workload (batch 4 per step, never shrunk).
               Without baseline/_ref the oracle port runs instead (kind "port").
+
+  --dump-outputs DIR    --impl ours only: after the K timed steps, write what the last of them handed its
+              caller as float32 DIR/<name>.npy (32 MB in all; see dump_outputs).  The inputs and the initial
+              weights are seeded, so two builds run with the same arguments can be compared output for output.
+              bench_outputs/ is git-ignored for such dumps.
+
+The benchmark writes nothing into the tree it runs from (which may be read-only).
 """
 from __future__ import annotations
 
@@ -39,6 +47,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True   # no __pycache__ in the tree (children run this file and set it too)
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "unet-segment-pytorch_b200")
@@ -198,17 +208,10 @@ def run_reference_arm(args):
             return loss.item()
 
     warm = max(0, min(args.warmup, 1))
-    t0 = time.perf_counter()
     for _ in range(warm):
         step()
-    est = (time.perf_counter() - t0) / max(warm, 1)
-    # the workload is never shrunk; if K steps of it cannot finish in ~5 minutes on this host, fewer steps
-    # are timed and the line says so
-    timed = max(1, args.steps)
-    if warm and est * timed > 300.0:
-        timed = max(2, int(300.0 / est))
     times = []
-    for _ in range(timed):
+    for _ in range(args.steps):   # the workload is never shrunk, and exactly --steps steps are timed
         t0 = time.perf_counter()
         step()
         times.append(time.perf_counter() - t0)
@@ -388,6 +391,33 @@ def replica_check(model, trainer, dev, world):
                     "per-rank fp64 checksums gathered: replicas must be bit-identical"}
 
 
+DUMP_SAMPLE = 1 << 22   # elements of the sampled arrays: 16 MiB each in float32
+
+
+def dump_outputs(out_dir, model, loss):
+    """What one training step hands its caller, as float32 .npy files under out_dir:
+      loss           the loss the step returned (0-dim)
+      bn_running     every BatchNorm running_mean / running_var the step updated, concatenated in model order
+      params_sample  the updated parameters, all of them flattened in model.parameters() order, at DUMP_SAMPLE
+                     positions drawn once from a generator seeded with 0 (in ascending order)
+      grads_sample   the gradients of the step at the same positions
+    AttentionUNet(1,2,True,64) has 17.6 M parameters (70 MB per full array), hence the fixed sample."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    params = list(model.parameters())
+    flat_p = torch.cat([p.detach().reshape(-1) for p in params])
+    flat_g = torch.cat([p.grad.detach().reshape(-1) for p in params])   # views into the trainer's buckets
+    idx = torch.randperm(flat_p.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE]
+    idx = idx.sort().values.to(flat_p.device)
+    running = [b.detach().reshape(-1) for n, b in model.named_buffers() if n.endswith(("running_mean", "running_var"))]
+    arrays = {"loss": loss.detach().reshape(()), "bn_running": torch.cat(running),
+              "params_sample": flat_p[idx], "grads_sample": flat_g[idx]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.float().cpu().numpy())
+
+
 def run_ours(args):
     for p in (PKG, ROOT):
         if p not in sys.path:
@@ -459,8 +489,15 @@ def run_ours(args):
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms = timed(lambda: trainer.step(x_dev, t_dev), args.steps)
+    last_loss = [None]
+
+    def timed_step():
+        last_loss[0] = trainer.step(x_dev, t_dev)
+
+    ms = timed(timed_step, args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, last_loss[0])   # before any later step changes the model
     dp_check_after_graph = replica_check(model, trainer, dev, world) if world > 1 else None
 
     def profile_eager(tr, x, t, steps):
@@ -723,7 +760,8 @@ def other_configs(dev, timed, profile_eager, make_trainer, roofline_peak, Infere
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps (--impl reference-gpu times its own fixed counts per precision mode)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--batch", type=int, default=4, help="images per GPU per step")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "reference-gpu"])
@@ -731,7 +769,15 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip sustained / other configs / library baseline")
     ap.add_argument("--sustain-seconds", type=float, default=3.0)
     ap.add_argument("--no-graph", action="store_true", help="issue every kernel eagerly (no CUDA-graph replay)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl ours only: write the loss, BatchNorm statistics and a fixed sample of the parameters "
+                         "and gradients after the last timed step as float32 DIR/<name>.npy (bench_outputs/ is "
+                         "git-ignored)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours only")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
         run_reference_arm(args)

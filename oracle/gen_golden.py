@@ -1,7 +1,7 @@
-"""Generate tests/golden/*.pt from the UNMODIFIED reference (run in the build container, where
-/root/reference is mounted; the reference cannot travel to the GPU box).
+"""Generate tests/golden/*.pt from the UNMODIFIED reference, a checkout of which $UNET_REFERENCE names.
 
-    python oracle/gen_golden.py
+    UNET_REFERENCE=<checkout> python oracle/gen_golden.py
+    python oracle/gen_golden.py --oracle-only     # tests/golden/random_cases.pt from the oracle alone
 
 Each fixture holds the seeds / configuration that regenerate the inputs (synthetic weights and
 batches come from oracle.unet_oracle's deterministic generators) and the reference's outputs:
@@ -16,7 +16,7 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("UNET_REFERENCE", "/root/reference")
+REF = os.environ.get("UNET_REFERENCE", "")
 sys.path.insert(0, ROOT)
 from oracle import unet_oracle as O  # noqa: E402
 
@@ -26,6 +26,9 @@ OUT = os.path.join(ROOT, "tests", "golden")
 def import_reference():
     """Import the reference's modules from files (its package is also called `unet`)."""
     import importlib.util
+
+    if not (REF and os.path.isdir(os.path.join(REF, "unet"))):
+        raise RuntimeError("set UNET_REFERENCE to a checkout of the unmodified reference")
 
     def load(name, rel):
         spec = importlib.util.spec_from_file_location(name, os.path.join(REF, rel))
@@ -211,11 +214,82 @@ def io_case():
             "mask": torch.from_numpy(np.stack(masks)), "positives": torch.tensor(counts)}
 
 
+# Seeded cases of tests/test_oracle_vs_reference.py that the model cases above do not cover: 3 input
+# channels and 3 classes (DiceBCE over more than one foreground class), odd non-square sizes under bilinear
+# up-sampling (the F.pad path), and a confusion matrix with an out-of-range label and no ignore_index.
+RANDOM_CASES = [(True, True, (33, 47)), (False, True, (40, 24)), (True, False, (32, 32))]
+
+
+def random_case_inputs(attention, bilinear, hw):
+    cfg = dict(n_channels=3, n_classes=3, bilinear=bilinear, base_features=8, attention=attention)
+    sd = O.synthetic_state_dict(9, **cfg)
+    g = torch.Generator().manual_seed(1)
+    x = torch.randn(2, 3, *hw, generator=g)
+    t = torch.randint(0, 3, (2, *hw), generator=g)
+    return cfg, sd, x, t
+
+
+def metrics_loop_inputs():
+    g = torch.Generator().manual_seed(2)
+    z = torch.randn(1, 4, 16, 16, generator=g)
+    t = torch.randint(0, 5, (1, 16, 16), generator=g)  # label 4 is out of range -> skipped
+    return z, t
+
+
+def reference_train_step(net, loss_mod, attention, bilinear, hw):
+    """(loss, train-mode logits, gradients by key) of the reference's modules on one random case."""
+    cfg, sd, x, t = random_case_inputs(attention, bilinear, hw)
+    mk = {k: cfg[k] for k in ("n_channels", "n_classes", "bilinear", "base_features")}
+    model = (net.AttentionUNet if attention else net.UNet)(**mk)
+    model.load_state_dict(sd, strict=True)
+    model.train()
+    out = model(x)
+    loss = loss_mod.DiceBCELoss()(out, t)
+    loss.backward()
+    return loss, out.detach(), {k: p.grad for k, p in model.named_parameters()}
+
+
+def random_cases(ref=None):
+    """Outputs on RANDOM_CASES -> tests/golden/random_cases.pt: train-mode logits, loss, per-parameter gradient
+    norm / largest magnitude / first 8 values, and the confusion matrix of metrics_loop_inputs().  With
+    ref = import_reference() they are the reference's and the oracle must reproduce them on the spot (the
+    tolerances of tests/test_oracle_vs_reference.py); without, they are the oracle's.  "source" says which."""
+    out = {"source": "oracle" if ref is None else "reference", "models": []}
+    for attention, bilinear, hw in RANDOM_CASES:
+        cfg, sd, x, t = random_case_inputs(attention, bilinear, hw)
+        o_loss, o_logits, o_grads = O.train_grads(x, t, O.clone_state(sd), attention=attention, bilinear=bilinear)
+        loss, logits, grads = o_loss, o_logits, o_grads
+        if ref is not None:
+            loss, logits, grads = reference_train_step(ref[1], ref[2], attention, bilinear, hw)
+            assert torch.allclose(o_logits, logits, rtol=1e-3, atol=1e-4)
+            assert abs(o_loss.item() - loss.item()) < 1e-5
+            for k, g in grads.items():
+                assert torch.allclose(o_grads[k], g, rtol=5e-3, atol=1e-5 * g.abs().max().item() + 1e-9), k
+        out["models"].append({"attention": attention, "bilinear": bilinear, "hw": hw, "logits": logits.detach().clone(),
+                              "loss": loss.item(),
+                              "grads": {k: {"norm": g.norm().item(), "absmax": g.abs().max().item(),
+                                            "head": g.flatten()[:8].clone()} for k, g in grads.items()}})
+    z, t = metrics_loop_inputs()
+    cm = O.confusion_matrix(z, t, 4)
+    if ref is not None:
+        m = ref[3].SegmentationMetrics(4)
+        m.update(z, t)
+        assert np.array_equal(m.get_confusion_matrix(), cm)
+        cm = m.get_confusion_matrix()
+    out["confusion"] = torch.from_numpy(np.asarray(cm))
+    return out
+
+
 def main():
     torch.manual_seed(0)
     torch.set_num_threads(8)
-    layers, net, loss_mod, metrics_mod = import_reference()
     os.makedirs(OUT, exist_ok=True)
+    if "--oracle-only" in sys.argv:
+        torch.save(random_cases(), os.path.join(OUT, "random_cases.pt"))
+        print("random_cases.pt", os.path.getsize(os.path.join(OUT, "random_cases.pt")), "bytes")
+        return
+    layers, net, loss_mod, metrics_mod = import_reference()
+    torch.save(random_cases((layers, net, loss_mod, metrics_mod)), os.path.join(OUT, "random_cases.pt"))
     cases = {
         "attn_bf32": model_case(net, loss_mod, True, 32, 1, 2, 32),
         "unet_bf16": model_case(net, loss_mod, False, 16, 2, 2, 48),

@@ -9,7 +9,7 @@ leg may import it, and only as the checker or the timed CPU baseline.
 Parity status: **pinned** — the reference itself ships no tests or golden vectors
 (SURVEY.md §4), so the oracle is pinned against outputs of the unmodified
 reference run in the build container (``oracle/gen_golden.py`` →
-``tests/golden/*.pt``) and, whenever ``/root/reference`` is present, directly
+``tests/golden/*.pt``) and, whenever ``$UNET_REFERENCE`` names a checkout, directly
 against the imported reference (``tests/test_oracle_vs_reference.py``).
 
 Every function cites the reference lines it restates (paths relative to the

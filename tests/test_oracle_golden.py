@@ -1,6 +1,9 @@
-"""CPU: the oracle against the golden vectors produced by the UNMODIFIED reference
-(oracle/gen_golden.py, run in the build container).  fp32 on both sides: tolerances are
-summation-order noise."""
+"""CPU: the oracle against the golden vectors of oracle/gen_golden.py.  fp32 on both sides: tolerances are
+summation-order noise.  models / loss / metrics / io / init_fingerprint hold outputs of the UNMODIFIED
+reference.  random_cases.pt names its origin in "source": the committed copy is the output of the oracle as
+it stood when it last matched the reference on these seeded cases (tests/test_oracle_vs_reference.py), so a
+later change of the oracle on those paths is caught without a reference checkout; with one,
+`UNET_REFERENCE=<checkout> python oracle/gen_golden.py` rewrites it from the reference."""
 import os
 
 import numpy as np
@@ -8,6 +11,7 @@ import pytest
 import torch
 
 from oracle import unet_oracle as O
+from oracle.gen_golden import RANDOM_CASES, metrics_loop_inputs, random_case_inputs
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -56,6 +60,29 @@ def test_metrics_cases():
             assert abs(res[k] - v) < 1e-12
         assert torch.allclose(O.iou_per_class(g["z"], g["t"], g["c"]), g["iou"])
         assert torch.allclose(O.dice_per_class(g["z"], g["t"], g["c"]), g["dice"])
+
+
+@pytest.mark.parametrize("i", range(len(RANDOM_CASES)), ids=[f"{a}-{b}-{h[0]}x{h[1]}" for a, b, h in RANDOM_CASES])
+def test_random_cases(i):
+    """3 channels / 3 classes, odd sizes through the F.pad path (oracle/gen_golden.py:random_cases); the
+    tolerances of tests/test_oracle_vs_reference.py."""
+    g = _load("random_cases.pt")["models"][i]
+    assert (g["attention"], g["bilinear"], tuple(g["hw"])) == RANDOM_CASES[i]
+    _, sd, x, t = random_case_inputs(*RANDOM_CASES[i])
+    loss, logits, grads = O.train_grads(x, t, sd, attention=g["attention"], bilinear=g["bilinear"])
+    assert torch.allclose(logits, g["logits"], rtol=1e-3, atol=1e-4)
+    assert abs(loss.item() - g["loss"]) < 1e-5
+    assert grads.keys() == g["grads"].keys()
+    for k, ref in g["grads"].items():
+        assert abs(grads[k].norm().item() - ref["norm"]) <= 5e-3 * ref["norm"] + 1e-9, k
+        assert torch.allclose(grads[k].flatten()[:8], ref["head"], rtol=5e-3, atol=1e-5 * ref["absmax"] + 1e-9), k
+
+
+def test_confusion_out_of_range_label():
+    """A label >= num_classes without ignore_index is skipped, as the reference's loop does."""
+    z, t = metrics_loop_inputs()
+    assert (t == 4).any()
+    assert np.array_equal(O.confusion_matrix(z, t, 4), _load("random_cases.pt")["confusion"].numpy())
 
 
 def test_state_dict_shapes_match_appendix_a():

@@ -4,7 +4,9 @@ The reference's scripts import, next to the hot-path modules this package rebuil
 modules it does not (scripts/train.py:28-35, scripts/predict.py:29-30).  With a reference checkout
 attached (``unet.overlay``) those imports must resolve — hot path here, the rest in the reference's
 own files — and the objects must work together the way train.py uses them.  Runs wherever a
-checkout is available: /root/reference in the build container, the staged baseline/_ref otherwise.
+checkout is available and skips elsewhere: $UNET_REFERENCE (the variable build() and the oracle tests
+read too), else the copy build() stages under baseline/_ref.  $UNET_REFERENCE_ROOT is what the package
+itself attaches at run time; the cases set or clear it themselves.
 Each case runs in a fresh interpreter (import state is the thing under test).
 """
 import os
@@ -19,8 +21,8 @@ PKG = os.path.join(ROOT, "unet-segment-pytorch_b200")
 
 
 def _checkout():
-    for c in ("/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if os.path.isfile(os.path.join(c, "unet", "__init__.py")) and os.path.isfile(os.path.join(c, "scripts", "train.py")):
+    for c in (os.environ.get("UNET_REFERENCE", ""), os.path.join(ROOT, "baseline", "_ref")):
+        if c and os.path.isfile(os.path.join(c, "unet", "__init__.py")) and os.path.isfile(os.path.join(c, "scripts", "train.py")):
             return c
     return None
 
