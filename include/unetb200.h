@@ -219,6 +219,12 @@ int ub2_conv_in_fwd(const float* x, const float* w, void* y, int ld_y, double* p
                     int Cin, int H, int W, int Cout, void* stream);
 int ub2_conv_in_wgrad(const float* x, const void* dy, int ld_dy, double* partials, int rows, float* grad,
                       int N, int Cin, int H, int W, int Cout, void* stream);
+/* Its data gradient (autograd of layers.py:32 when the network input requires grad): dy NHWC bf16 with
+ * channel stride ld_dy (multiple of 8, >= Cout), w the fp32 OIHW parameter, dx fp32 NCHW (N,Cin,H,W), each
+ * element written once in a fixed summation order (no atomics).  Same Cin / Cout limits as ub2_conv_in_fwd;
+ * for Cin > 1, W % 4 != 0 or pointers not 16-byte aligned also Cin * 9 * Cout <= 12288. */
+int ub2_conv_in_dgrad(const void* dy, int ld_dy, const float* w, float* dx, int N, int Cin, int H, int W, int Cout,
+                      void* stream);
 /* OutConv (layers.py:120-123): 1x1 conv with bias to fp32 NCHW logits, and its backward. */
 int ub2_outc_rows(int N, int H, int W, int C);
 int ub2_outc_fwd(const void* a, int ld_a, const float* w, const float* bias, float* logits, int N, int H,
@@ -349,6 +355,9 @@ int ub2_f32_outc_rows(int N, int H, int W);
 int ub2_f32_outc_bwd(const float* dlogits, const float* a, const float* w, float* da, double* partials, int rows, float* dw, float* db, int N, int H, int W, int C, int K, void* stream);
 int ub2_f32_conv_in_raw(const float* x, const float* w, float* out, int N, int Cin, int H, int W, int Cout, void* stream);
 int ub2_f32_conv_in_wgrad(const float* x, const float* dy, double* partials, int rows, float* grad, int N, int Cin, int H, int W, int Cout, void* stream);
+/* ub2_conv_in_dgrad with fp32 dy (ld_dy multiple of 4, >= Cout): Cout % 4 == 0, any Cin >= 1, with the same
+ * shared-memory limit. */
+int ub2_f32_conv_in_dgrad(const float* dy, int ld_dy, const float* w, float* dx, int N, int Cin, int H, int W, int Cout, void* stream);
 int ub2_f32_split_bf16(const float* x, void* hi, void* lo, long long n, void* stream);
 int ub2_f32_split_tf32(const float* x0, int ld0, int C0, const float* x1, int ld1, int C1, float* out, long long pixels, void* stream);
 int ub2_f32_pack_weight3(const float* w, float* out, int Cout, int Cin, int taps, int dgrad, void* stream);

@@ -3,7 +3,10 @@
 //  * conv_in: the first 3x3 convolution (inc.double_conv.0, layers.py:32) with Cin = n_channels
 //    (1 for CT slices): K = 9*Cin, arithmetic intensity ~9 flop/B -> a direct fp32 CUDA-core
 //    convolution reading the fp32 NCHW input and writing NHWC bf16 + BatchNorm statistics,
-//    and its weight gradient (no data gradient: the input needs none).
+//    its weight gradient, and its data gradient dx (fp32 NCHW, the network input's layout) for
+//    callers that differentiate with respect to the input (saliency maps, adversarial steps, a
+//    U-Net behind another trainable stage).  The data-gradient kernels are templated over the dy
+//    element type and serve both precisions (bf16 dy here, fp32 dy of the fp32 / TF32 mode).
 //  * outc: OutConv's 1x1 conv with bias (layers.py:120) C -> n_classes, writing fp32 NCHW
 //    logits, and its backward (data gradient NHWC bf16, weight / bias gradients).
 #include "launch.cuh"
@@ -329,6 +332,186 @@ __global__ void conv_in_wgrad_finalize_kernel(const double* __restrict__ partial
   grad[co * Cin * 9 + r] += static_cast<float>(s[0]);
 }
 
+// dx[n][ci][h][w] = sum_{r,s} sum_co dy[n][h-r+1][w-s+1][co] * W[co][ci][r][s]  (dy outside the image = 0)
+//
+// dy is read as 16-byte vectors of V channels (8 bf16 or 4 fp32).  Every element offset is 64-bit: N*H*W*ld_dy
+// passes 2^31 at batch 128 of 512^2 x 64.  No pointer to a dy row outside the image is formed.
+template <typename T>
+struct DyVec;
+template <>
+struct DyVec<__nv_bfloat16> {
+  static constexpr int V = 8;
+  __device__ __forceinline__ static void load(const __nv_bfloat16* p, float (&v)[V]) {
+    const F8 f = unpack8(__ldg(reinterpret_cast<const uint4*>(p)));
+#pragma unroll
+    for (int k = 0; k < V; ++k) v[k] = f.v[k];
+  }
+  __device__ __forceinline__ static float one(const __nv_bfloat16* p) {
+    return __uint_as_float(static_cast<unsigned>(__ldg(reinterpret_cast<const unsigned short*>(p))) << 16);
+  }
+};
+template <>
+struct DyVec<float> {
+  static constexpr int V = 4;
+  __device__ __forceinline__ static void load(const float* p, float (&v)[V]) {
+    const float4 f = __ldg(reinterpret_cast<const float4*>(p));
+    v[0] = f.x; v[1] = f.y; v[2] = f.z; v[3] = f.w;
+  }
+  __device__ __forceinline__ static float one(const float* p) { return __ldg(p); }
+};
+
+// Cin == 1, W % 4 == 0, dy / dx 16-byte aligned (as conv_in_fwd4): a thread owns 4 consecutive pixels x one
+// V-channel group of dy with its 9*V weights in registers, reads the 3x6 window of dy vectors around them and
+// does 36*V FMAs into 4 per-pixel partial sums.  The Cout/V group partials of a pixel group are then folded in a
+// fixed order — by xor shuffles when Cout/V is a power of two <= 32 (the group threads are adjacent lanes of one
+// warp), else through shared memory — and written with one float4 store.  The block walks trips of
+// (image row, chunk of lanes*4 columns) together, so the fold's barriers are reached by every thread.
+template <typename T, bool SHFL>
+__global__ void __launch_bounds__(kHeadThreads, 2)
+conv_in_dgrad4_kernel(const T* __restrict__ dy, int ld_dy, const float* __restrict__ w, float* __restrict__ dx,
+                      int N, int H, int W, int Cout) {
+  pdl_trigger();
+  pdl_wait();
+  constexpr int V = DyVec<T>::V;
+  extern __shared__ float4 s_part[];  // [lanes][cgs] (SHFL == false)
+  const int cgs = Cout / V;
+  const int lanes = blockDim.x / cgs;
+  const int lane = threadIdx.x / cgs, cg = threadIdx.x % cgs;
+  const int span = lanes * 4;
+  const int chunks = (W + span - 1) / span;
+  const int trips = N * H * chunks;  // host: < 2^31
+  float wr[9][V];
+#pragma unroll
+  for (int t = 0; t < 9; ++t)
+#pragma unroll
+    for (int k = 0; k < V; ++k) wr[t][k] = __ldg(w + static_cast<size_t>(cg * V + k) * 9 + t);
+  for (int trip = blockIdx.x; trip < trips; trip += gridDim.x) {
+    const int row = trip / chunks;  // n*H + h
+    const int wq = (trip - row * chunks) * span + lane * 4;
+    const int hq = row % H;
+    const bool active = wq < W;
+    float acc[4] = {0.f, 0.f, 0.f, 0.f};
+    if (active) {
+#pragma unroll
+      for (int r = 0; r < 3; ++r) {  // dy row hq + r - 1 meets the weight row 2 - r
+        const int hh = hq + r - 1;
+        if (hh < 0 || hh >= H) continue;
+        const T* p = dy + (static_cast<size_t>(row + r - 1) * W + wq) * ld_dy + cg * V;
+        float v[6][V];
+        if (wq > 0) DyVec<T>::load(p - ld_dy, v[0]);
+        else {
+#pragma unroll
+          for (int k = 0; k < V; ++k) v[0][k] = 0.f;
+        }
+#pragma unroll
+        for (int c = 1; c < 5; ++c) DyVec<T>::load(p + static_cast<size_t>(c - 1) * ld_dy, v[c]);
+        if (wq + 4 < W) DyVec<T>::load(p + static_cast<size_t>(4) * ld_dy, v[5]);
+        else {
+#pragma unroll
+          for (int k = 0; k < V; ++k) v[5][k] = 0.f;
+        }
+        // pixel wq+px takes dy column wq+px+j-1 (window column px+j) with weight column 2-j
+#pragma unroll
+        for (int px = 0; px < 4; ++px)
+#pragma unroll
+          for (int j = 0; j < 3; ++j)
+#pragma unroll
+            for (int k = 0; k < V; ++k) acc[px] = fmaf(v[px + j][k], wr[(2 - r) * 3 + (2 - j)][k], acc[px]);
+      }
+    }
+    if (SHFL) {
+#pragma unroll
+      for (int px = 0; px < 4; ++px)
+        for (int o = cgs >> 1; o > 0; o >>= 1) acc[px] += __shfl_xor_sync(0xffffffffu, acc[px], o);
+    } else {
+      s_part[threadIdx.x] = make_float4(acc[0], acc[1], acc[2], acc[3]);
+      __syncthreads();
+      if (cg == 0 && active) {
+        for (int c = 1; c < cgs; ++c) {
+          const float4 q = s_part[lane * cgs + c];
+          acc[0] += q.x; acc[1] += q.y; acc[2] += q.z; acc[3] += q.w;
+        }
+      }
+      __syncthreads();
+    }
+    if (cg == 0 && active)
+      *reinterpret_cast<float4*>(dx + static_cast<size_t>(row) * W + wq) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+  }
+}
+
+// Every other Cin, W or alignment: one dx element per thread (NCHW order, coalesced stores), weights in shared
+// memory as [ci][tap][co], every tap bounds-checked, dy read one element at a time.
+template <typename T>
+__global__ void __launch_bounds__(kHeadThreads)
+conv_in_dgrad_kernel(const T* __restrict__ dy, int ld_dy, const float* __restrict__ w, float* __restrict__ dx,
+                     int N, int Cin, int H, int W, int Cout) {
+  pdl_trigger();
+  pdl_wait();
+  extern __shared__ float s_w[];  // [Cin*9][Cout]
+  for (int i = threadIdx.x; i < Cout * Cin * 9; i += blockDim.x) {
+    const int co = i / (Cin * 9), r = i % (Cin * 9);
+    s_w[r * Cout + co] = w[i];
+  }
+  __syncthreads();
+  const long long total = static_cast<long long>(N) * Cin * H * W;
+  for (long long e = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; e < total;
+       e += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const int wq = static_cast<int>(e % W);
+    const long long q = e / W;
+    const int hq = static_cast<int>(q % H);
+    const long long nc = q / H;
+    const int ci = static_cast<int>(nc % Cin);
+    const long long n = nc / Cin;
+    float acc = 0.f;
+    for (int r = 0; r < 3; ++r) {
+      const int hh = hq - r + 1;
+      if (hh < 0 || hh >= H) continue;
+      for (int s = 0; s < 3; ++s) {
+        const int ww = wq - s + 1;
+        if (ww < 0 || ww >= W) continue;
+        const T* p = dy + ((n * H + hh) * W + ww) * static_cast<long long>(ld_dy);
+        const float* wp = s_w + (ci * 9 + r * 3 + s) * Cout;
+#pragma unroll 4
+        for (int co = 0; co < Cout; ++co) acc = fmaf(DyVec<T>::one(p + co), wp[co], acc);
+      }
+    }
+    dx[e] = acc;
+  }
+}
+
+// Variant choice and launch, after the entry point's argument checks.  The general variant's weights must fit the
+// 48 KB of dynamic shared memory that needs no opt-in (Cin * 9 * Cout <= 12288).
+template <typename T>
+static int conv_in_dgrad_launch(const T* dy, int ld_dy, const float* w, float* dx, int N, int Cin, int H, int W,
+                                int Cout, void* stream) {
+  constexpr int V = DyVec<T>::V;
+  const int cgs = Cout / V;
+  const long long rows = static_cast<long long>(N) * H;
+  const bool aligned16 = ((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(dx)) & 15) == 0;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (Cin == 1 && W % 4 == 0 && aligned16 && cgs <= kHeadThreads) {
+    const int lanes = kHeadThreads / cgs;
+    const int block = lanes * cgs;
+    const long long span = lanes * 4;
+    const long long trips = rows * ((W + span - 1) / span);
+    if (trips < (1LL << 31) && W + span < (1LL << 31)) {  // the kernel's 32-bit trip and column indices
+      const bool shfl = (cgs & (cgs - 1)) == 0 && cgs <= 32;
+      const size_t smem = shfl ? 0 : static_cast<size_t>(block) * sizeof(float4);
+      const int grid = stream_grid(trips, 1, num_sms(), 4);
+      if (shfl)
+        launch(conv_in_dgrad4_kernel<T, true>, grid, block, smem, s, dy, ld_dy, w, dx, N, H, W, Cout);
+      else
+        launch(conv_in_dgrad4_kernel<T, false>, grid, block, smem, s, dy, ld_dy, w, dx, N, H, W, Cout);
+      return static_cast<int>(cudaGetLastError());
+    }
+  }
+  const size_t smem = static_cast<size_t>(Cin) * 9 * Cout * sizeof(float);
+  if (smem > 48 * 1024) return UB2_ERR_SHAPE;
+  const int grid = stream_grid(static_cast<long long>(N) * Cin * H * W, kHeadThreads, num_sms(), 8);
+  launch(conv_in_dgrad_kernel<T>, grid, kHeadThreads, smem, s, dy, ld_dy, w, dx, N, Cin, H, W, Cout);
+  return static_cast<int>(cudaGetLastError());
+}
+
 // ------------------------------------------------------------------------------ outc
 struct HeadGeom {
   int C, cgs, tpp, slots, K;
@@ -607,6 +790,26 @@ int ub2_conv_in_wgrad(const float* x, const void* dy, int ld_dy, double* partial
   const int total = Cout * Cin * 9;
   launch(conv_in_wgrad_finalize_kernel, (total + 31) / 32, dim3(32, 32), 0, s, partials, grid, Cin, Cout, grad);
   return static_cast<int>(cudaGetLastError());
+}
+
+int ub2_conv_in_dgrad(const void* dy, int ld_dy, const float* w, float* dx, int N, int Cin, int H, int W, int Cout,
+                      void* stream) {
+  if (dy == nullptr || w == nullptr || dx == nullptr || N <= 0 || H <= 0 || W <= 0) return UB2_ERR_SHAPE;
+  if (Cout <= 0 || Cout % 8 != 0 || Cout / 8 > kHeadThreads || Cin < 1 || Cin > kMaxCin || ld_dy < Cout) return UB2_ERR_SHAPE;
+  if (static_cast<double>(N) * H * W * Cin >= 2.0e9) return UB2_ERR_SHAPE;  // the forward's limit
+  if (ld_dy % 8 != 0 || (reinterpret_cast<uintptr_t>(dy) & 1) || (reinterpret_cast<uintptr_t>(w) & 3) ||
+      (reinterpret_cast<uintptr_t>(dx) & 3))
+    return UB2_ERR_ALIGN;
+  return conv_in_dgrad_launch(static_cast<const __nv_bfloat16*>(dy), ld_dy, w, dx, N, Cin, H, W, Cout, stream);
+}
+
+int ub2_f32_conv_in_dgrad(const float* dy, int ld_dy, const float* w, float* dx, int N, int Cin, int H, int W, int Cout,
+                          void* stream) {
+  if (dy == nullptr || w == nullptr || dx == nullptr || N <= 0 || H <= 0 || W <= 0) return UB2_ERR_SHAPE;
+  if (Cout <= 0 || Cout % 4 != 0 || Cin < 1 || ld_dy < Cout) return UB2_ERR_SHAPE;
+  if (ld_dy % 4 != 0 || ((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(w) | reinterpret_cast<uintptr_t>(dx)) & 3))
+    return UB2_ERR_ALIGN;
+  return conv_in_dgrad_launch(dy, ld_dy, w, dx, N, Cin, H, W, Cout, stream);
 }
 
 int ub2_outc_rows(int N, int H, int W, int C) {

@@ -389,8 +389,7 @@ class ConvInBnReluF32(torch.autograd.Function):
     def forward(ctx, x, weight, gamma, beta, bn):
         if not x.is_cuda:
             raise RuntimeError("unet-b200 modules run on CUDA tensors only (no CPU fallback)")
-        if ctx.needs_input_grad[0]:
-            raise NotImplementedError("gradient w.r.t. the network input is not implemented")
+        x_dtype = x.dtype
         x = x.contiguous().float()
         n, cin, h, w = x.shape
         cout = weight.shape[0]
@@ -398,15 +397,17 @@ class ConvInBnReluF32(torch.autograd.Function):
         _C.call("ub2_f32_conv_in_raw", ptr(x), ptr(weight.contiguous()), ptr(y), n, cin, h, w, cout, stream())
         scale, shift, mean, invstd, batch = _bn_stage(y, bn)
         a = affine_act(y, scale, shift, relu=True)
-        ctx.save_for_backward(x, y, scale, shift, mean, invstd, gamma)
-        ctx.meta = (weight.shape, batch)
+        ctx.save_for_backward(x, y, scale, shift, mean, invstd, gamma,
+                              weight if ctx.needs_input_grad[0] else None)
+        ctx.meta = (weight.shape, batch, x_dtype)
         return nchw(a)
 
     @staticmethod
     def backward(ctx, dA):
-        x, y, scale, shift, mean, invstd, gamma = ctx.saved_tensors
-        wshape, batch = ctx.meta
+        x, y, scale, shift, mean, invstd, gamma, weight = ctx.saved_tensors
+        wshape, batch, x_dtype = ctx.meta
         dy, dgamma, dbeta = act_backward(nhwc_view(dA), None, None, y, scale, shift, mean, invstd, gamma, batch)
+        dx = K.conv_in_dgrad(dy, weight.contiguous(), wshape[1]).to(x_dtype) if ctx.needs_input_grad[0] else None
         gw = None
         if ctx.needs_input_grad[1]:
             n, cin, h, w = x.shape
@@ -415,7 +416,7 @@ class ConvInBnReluF32(torch.autograd.Function):
             part = torch.empty((rows, cin, 9, cout), device=x.device, dtype=F64)
             gw = torch.zeros(wshape, device=x.device, dtype=F32)
             _C.call("ub2_f32_conv_in_wgrad", ptr(x), ptr(dy), ptr(part), rows, ptr(gw), n, cin, h, w, cout, stream())
-        return None, gw, dgamma, dbeta, None
+        return dx, gw, dgamma, dbeta, None
 
 
 class MaxPoolF32(torch.autograd.Function):

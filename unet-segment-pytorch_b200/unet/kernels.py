@@ -430,6 +430,22 @@ def conv_in_wgrad(x, dy, cout, grad=None):
     return grad
 
 
+def conv_in_dgrad(dy, w, cin):
+    """First conv's data gradient: dy (N,H,W,Cout) NHWC bf16 or fp32 (the fp32 / TF32 mode), w (Cout,Cin,3,3)
+    fp32 -> dx (N,Cin,H,W) fp32 NCHW."""
+    assert w.dtype == F32 and w.is_contiguous()
+    if dy.dtype == F32:
+        n, h, wd, cout, ld = _nhwc32(dy)
+        name = "ub2_f32_conv_in_dgrad"
+    else:
+        n, h, wd, cout, ld = _nhwc(dy)
+        name = "ub2_conv_in_dgrad"
+    dx = torch.empty((n, cin, h, wd), device=dy.device, dtype=F32)
+    _C.call(name, ptr(dy), ld, ptr(w), ptr(dx), n, cin, h, wd, cout, stream(),
+            work=(2.0 * n * h * wd * cout * 9 * cin, _nbytes(dy, dx)))
+    return dx
+
+
 def outc_fwd(a, w, bias):
     n, h, wd, c, ld = _nhwc(a)
     k = w.shape[0]

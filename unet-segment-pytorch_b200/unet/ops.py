@@ -234,8 +234,7 @@ class ConvInBnRelu(torch.autograd.Function):
     def forward(ctx, x, weight, gamma, beta, bn):
         if not x.is_cuda:
             raise RuntimeError("unet-b200 modules run on CUDA tensors only (no CPU fallback)")
-        if ctx.needs_input_grad[0]:
-            raise NotImplementedError("gradient w.r.t. the network input is not implemented")
+        x_dtype = x.dtype
         x = x.contiguous().float()
         n, _, h, w = x.shape
         batch = _use_batch_stats(bn)
@@ -246,21 +245,23 @@ class ConvInBnRelu(torch.autograd.Function):
             scale, shift, mean, invstd = _bn_frozen_coeffs(bn)
         a, _ = K.bn_act(y, scale, shift, relu=True, pool=False)
         if any(ctx.needs_input_grad):
-            ctx.save_for_backward(x, y, scale, shift, mean, invstd, gamma)
-            ctx.meta = (weight.shape, batch)
+            ctx.save_for_backward(x, y, scale, shift, mean, invstd, gamma,
+                                  weight if ctx.needs_input_grad[0] else None)
+            ctx.meta = (weight.shape, batch, x_dtype)
             ctx.params = (weight, gamma, beta)
         return from_nhwc(a)
 
     @staticmethod
     def backward(ctx, dA):
-        x, y, scale, shift, mean, invstd, gamma = ctx.saved_tensors
-        wshape, batch = ctx.meta
+        x, y, scale, shift, mean, invstd, gamma, weight = ctx.saved_tensors
+        wshape, batch, x_dtype = ctx.meta
         p_w, p_gamma, p_beta = ctx.params
         bn_t = _grad_targets(p_gamma, p_beta) if ctx.needs_input_grad[2] and ctx.needs_input_grad[3] else None
         dy, dgamma, dbeta = _bn_backward(to_nhwc(dA), None, None, y, scale, shift, mean, invstd, gamma, batch,
                                          targets=bn_t)
         if bn_t is not None:
             _grads_done(p_gamma, p_beta)
+        dx = K.conv_in_dgrad(dy, weight.contiguous(), wshape[1]).to(x_dtype) if ctx.needs_input_grad[0] else None
         gw = None
         if ctx.needs_input_grad[1]:
             w_t = _grad_targets(p_w)
@@ -269,7 +270,7 @@ class ConvInBnRelu(torch.autograd.Function):
                 _grads_done(p_w)
             else:
                 gw = K.conv_in_wgrad(x, dy, wshape[0])
-        return None, gw, dgamma, dbeta, None
+        return dx, gw, dgamma, dbeta, None
 
 
 class Upsample2x(torch.autograd.Function):
