@@ -263,7 +263,11 @@ int ub2_confusion(const void* pred, const long long* target, int mode, int N, in
 /* BASELINE configs[0] (AttentionUNet fp32 forward) and north_star's "fp32/TF32 mode, logits within
  * 1e-3": the eval-mode forward of every block of unet/models/layers.py with fp32 NHWC activations
  * (element strides), BatchNorm folded with the running statistics, the 3x3 / 1x1 convolutions on
- * the tensor cores as kind::tf32.  Forward only. */
+ * the tensor cores as kind::tf32.  Forward only.
+ * Every count (N, H, W, C, Ci, Cx, K, hin, win, hu, wu) must be > 0 and channel counts multiples of 4, with
+ * Ho >= hu and Wo >= wu, H and W >= 2 for the max-pool and K <= 8 for the head; every pointer is required except the
+ * head's bias; float4-accessed tensors (activations, q, xp) need 16-byte-aligned pointers.  Anything else returns
+ * UB2_ERR_SHAPE (or UB2_ERR_ALIGN) before the device is touched. */
 /* nn.Conv2d (+ folded BN + ReLU) of layers.py:32-37,152,158: in0/in1 fp32 NHWC (virtual concat),
  * wgt = ub2_f32_pack_weight output (Cout,taps,C0+C1) fp32, out fp32 NHWC; out = relu?(scale*acc+shift).
  * exact_out = 0: the result is rounded to TF32 (it feeds the next single-pass convolution: inference);
@@ -335,7 +339,18 @@ int ub2_predict_mask(const float* logits, int N, int C, long long HW, float thre
  * w_lo] (ub2_f32_split_tf32, ub2_f32_pack_weight3); weight gradient: ub2_conv_wgrad on the (hi, lo) bf16 halves of
  * ub2_f32_split_bf16 (kind::tf32 has no MN-major operand mode).  Reductions write one fp64 row per block
  * (`rows` = the matching *_rows query) that the bf16 path's finalize entry points fold (ub2_bn_finalize,
- * ub2_bn_bwd_finalize, ub2_gate_bwd_finalize).  See csrc/fp32_train.cu for the per-kernel reference lines. */
+ * ub2_bn_bwd_finalize, ub2_gate_bwd_finalize).  See csrc/fp32_train.cu for the per-kernel reference lines.
+ * Arguments are checked before the device is touched.  UB2_ERR_SHAPE: a count <= 0 (N, H, W, C, Ci, Cx, K, n, pixels,
+ * hin, win, hu, wu), a channel count not a multiple of 4, Ho < hu or Wo < wu, a channel stride ld* below its channel
+ * count, C > 1024 for the per-channel reductions, Ci > 512 for ub2_f32_gate_bwd_s, K > 8 or 8*(K*C + K) floats over
+ * 48 KB for ub2_f32_outc_bwd, or a NULL pointer other than these optional ones:
+ *   - dA or dP of the act_bwd passes (not both; dP needs idx; ld_da is ignored without dA), and scale / shift of
+ *     ub2_f32_act_bwd_apply when relu == 0;
+ *   - x1 of ub2_f32_split_tf32 when C1 == 0 (ld1 is then ignored);
+ *   - a_out of ub2_f32_gate_apply; da, dw and db of ub2_f32_outc_bwd (dw and db accumulate: +=).
+ * UB2_ERR_ALIGN: a channel stride not a multiple of 4, or a float4-accessed pointer not 16-byte aligned (idx: 4,
+ * partials: 8).  UB2_ERR_WORKSPACE: rows other than the matching *_rows query.  ub2_f32_conv_in_wgrad's grad
+ * accumulates (+=). */
 int ub2_f32_channel_rows(long long pixels, int C);
 int ub2_f32_channel_stats(const float* x, int ld, long long pixels, int C, double* partials, int rows, void* stream);
 int ub2_f32_scalar_rows(long long n);

@@ -230,8 +230,16 @@ using namespace ub2;
 
 extern "C" {
 
+// Argument checks as in fp32_train.cu, before the device is touched: counts <= 0, channel counts that are not
+// multiples of 4, Ho < hu or NULL pointers (bias alone is optional) return UB2_ERR_SHAPE; a pointer that a float4
+// access cannot use, UB2_ERR_ALIGN.
+static bool c4(int C) { return C > 0 && C % 4 == 0; }
+static bool al16(const void* p) { return aligned_to(p, 16); }
+static bool al4(const void* p) { return aligned_to(p, 4); }
+
 int ub2_f32_pack_weight(const float* w, float* out, int Cout, int Cin, int taps, void* stream) {
-  if (Cout <= 0 || Cin <= 0 || (taps != 1 && taps != 9)) return UB2_ERR_SHAPE;
+  if (w == nullptr || out == nullptr || Cout <= 0 || Cin <= 0 || (taps != 1 && taps != 9)) return UB2_ERR_SHAPE;
+  if (!al4(w) || !al4(out)) return UB2_ERR_ALIGN;
   const long long total = static_cast<long long>(Cout) * Cin * taps;
   launch(f32_pack_weight_kernel, stream_grid(total, 256, num_sms(), 8), 256, 0, static_cast<cudaStream_t>(stream), w, out, Cout, Cin, taps);
   return static_cast<int>(cudaGetLastError());
@@ -239,14 +247,18 @@ int ub2_f32_pack_weight(const float* w, float* out, int Cout, int Cin, int taps,
 
 int ub2_f32_conv_in(const float* x, const float* w, const float* scale, const float* shift, float* out, int N,
                     int Cin, int H, int W, int Cout, void* stream) {
-  if (Cout % 4 != 0 || Cin <= 0 || N <= 0) return UB2_ERR_SHAPE;
+  if (x == nullptr || w == nullptr || scale == nullptr || shift == nullptr || out == nullptr || !c4(Cout) || Cin <= 0 ||
+      N <= 0 || H <= 0 || W <= 0)
+    return UB2_ERR_SHAPE;
+  if (!al4(x) || !al4(w) || !al4(scale) || !al4(shift) || !al16(out)) return UB2_ERR_ALIGN;
   const long long total = static_cast<long long>(N) * H * W * (Cout / 4);
   launch(f32_conv_in_kernel, stream_grid(total, 256, num_sms(), 8), 256, 0, static_cast<cudaStream_t>(stream), x, w, scale, shift, out, N, Cin, H, W, Cout);
   return static_cast<int>(cudaGetLastError());
 }
 
 int ub2_f32_maxpool(const float* in, float* out, int N, int H, int W, int C, void* stream) {
-  if (C % 4 != 0 || H < 2 || W < 2 || N <= 0) return UB2_ERR_SHAPE;
+  if (in == nullptr || out == nullptr || !c4(C) || H < 2 || W < 2 || N <= 0) return UB2_ERR_SHAPE;
+  if (!al16(in) || !al16(out)) return UB2_ERR_ALIGN;
   const long long total = static_cast<long long>(N) * (H / 2) * (W / 2) * (C / 4);
   launch(f32_maxpool_kernel, stream_grid(total, 256, num_sms(), 8), 256, 0, static_cast<cudaStream_t>(stream), in, out, N, H, W, C);
   return static_cast<int>(cudaGetLastError());
@@ -254,7 +266,9 @@ int ub2_f32_maxpool(const float* in, float* out, int N, int H, int W, int C, voi
 
 int ub2_f32_upsample(const float* in, float* out, int N, int hin, int win, int hu, int wu, int Ho, int Wo, int C,
                      void* stream) {
-  if (C % 4 != 0 || Ho < hu || Wo < wu || N <= 0) return UB2_ERR_SHAPE;
+  if (in == nullptr || out == nullptr || !c4(C) || N <= 0 || hin <= 0 || win <= 0 || hu <= 0 || wu <= 0 || Ho < hu || Wo < wu)
+    return UB2_ERR_SHAPE;
+  if (!al16(in) || !al16(out)) return UB2_ERR_ALIGN;
   const long long total = static_cast<long long>(N) * Ho * Wo * (C / 4);
   launch(f32_upsample_kernel, stream_grid(total, 256, num_sms(), 8), 256, 0, static_cast<cudaStream_t>(stream), in, out, N, hin, win, hu, wu, Ho, Wo, C, ratio(hin, hu), ratio(win, wu));
   return static_cast<int>(cudaGetLastError());
@@ -264,7 +278,13 @@ int ub2_f32_gate(const float* q, const float* xp, const float* x, const float* s
                  const float* scale_x, const float* shift_x, const float* w_psi, const float* scale_psi,
                  const float* shift_psi, float* out, int N, int hin, int win, int H, int W, int Ci, int Cx,
                  void* stream) {
-  if (Ci % 4 != 0 || Cx % 4 != 0 || N <= 0) return UB2_ERR_SHAPE;
+  if (q == nullptr || xp == nullptr || x == nullptr || scale_g == nullptr || shift_g == nullptr || scale_x == nullptr ||
+      shift_x == nullptr || w_psi == nullptr || scale_psi == nullptr || shift_psi == nullptr || out == nullptr)
+    return UB2_ERR_SHAPE;
+  if (!c4(Ci) || !c4(Cx) || N <= 0 || hin <= 0 || win <= 0 || H <= 0 || W <= 0) return UB2_ERR_SHAPE;
+  if (!al16(q) || !al16(xp) || !al16(x) || !al16(out) || !al4(scale_g) || !al4(shift_g) || !al4(scale_x) || !al4(shift_x) ||
+      !al4(w_psi) || !al4(scale_psi) || !al4(shift_psi))
+    return UB2_ERR_ALIGN;
   const long long pixels = static_cast<long long>(N) * H * W;
   launch(f32_gate_kernel, stream_grid(pixels, 8, num_sms(), 8), 256, 0, static_cast<cudaStream_t>(stream), q, xp, x, scale_g, shift_g, scale_x, shift_x, w_psi, scale_psi, shift_psi, out, N, hin, win, H, W, Ci, Cx, ratio(hin, H), ratio(win, W));
   return static_cast<int>(cudaGetLastError());
@@ -272,7 +292,9 @@ int ub2_f32_gate(const float* q, const float* xp, const float* x, const float* s
 
 int ub2_f32_outc(const float* a, const float* w, const float* bias, float* logits, int N, int H, int W, int C,
                  int K, void* stream) {
-  if (C % 4 != 0 || K <= 0 || K > 8 || N <= 0) return UB2_ERR_SHAPE;
+  if (a == nullptr || w == nullptr || logits == nullptr || !c4(C) || K <= 0 || K > 8 || N <= 0 || H <= 0 || W <= 0)
+    return UB2_ERR_SHAPE;
+  if (!al16(a) || !al4(w) || !al4(bias) || !al4(logits)) return UB2_ERR_ALIGN;
   const long long pixels = static_cast<long long>(N) * H * W;
   launch(f32_outc_kernel, stream_grid(pixels, 256, num_sms(), 8), 256, 0, static_cast<cudaStream_t>(stream), a, w, bias, logits, N, H, W, C, K);
   return static_cast<int>(cudaGetLastError());

@@ -214,7 +214,7 @@ f32_act_bwd_reduce_kernel(const float* __restrict__ dA, int ld_da, const float* 
   fold_channels<2>(acc, lane, lanes, c4, c4s, C, partials + static_cast<size_t>(blockIdx.x) * 2 * C, smem);
 }
 
-// dy = coef0*dz + coef1*y + coef2 (TF32-rounded: it feeds the weight- and data-gradient convolutions)
+// dy = coef0*dz + coef1*y + coef2, unrounded (the convolutions that take it split it themselves)
 __global__ void __launch_bounds__(kFT)
 f32_act_bwd_apply_kernel(const float* __restrict__ dA, int ld_da, const float* __restrict__ dP,
                          const unsigned char* __restrict__ idx, const float* __restrict__ y,
@@ -705,13 +705,23 @@ extern "C" {
 #define F32_STREAM static_cast<cudaStream_t>(stream)
 #define F32_DONE return static_cast<int>(cudaGetLastError())
 
+// Every entry point checks its arguments before it touches the device: a count <= 0, a channel count that is not a
+// multiple of 4, a channel stride below its channel count or a NULL pointer the kernel reads or writes returns
+// UB2_ERR_SHAPE; a channel stride that is not a multiple of 4, or a pointer that a float4 (uchar4, double) access
+// cannot use, UB2_ERR_ALIGN; `rows` other than the matching *_rows query, UB2_ERR_WORKSPACE.
+static bool c4(int C) { return C > 0 && C % 4 == 0; }
+static bool al16(const void* p) { return aligned_to(p, 16); }
+static bool al8(const void* p) { return aligned_to(p, 8); }
+static bool al4(const void* p) { return aligned_to(p, 4); }
+
 int ub2_f32_channel_rows(long long pixels, int C) {
-  if (C <= 0 || C % 4 != 0 || C > 4 * kFT || pixels <= 0) return UB2_ERR_SHAPE;
+  if (!c4(C) || C > 4 * kFT || pixels <= 0) return UB2_ERR_SHAPE;
   return chan_grid(pixels, C);
 }
 
 int ub2_f32_channel_stats(const float* x, int ld, long long pixels, int C, double* partials, int rows, void* stream) {
-  if (C <= 0 || C % 4 != 0 || C > 4 * kFT || ld % 4 != 0 || pixels <= 0) return UB2_ERR_SHAPE;
+  if (x == nullptr || partials == nullptr || !c4(C) || C > 4 * kFT || ld < C || pixels <= 0) return UB2_ERR_SHAPE;
+  if (ld % 4 != 0 || !al16(x) || !al8(partials)) return UB2_ERR_ALIGN;
   if (rows != chan_grid(pixels, C)) return UB2_ERR_WORKSPACE;
   launch(f32_channel_stats_kernel, rows, chan_lanes(C) * (C / 4), 0, F32_STREAM, x, ld, pixels, C, partials);
   F32_DONE;
@@ -720,7 +730,8 @@ int ub2_f32_channel_stats(const float* x, int ld, long long pixels, int C, doubl
 int ub2_f32_scalar_rows(long long n) { return n > 0 ? elem_grid(n) : UB2_ERR_SHAPE; }
 
 int ub2_f32_scalar_stats(const float* x, long long n, double* partials, int rows, void* stream) {
-  if (n <= 0) return UB2_ERR_SHAPE;
+  if (x == nullptr || partials == nullptr || n <= 0) return UB2_ERR_SHAPE;
+  if (!al4(x) || !al8(partials)) return UB2_ERR_ALIGN;
   if (rows != elem_grid(n)) return UB2_ERR_WORKSPACE;
   launch(f32_scalar_stats_kernel, rows, kFT, 0, F32_STREAM, x, n, partials);
   F32_DONE;
@@ -728,23 +739,36 @@ int ub2_f32_scalar_stats(const float* x, long long n, double* partials, int rows
 
 int ub2_f32_affine_act(const float* y, const float* scale, const float* shift, float* out, long long pixels, int C,
                        int relu, void* stream) {
-  if (C <= 0 || C % 4 != 0 || pixels <= 0) return UB2_ERR_SHAPE;
+  if (y == nullptr || scale == nullptr || shift == nullptr || out == nullptr || !c4(C) || pixels <= 0) return UB2_ERR_SHAPE;
+  if (!al16(y) || !al16(scale) || !al16(shift) || !al16(out)) return UB2_ERR_ALIGN;
   launch(f32_affine_act_kernel, elem_grid(pixels * (C / 4)), kFT, 0, F32_STREAM, y, scale, shift, out, pixels, C, relu);
   F32_DONE;
 }
 
 int ub2_f32_maxpool_idx(const float* a, float* p, unsigned char* idx, int N, int H, int W, int C, void* stream) {
-  if (C <= 0 || C % 4 != 0 || N <= 0 || H < 2 || W < 2) return UB2_ERR_SHAPE;
+  if (a == nullptr || p == nullptr || idx == nullptr || !c4(C) || N <= 0 || H < 2 || W < 2) return UB2_ERR_SHAPE;
+  if (!al16(a) || !al16(p) || !al4(idx)) return UB2_ERR_ALIGN;
   launch(f32_maxpool_idx_kernel, elem_grid(static_cast<long long>(N) * (H / 2) * (W / 2) * (C / 4)), kFT, 0, F32_STREAM, a, p, idx, N,
          H, W, C);
   F32_DONE;
 }
 
+// The gradient sources of the two BatchNorm-backward passes: dA (channel stride ld_da), dP routed through idx, or both.
+static int act_bwd_args(const float* dA, int ld_da, const float* dP, const unsigned char* idx, const float* y, int N, int H,
+                        int W, int C) {
+  if (y == nullptr || !c4(C) || N <= 0 || H <= 0 || W <= 0) return UB2_ERR_SHAPE;
+  if ((dA == nullptr && dP == nullptr) || (dP != nullptr && idx == nullptr) || (dA != nullptr && ld_da < C)) return UB2_ERR_SHAPE;
+  if ((dA != nullptr && ld_da % 4 != 0) || !al16(dA) || !al16(dP) || !al4(idx) || !al16(y)) return UB2_ERR_ALIGN;
+  return UB2_OK;
+}
+
 int ub2_f32_act_bwd_reduce(const float* dA, int ld_da, const float* dP, const unsigned char* idx, const float* y,
                            const float* scale, const float* shift, double* partials, int rows, int N, int H, int W, int C,
                            int relu, void* stream) {
-  if (C <= 0 || C % 4 != 0 || C > 4 * kFT || N <= 0 || H <= 0 || W <= 0 || (dA == nullptr && dP == nullptr)) return UB2_ERR_SHAPE;
-  if (dA != nullptr && ld_da % 4 != 0) return UB2_ERR_ALIGN;
+  const int rc = act_bwd_args(dA, ld_da, dP, idx, y, N, H, W, C);
+  if (rc != UB2_OK) return rc;
+  if (scale == nullptr || shift == nullptr || partials == nullptr || C > 4 * kFT) return UB2_ERR_SHAPE;
+  if (!al16(scale) || !al16(shift) || !al8(partials)) return UB2_ERR_ALIGN;
   const long long pixels = static_cast<long long>(N) * H * W;
   if (rows != chan_grid(pixels, C)) return UB2_ERR_WORKSPACE;
   launch(f32_act_bwd_reduce_kernel, rows, chan_lanes(C) * (C / 4), 0, F32_STREAM, dA, ld_da, dP, idx, y, scale, shift, partials, N, H,
@@ -755,16 +779,24 @@ int ub2_f32_act_bwd_reduce(const float* dA, int ld_da, const float* dP, const un
 int ub2_f32_act_bwd_apply(const float* dA, int ld_da, const float* dP, const unsigned char* idx, const float* y,
                           const float* scale, const float* shift, const float* coef, float* dy, int N, int H, int W, int C,
                           int relu, void* stream) {
-  if (C <= 0 || C % 4 != 0 || N <= 0 || H <= 0 || W <= 0 || (dA == nullptr && dP == nullptr)) return UB2_ERR_SHAPE;
-  if (dA != nullptr && ld_da % 4 != 0) return UB2_ERR_ALIGN;
+  const int rc = act_bwd_args(dA, ld_da, dP, idx, y, N, H, W, C);
+  if (rc != UB2_OK) return rc;
+  if (coef == nullptr || dy == nullptr || (relu && (scale == nullptr || shift == nullptr))) return UB2_ERR_SHAPE;
+  if (!al16(scale) || !al16(shift) || !al16(coef) || !al16(dy)) return UB2_ERR_ALIGN;
   launch(f32_act_bwd_apply_kernel, elem_grid(static_cast<long long>(N) * H * W * (C / 4)), kFT, 0, F32_STREAM, dA, ld_da, dP, idx, y,
          scale, shift, coef, dy, N, H, W, C, relu);
   F32_DONE;
 }
 
+// (hin,win) resampled to (hu,wu) inside an (Ho,Wo) canvas
+static bool resample_geom_ok(int N, int hin, int win, int hu, int wu, int Ho, int Wo, int C) {
+  return c4(C) && N > 0 && hin > 0 && win > 0 && hu > 0 && wu > 0 && Ho >= hu && Wo >= wu;
+}
+
 int ub2_f32_upsample_bwd(const float* dout, int ld_dout, float* din, int N, int hin, int win, int hu, int wu, int Ho, int Wo,
                          int C, void* stream) {
-  if (C <= 0 || C % 4 != 0 || Ho < hu || Wo < wu || N <= 0 || hin <= 0 || win <= 0 || ld_dout % 4 != 0) return UB2_ERR_SHAPE;
+  if (dout == nullptr || din == nullptr || !resample_geom_ok(N, hin, win, hu, wu, Ho, Wo, C) || ld_dout < C) return UB2_ERR_SHAPE;
+  if (ld_dout % 4 != 0 || !al16(dout) || !al16(din)) return UB2_ERR_ALIGN;
   launch(f32_upsample_bwd_kernel, elem_grid(static_cast<long long>(N) * hin * win * (C / 4)), kFT, 0, F32_STREAM, dout, ld_dout, din, N,
          hin, win, hu, wu, Ho, Wo, C, ratio_f(hin, hu), ratio_f(win, wu));
   F32_DONE;
@@ -772,7 +804,10 @@ int ub2_f32_upsample_bwd(const float* dout, int ld_dout, float* din, int N, int 
 
 int ub2_f32_gate_psi(const float* u, const float* xp, const float* sg, const float* hg, const float* sx, const float* hx,
                      const float* wpsi, float* psi_raw, long long pixels, int Ci, void* stream) {
-  if (Ci <= 0 || Ci % 4 != 0 || pixels <= 0) return UB2_ERR_SHAPE;
+  if (u == nullptr || xp == nullptr || sg == nullptr || hg == nullptr || sx == nullptr || hx == nullptr || wpsi == nullptr ||
+      psi_raw == nullptr || !c4(Ci) || pixels <= 0)
+    return UB2_ERR_SHAPE;
+  if (!al16(u) || !al16(xp) || !al16(sg) || !al16(hg) || !al16(sx) || !al16(hx) || !al16(wpsi) || !al4(psi_raw)) return UB2_ERR_ALIGN;
   launch(f32_gate_psi_kernel, stream_grid(pixels, kFT / 32, num_sms(), 8), kFT, 0, F32_STREAM, u, xp, sg, hg, sx, hx, wpsi, psi_raw,
          pixels, Ci);
   F32_DONE;
@@ -780,7 +815,9 @@ int ub2_f32_gate_psi(const float* u, const float* xp, const float* sg, const flo
 
 int ub2_f32_gate_apply(const float* psi_raw, const float* spsi, const float* hpsi, const float* x, float* out, float* a_out,
                        long long pixels, int Cx, void* stream) {
-  if (Cx <= 0 || Cx % 4 != 0 || pixels <= 0) return UB2_ERR_SHAPE;
+  if (psi_raw == nullptr || spsi == nullptr || hpsi == nullptr || x == nullptr || out == nullptr || !c4(Cx) || pixels <= 0)
+    return UB2_ERR_SHAPE;
+  if (!al16(x) || !al16(out) || !al4(a_out)) return UB2_ERR_ALIGN;
   launch(f32_gate_apply_kernel, elem_grid(pixels * (Cx / 4)), kFT, 0, F32_STREAM, psi_raw, spsi, hpsi, x, out, a_out, pixels, Cx);
   F32_DONE;
 }
@@ -789,7 +826,10 @@ int ub2_f32_gate_rows(long long pixels) { return pixels > 0 ? stream_grid(pixels
 
 int ub2_f32_gate_bwd_a(const float* dout, int ld_do, const float* x, const float* a, const float* psi_raw, float* dx,
                        float* dpsin, double* partials, int rows, long long pixels, int Cx, void* stream) {
-  if (Cx <= 0 || Cx % 4 != 0 || pixels <= 0 || ld_do % 4 != 0) return UB2_ERR_SHAPE;
+  if (dout == nullptr || x == nullptr || a == nullptr || psi_raw == nullptr || dx == nullptr || dpsin == nullptr ||
+      partials == nullptr || !c4(Cx) || pixels <= 0 || ld_do < Cx)
+    return UB2_ERR_SHAPE;
+  if (ld_do % 4 != 0 || !al16(dout) || !al16(x) || !al16(dx) || !al8(partials)) return UB2_ERR_ALIGN;
   if (rows != stream_grid(pixels, kFT / 32, num_sms(), 4)) return UB2_ERR_WORKSPACE;
   launch(f32_gate_bwd_a_kernel, rows, kFT, 0, F32_STREAM, dout, ld_do, x, a, psi_raw, dx, dpsin, partials, pixels, Cx);
   F32_DONE;
@@ -798,7 +838,12 @@ int ub2_f32_gate_bwd_a(const float* dout, int ld_do, const float* x, const float
 int ub2_f32_gate_bwd_s(const float* dpsin, const float* psi_raw, const float* coef_psi, const float* u, const float* xp,
                        const float* sg, const float* hg, const float* sx, const float* hx, const float* wpsi, float* ds,
                        double* partials, int rows, long long pixels, int Ci, void* stream) {
-  if (Ci <= 0 || Ci % 4 != 0 || Ci > 128 * kGI || pixels <= 0) return UB2_ERR_SHAPE;
+  if (dpsin == nullptr || psi_raw == nullptr || coef_psi == nullptr || u == nullptr || xp == nullptr || sg == nullptr ||
+      hg == nullptr || sx == nullptr || hx == nullptr || wpsi == nullptr || ds == nullptr || partials == nullptr ||
+      !c4(Ci) || Ci > 128 * kGI || pixels <= 0)
+    return UB2_ERR_SHAPE;
+  if (!al16(u) || !al16(xp) || !al16(sg) || !al16(hg) || !al16(sx) || !al16(hx) || !al16(wpsi) || !al16(ds) || !al8(partials))
+    return UB2_ERR_ALIGN;
   if (rows != stream_grid(pixels, kFT / 32, num_sms(), 4)) return UB2_ERR_WORKSPACE;
   const size_t smem = static_cast<size_t>(kFT / 32) * 4 * Ci * sizeof(float);
   if (smem > 48 * 1024) {
@@ -812,7 +857,10 @@ int ub2_f32_gate_bwd_s(const float* dpsin, const float* psi_raw, const float* co
 
 int ub2_f32_gate_bwd_xg(const float* ds, const float* xp, const float* u, const float* coef, float* dxp, float* du,
                         long long pixels, int Ci, void* stream) {
-  if (Ci <= 0 || Ci % 4 != 0 || pixels <= 0) return UB2_ERR_SHAPE;
+  if (ds == nullptr || xp == nullptr || u == nullptr || coef == nullptr || dxp == nullptr || du == nullptr || !c4(Ci) ||
+      pixels <= 0)
+    return UB2_ERR_SHAPE;
+  if (!al16(ds) || !al16(xp) || !al16(u) || !al16(coef) || !al16(dxp) || !al16(du)) return UB2_ERR_ALIGN;
   launch(f32_gate_bwd_xg_kernel, elem_grid(pixels * (Ci / 4)), kFT, 0, F32_STREAM, ds, xp, u, coef, dxp, du, pixels, Ci);
   F32_DONE;
 }
@@ -824,7 +872,10 @@ int ub2_f32_outc_rows(int N, int H, int W) {
 
 int ub2_f32_outc_bwd(const float* dlogits, const float* a, const float* w, float* da, double* partials, int rows, float* dw,
                      float* db, int N, int H, int W, int C, int K, void* stream) {
-  if (C <= 0 || C % 4 != 0 || K < 1 || K > 8 || N <= 0 || H <= 0 || W <= 0) return UB2_ERR_SHAPE;
+  if (dlogits == nullptr || a == nullptr || w == nullptr || partials == nullptr || !c4(C) || K < 1 || K > 8 || N <= 0 ||
+      H <= 0 || W <= 0)
+    return UB2_ERR_SHAPE;
+  if (!al4(dlogits) || !al16(a) || !al16(w) || !al16(da) || !al8(partials) || !al4(dw) || !al4(db)) return UB2_ERR_ALIGN;
   if (rows != ub2_f32_outc_rows(N, H, W)) return UB2_ERR_WORKSPACE;
   const int cols = K * C + K;
   const size_t smem = static_cast<size_t>(kFT / 32) * cols * sizeof(float);
@@ -838,7 +889,8 @@ int ub2_f32_outc_bwd(const float* dlogits, const float* a, const float* w, float
 }
 
 int ub2_f32_conv_in_raw(const float* x, const float* w, float* out, int N, int Cin, int H, int W, int Cout, void* stream) {
-  if (Cout <= 0 || Cout % 4 != 0 || Cin <= 0 || N <= 0 || H <= 0 || W <= 0) return UB2_ERR_SHAPE;
+  if (x == nullptr || w == nullptr || out == nullptr || !c4(Cout) || Cin <= 0 || N <= 0 || H <= 0 || W <= 0) return UB2_ERR_SHAPE;
+  if (!al4(x) || !al4(w) || !al16(out)) return UB2_ERR_ALIGN;
   launch(f32_conv_in_raw_kernel, elem_grid(static_cast<long long>(N) * H * W * (Cout / 4)), kFT, 0, F32_STREAM, x, w, out, N, Cin, H, W,
          Cout);
   F32_DONE;
@@ -846,7 +898,10 @@ int ub2_f32_conv_in_raw(const float* x, const float* w, float* out, int N, int C
 
 int ub2_f32_conv_in_wgrad(const float* x, const float* dy, double* partials, int rows, float* grad, int N, int Cin, int H,
                           int W, int Cout, void* stream) {
-  if (Cout <= 0 || Cout % 4 != 0 || Cout > 4 * kFT || Cin <= 0 || N <= 0 || H <= 0 || W <= 0) return UB2_ERR_SHAPE;
+  if (x == nullptr || dy == nullptr || partials == nullptr || grad == nullptr || !c4(Cout) || Cout > 4 * kFT || Cin <= 0 ||
+      N <= 0 || H <= 0 || W <= 0)
+    return UB2_ERR_SHAPE;
+  if (!al4(x) || !al16(dy) || !al8(partials) || !al4(grad)) return UB2_ERR_ALIGN;
   const long long pixels = static_cast<long long>(N) * H * W;
   if (rows != chan_grid(pixels, Cout)) return UB2_ERR_WORKSPACE;
   launch(f32_conv_in_wgrad_kernel, rows, chan_lanes(Cout) * (Cout / 4), 0, F32_STREAM, x, dy, partials, N, Cin, H, W, Cout);
@@ -857,7 +912,8 @@ int ub2_f32_conv_in_wgrad(const float* x, const float* dy, double* partials, int
 }
 
 int ub2_f32_split_bf16(const float* x, void* hi, void* lo, long long n, void* stream) {
-  if (n <= 0 || n % 4 != 0) return UB2_ERR_SHAPE;
+  if (x == nullptr || hi == nullptr || lo == nullptr || n <= 0 || n % 4 != 0) return UB2_ERR_SHAPE;
+  if (!al16(x) || !al8(hi) || !al8(lo)) return UB2_ERR_ALIGN;
   launch(f32_split_bf16_kernel, elem_grid(n / 4), kFT, 0, F32_STREAM, x, static_cast<__nv_bfloat16*>(hi), static_cast<__nv_bfloat16*>(lo),
          n / 4);
   F32_DONE;
@@ -865,20 +921,24 @@ int ub2_f32_split_bf16(const float* x, void* hi, void* lo, long long n, void* st
 
 int ub2_f32_split_tf32(const float* x0, int ld0, int C0, const float* x1, int ld1, int C1, float* out, long long pixels,
                        void* stream) {
-  if (C0 <= 0 || C0 % 4 != 0 || C1 < 0 || C1 % 4 != 0 || ld0 % 4 != 0 || (C1 > 0 && ld1 % 4 != 0) || pixels <= 0) return UB2_ERR_SHAPE;
+  if (x0 == nullptr || out == nullptr || !c4(C0) || ld0 < C0 || C1 < 0 || C1 % 4 != 0 || pixels <= 0) return UB2_ERR_SHAPE;
+  if (C1 > 0 && (x1 == nullptr || ld1 < C1)) return UB2_ERR_SHAPE;
+  if (ld0 % 4 != 0 || (C1 > 0 && ld1 % 4 != 0) || !al16(x0) || !al16(x1) || !al16(out)) return UB2_ERR_ALIGN;
   launch(f32_split_tf32_kernel, elem_grid(pixels * ((C0 + C1) / 4)), kFT, 0, F32_STREAM, x0, ld0, C0, x1, ld1, C1, out, pixels);
   F32_DONE;
 }
 
 int ub2_f32_pack_weight3(const float* w, float* out, int Cout, int Cin, int taps, int dgrad, void* stream) {
-  if (Cout <= 0 || Cin <= 0 || taps <= 0) return UB2_ERR_SHAPE;
+  if (w == nullptr || out == nullptr || Cout <= 0 || Cin <= 0 || taps <= 0) return UB2_ERR_SHAPE;
+  if (!al4(w) || !al4(out)) return UB2_ERR_ALIGN;
   launch(f32_pack_weight3_kernel, elem_grid(static_cast<long long>(Cout) * Cin * taps), kFT, 0, F32_STREAM, w, out, Cout, Cin, taps, dgrad);
   F32_DONE;
 }
 
 int ub2_f32_upsample_fwd(const float* in, float* out, int N, int hin, int win, int hu, int wu, int Ho, int Wo, int C,
                          void* stream) {
-  if (C <= 0 || C % 4 != 0 || Ho < hu || Wo < wu || N <= 0 || hin <= 0 || win <= 0) return UB2_ERR_SHAPE;
+  if (in == nullptr || out == nullptr || !resample_geom_ok(N, hin, win, hu, wu, Ho, Wo, C)) return UB2_ERR_SHAPE;
+  if (!al16(in) || !al16(out)) return UB2_ERR_ALIGN;
   launch(f32_upsample_fwd_kernel, elem_grid(static_cast<long long>(N) * Ho * Wo * (C / 4)), kFT, 0, F32_STREAM, in, out, N, hin, win, hu,
          wu, Ho, Wo, C, ratio_f(hin, hu), ratio_f(win, wu));
   F32_DONE;

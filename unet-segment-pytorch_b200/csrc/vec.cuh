@@ -137,6 +137,9 @@ __device__ __forceinline__ void rows_sum_wide(const double* __restrict__ partial
   }
 }
 
+// Host-side argument checks: the pointer is a multiple of `bytes` (NULL passes; callers check it separately).
+inline bool aligned_to(const void* p, uintptr_t bytes) { return (reinterpret_cast<uintptr_t>(p) & (bytes - 1)) == 0; }
+
 // Grid for a bandwidth-bound grid-stride kernel: a multiple of the SM count.
 inline int stream_grid(long long work_items, int threads, int sms, int blocks_per_sm = 8) {
   long long need = (work_items + threads - 1) / threads;

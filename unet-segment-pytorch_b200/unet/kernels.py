@@ -54,7 +54,8 @@ def _nhwc32(t: torch.Tensor):
     """fp32 / TF32 mode: (N,H,W,C) fp32 whose channel stride may exceed C (a channel slice)."""
     assert t.dim() == 4 and t.dtype == F32 and t.stride(3) == 1, "expected NHWC fp32"
     n, h, w, c = t.shape
-    ld = t.stride(2) if w > 1 else c
+    # the stride between consecutive pixels: across a row, or (W = 1) down the rows, or (H = W = 1) across images
+    ld = t.stride(2) if w > 1 else t.stride(1) if h > 1 else t.stride(0) if n > 1 else c
     if h > 1:
         assert t.stride(1) == w * ld, "expected dense NHWC rows"
     if n > 1:
