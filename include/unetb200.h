@@ -377,6 +377,18 @@ int ub2_f32_split_bf16(const float* x, void* hi, void* lo, long long n, void* st
 int ub2_f32_split_tf32(const float* x0, int ld0, int C0, const float* x1, int ld1, int C1, float* out, long long pixels, void* stream);
 int ub2_f32_pack_weight3(const float* w, float* out, int Cout, int Cin, int taps, int dgrad, void* stream);
 int ub2_f32_upsample_fwd(const float* in, float* out, int N, int hin, int win, int hu, int wu, int Ho, int Wo, int C, void* stream);
+/* ConvTranspose2d(C, C/2, 2, stride 2) + F.pad in fp32 (layers.py:81, :98-102, :217-221): the ub2_shuffle2x2_* pixel
+ * shuffle, its transpose and the bias gradient on fp32 tensors.  t / dt: (N,h,w,4*C) with channel stride ld_t / ld_dt
+ * >= 4*C; out / dout: (N,Ho,Wo,C) with stride ld_out / ld_dout >= C (dout may be a channel slice of a wider
+ * tensor).  C % 4 == 0 and C <= 1024, Ho >= 2h, Wo >= 2w.  `partials`: (rows, C) doubles with rows =
+ * ub2_f32_shuffle2x2_rows(...), folded into dbias (+=); partials == NULL skips the bias gradient and dbias is then
+ * ignored.  ub2_f32_pack_convt_weight writes the exact fp32 (4*Cout, Cin) 1x1 weight (row (i*2+j)*Cout + co) that
+ * ub2_f32_pack_weight / ub2_f32_pack_weight3 (taps = 1) take as OIHW (4*Cout, Cin, 1, 1), and the epilogue vectors
+ * scale4 = 1, shift4 = bias tiled four times (zeros when bias is NULL). */
+int ub2_f32_shuffle2x2_fwd(const float* t, int ld_t, float* out, int ld_out, int N, int h, int w, int C, int Ho, int Wo, void* stream);
+int ub2_f32_shuffle2x2_rows(int N, int h, int w, int C, int Ho, int Wo);
+int ub2_f32_shuffle2x2_bwd(const float* dout, int ld_dout, float* dt, int ld_dt, double* partials, int rows, float* dbias, int N, int h, int w, int C, int Ho, int Wo, void* stream);
+int ub2_f32_pack_convt_weight(const float* w, const float* bias, float* fwd, float* scale4, float* shift4, int Cin, int Cout, void* stream);
 
 #ifdef __cplusplus
 }

@@ -46,7 +46,7 @@ __device__ __forceinline__ F8 load8_stream(const __nv_bfloat16* p) {
                : "l"(p));
   return unpack8(u);
 }
-__device__ __forceinline__ uint4 ld_stream16(const __nv_bfloat16* p) {
+__device__ __forceinline__ uint4 ld_stream16(const void* p) {   // any 16 bytes: 8 bf16 or 4 fp32
   uint4 u;
   asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
                : "=r"(u.x), "=r"(u.y), "=r"(u.z), "=r"(u.w)

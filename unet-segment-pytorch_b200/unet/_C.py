@@ -87,7 +87,7 @@ def stream() -> ctypes.c_void_p:
 
 # kernels launched per entry point (default 1); used for the bench's `gpu_launches` claim
 _KERNELS_PER_CALL = {"ub2_conv_in_wgrad": 2, "ub2_outc_bwd": 2, "ub2_seg_stats": 2, "ub2_wgrad_reduce_multi": 2,
-                     "ub2_shuffle2x2_bwd": 2}
+                     "ub2_shuffle2x2_bwd": 2, "ub2_f32_shuffle2x2_bwd": 2}
 LAUNCHES = 0
 
 

@@ -14,7 +14,7 @@ plain fp32 kernels.
   halves (three launches, 2^-16 relative: ``kind::tf32`` has no MN-major operand mode).  This is the
   accuracy mode — what the reference's own fp32 training computes — not the fast one: train in bf16 for speed.
 
-Reference semantics: unet/models/layers.py:16-255.  ``bilinear=False`` is bf16-only.
+Reference semantics: unet/models/layers.py:16-255.
 """
 from __future__ import annotations
 
@@ -180,6 +180,18 @@ def upsample(x, out_h, out_w):
     return nchw(out)
 
 
+def conv_transpose2x2(module, x, out_h, out_w):
+    """nn.ConvTranspose2d(C, C/2, kernel_size=2, stride=2) + F.pad to (out_h, out_w) (layers.py:81, :98-102,
+    :217-221): a 1x1 tensor-core convolution to 4*Cout channels with the bias in its epilogue, then the pixel
+    shuffle of csrc/shuffle.cu."""
+    _check(module, x)
+    if _training_path(module, x):
+        return ConvTranspose2x2F32.apply(x, module.weight, module.bias, int(out_h), int(out_w))
+    w1, scale4, shift4 = pack_convt_weight(module.weight, module.bias)
+    t = conv_packed(nhwc(x), None, _pack(w1), w1.shape[0], 1, scale4, shift4)
+    return nchw(shuffle2x2(t, module.weight.shape[1], out_h, out_w))
+
+
 def gate(module, g, x):
     """AttentionGate.forward (layers.py:171-192)."""
     _check(module, g, x)
@@ -310,6 +322,43 @@ def upsample_bwd_nhwc(dout, hin, win, hu, wu):
     return din
 
 
+def pack_convt_weight(weight, bias):
+    """(Cin, Cout, 2, 2) fp32 parameter -> (the exact 1x1 weight (4*Cout, Cin, 1, 1) OIHW, row (i*2+j)*Cout + co;
+    scale4 = ones, shift4 = bias tiled four times)."""
+    cin, cout = weight.shape[0], weight.shape[1]
+    w1 = torch.empty((4 * cout, cin, 1, 1), device=weight.device, dtype=F32)
+    ss = torch.empty((2, 4 * cout), device=weight.device, dtype=F32)
+    _C.call("ub2_f32_pack_convt_weight", ptr(weight.contiguous()), ptr(bias), ptr(w1), ptr(ss[0]), ptr(ss[1]), cin, cout,
+            stream())
+    return w1, ss[0], ss[1]
+
+
+def shuffle2x2(t, cout, out_h, out_w):
+    """t (N,h,w,4*Cout) fp32 -> (N,out_h,out_w,Cout): pixel shuffle of the transposed convolution + F.pad (zeros)."""
+    n, h, w, c4, ld = K._nhwc32(t)
+    assert c4 == 4 * cout
+    out = torch.empty((n, out_h, out_w, cout), device=t.device, dtype=F32)
+    _C.call("ub2_f32_shuffle2x2_fwd", ptr(t), ld, ptr(out), cout, n, h, w, cout, out_h, out_w, stream(),
+            work=(0.0, K._nbytes(t, out)))
+    return out
+
+
+def shuffle2x2_bwd(dout, h, w, want_bias=True):
+    """Transpose of shuffle2x2: dout (N,Ho,Wo,Cout), channel stride may exceed Cout -> (dt (N,h,w,4*Cout),
+    bias gradient (Cout,) or None)."""
+    n, ho, wo, cout, ld = K._nhwc32(dout)
+    dt = torch.empty((n, h, w, 4 * cout), device=dout.device, dtype=F32)
+    partials = db = None
+    rows = 0
+    if want_bias:
+        rows = K._rows("ub2_f32_shuffle2x2_rows", n, h, w, cout, ho, wo)
+        partials = torch.empty((rows, cout), device=dout.device, dtype=F64)
+        db = torch.zeros((cout,), device=dout.device, dtype=F32)
+    _C.call("ub2_f32_shuffle2x2_bwd", ptr(dout), ld, ptr(dt), 4 * cout, ptr(partials), rows, ptr(db), n, h, w, cout, ho, wo,
+            stream(), work=(0.0, K._nbytes(dout, dt)))
+    return dt, db
+
+
 def split_bf16(x):
     """fp32 NHWC -> (hi, lo) bf16 NHWC with x = hi + lo to 2^-16 relative."""
     x = _dense(x)
@@ -319,18 +368,33 @@ def split_bf16(x):
     return hi, lo
 
 
-def weight_grad(x0, x1, dy, wshape):
-    """dW of a convolution from fp32 operands: three bf16 tensor-core weight-gradient launches on the hi / lo
-    halves (a_hi.dy_hi + a_lo.dy_hi + a_hi.dy_lo) folded in a fixed order into an OIHW fp32 tensor."""
-    cout, cin, kh, kw = wshape
-    taps = kh * kw
+def _hilo_wgrad(x0, x1, dy, taps, fold):
+    """Weight gradient from fp32 operands: three bf16 tensor-core weight-gradient launches on the hi / lo halves
+    (a_hi.dy_hi + a_lo.dy_hi + a_hi.dy_lo); ``fold(partial, accumulate)`` reduces each launch's split-K partials
+    into the caller's fp32 gradient, the first one overwriting it, in this fixed order."""
     x0h, x0l = split_bf16(x0)
     x1h, x1l = split_bf16(x1) if x1 is not None else (None, None)
     dyh, dyl = split_bf16(dy)
+    fold(K.conv_wgrad(x0h, dyh, taps, x1=x1h), False)
+    fold(K.conv_wgrad(x0l, dyh, taps, x1=x1l), True)
+    fold(K.conv_wgrad(x0h, dyl, taps, x1=x1h), True)
+
+
+def weight_grad(x0, x1, dy, wshape):
+    """dW (OIHW fp32) of a convolution from fp32 operands (see _hilo_wgrad)."""
+    cout, cin, kh, kw = wshape
+    taps = kh * kw
     gw = torch.empty(wshape, device=dy.device, dtype=F32)
-    K.wgrad_reduce(K.conv_wgrad(x0h, dyh, taps, x1=x1h), cout, cin, taps, gw)
-    K.wgrad_reduce(K.conv_wgrad(x0l, dyh, taps, x1=x1l), cout, cin, taps, gw, accumulate=True)
-    K.wgrad_reduce(K.conv_wgrad(x0h, dyl, taps, x1=x1h), cout, cin, taps, gw, accumulate=True)
+    _hilo_wgrad(x0, x1, dy, taps, lambda part, acc: K.wgrad_reduce(part, cout, cin, taps, gw, accumulate=acc))
+    return gw
+
+
+def convt_weight_grad(a, dt, wshape):
+    """dW (Cin, Cout, 2, 2) fp32 of the transposed convolution: the 1x1 weight gradient of a (N,h,w,Cin) against the
+    shuffled gradient dt (N,h,w,4*Cout), folded into the ConvTranspose2d layout."""
+    cin, cout = wshape[0], wshape[1]
+    gw = torch.empty(wshape, device=dt.device, dtype=F32)
+    _hilo_wgrad(a, None, dt, 1, lambda part, acc: K.convt_wgrad_reduce(part, cin, cout, gw, accumulate=acc))
     return gw
 
 
@@ -454,6 +518,33 @@ class UpsampleF32(torch.autograd.Function):
     def backward(ctx, dout):
         h, w = ctx.geom
         return nchw(upsample_bwd_nhwc(nhwc_view(dout), h, w, 2 * h, 2 * w)), None, None
+
+
+class ConvTranspose2x2F32(torch.autograd.Function):
+    """nn.ConvTranspose2d(C, C/2, 2, stride 2) + F.pad in fp32 / TF32 training: the 1x1 convolution to 4*Cout
+    channels as one 3xTF32 launch (bias in its epilogue) and the fp32 pixel shuffle; backward: the shuffle's
+    transpose with the bias gradient, the hi/lo bf16 weight gradient and one 3xTF32 data-gradient launch."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias, out_h, out_w):
+        a = nhwc_view(x)
+        cin, cout = weight.shape[0], weight.shape[1]
+        w1, scale4, shift4 = pack_convt_weight(weight, bias)
+        split = split_tf32(a)
+        t = conv_packed(split, split[..., :cin], _pack3(w1), 4 * cout, 1, scale4, shift4, exact=True)
+        ctx.save_for_backward(a, w1)
+        ctx.meta = (weight.shape, bias is not None)
+        return nchw(shuffle2x2(t, cout, out_h, out_w))
+
+    @staticmethod
+    def backward(ctx, dout):
+        a, w1 = ctx.saved_tensors
+        wshape, has_bias = ctx.meta
+        need_x, need_w, need_b = ctx.needs_input_grad[:3]
+        dt, db = shuffle2x2_bwd(nhwc_view(dout), a.shape[1], a.shape[2], want_bias=has_bias and need_b)
+        gw = convt_weight_grad(a, dt, wshape) if need_w else None
+        dx = nchw(conv3(dt, None, w1, dgrad=True)) if need_x else None
+        return dx, gw, db, None, None
 
 
 class AttentionGateF32(torch.autograd.Function):

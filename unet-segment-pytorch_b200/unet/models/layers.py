@@ -94,7 +94,7 @@ class Up(nn.Module):
     def _upsampled(self, x1, skip):
         if fp32.active():
             if isinstance(self.up, nn.ConvTranspose2d):
-                raise NotImplementedError("TF32 mode supports bilinear=True only")
+                return fp32.conv_transpose2x2(self.up, x1, skip.shape[2], skip.shape[3])
             return fp32.upsample(x1, skip.shape[2], skip.shape[3])
         if isinstance(self.up, nn.ConvTranspose2d):
             return ops.conv_transpose2x2(x1, self.up.weight, self.up.bias, skip.shape[2], skip.shape[3])
