@@ -134,7 +134,7 @@ int ub2_bn_bwd_apply(const void* dA, int ld_da, const void* dP, int ld_dp, const
 
 /* nn.Upsample(scale_factor=2, bilinear, align_corners=True) + F.pad to the skip size
  * (layers.py:78, :98-102, :212, :247-251): (hin,win) -> (hu,wu) placed centred in (Ho,Wo). */
-int ub2_upsample_fwd(const void* in, int ld_in, void* out, int ld_out, int N, int hin, int win, int hu,
+int ub2_upsample_fwd(const void* src, int ld_src, void* out, int ld_out, int N, int hin, int win, int hu,
                      int wu, int Ho, int Wo, int C, void* stream);
 /* Its transpose in gather form (deterministic; ATen's backward uses atomics). */
 int ub2_upsample_bwd(const void* dout, int ld_dout, void* din, int ld_din, int accumulate, int N,
@@ -162,7 +162,7 @@ int ub2_convt_wgrad_reduce(const float* partial, int splits, int Cin, int Cout, 
 /* F.interpolate(x, size, mode='bilinear', align_corners=True) of the deep-supervision logits
  * (unet/models/unet.py:206-208) and its transpose in gather form (deterministic): fp32 NCHW,
  * planes = N * channels, (hin,win) -> (Ho,Wo), any scale. */
-int ub2_resize_planes_fwd(const float* in, float* out, int planes, int hin, int win, int Ho, int Wo, void* stream);
+int ub2_resize_planes_fwd(const float* src, float* out, int planes, int hin, int win, int Ho, int Wo, void* stream);
 int ub2_resize_planes_bwd(const float* dout, float* din, int planes, int hin, int win, int Ho, int Wo,
                           void* stream);
 
@@ -279,8 +279,8 @@ int ub2_f32_pack_weight(const float* w, float* out, int Cout, int Cin, int taps,
 /* first conv + folded BN + ReLU: x fp32 NCHW -> out fp32 NHWC (layers.py:32-34, Cin = n_channels) */
 int ub2_f32_conv_in(const float* x, const float* w, const float* scale, const float* shift, float* out, int N,
                     int Cin, int H, int W, int Cout, void* stream);
-int ub2_f32_maxpool(const float* in, float* out, int N, int H, int W, int C, void* stream);          /* layers.py:56 */
-int ub2_f32_upsample(const float* in, float* out, int N, int hin, int win, int hu, int wu, int Ho, int Wo, int C,
+int ub2_f32_maxpool(const float* src, float* out, int N, int H, int W, int C, void* stream);          /* layers.py:56 */
+int ub2_f32_upsample(const float* src, float* out, int N, int hin, int win, int hu, int wu, int Ho, int Wo, int C,
                      void* stream);                                                              /* layers.py:78,98-102 */
 /* AttentionGate.forward after the two 1x1 projections q = W_g g (low resolution), xp = W_x x
  * (layers.py:183-192): out = x * sigmoid(BN_psi(w_psi . relu(BN_g(up q) + BN_x(xp)))) */
@@ -376,7 +376,7 @@ int ub2_f32_conv_in_dgrad(const float* dy, int ld_dy, const float* w, float* dx,
 int ub2_f32_split_bf16(const float* x, void* hi, void* lo, long long n, void* stream);
 int ub2_f32_split_tf32(const float* x0, int ld0, int C0, const float* x1, int ld1, int C1, float* out, long long pixels, void* stream);
 int ub2_f32_pack_weight3(const float* w, float* out, int Cout, int Cin, int taps, int dgrad, void* stream);
-int ub2_f32_upsample_fwd(const float* in, float* out, int N, int hin, int win, int hu, int wu, int Ho, int Wo, int C, void* stream);
+int ub2_f32_upsample_fwd(const float* src, float* out, int N, int hin, int win, int hu, int wu, int Ho, int Wo, int C, void* stream);
 /* ConvTranspose2d(C, C/2, 2, stride 2) + F.pad in fp32 (layers.py:81, :98-102, :217-221): the ub2_shuffle2x2_* pixel
  * shuffle, its transpose and the bias gradient on fp32 tensors.  t / dt: (N,h,w,4*C) with channel stride ld_t / ld_dt
  * >= 4*C; out / dout: (N,Ho,Wo,C) with stride ld_out / ld_dout >= C (dout may be a channel slice of a wider

@@ -39,6 +39,80 @@ def test_header_declares_every_exported_symbol():
     assert exported == _declared_symbols()
 
 
+def test_every_entry_point_is_typed_from_the_header():
+    """lib() sets restype and argtypes of every prototype from include/unetb200.h, once: SIGNATURES is that
+    table and the loaded functions carry it."""
+    from unet import _C
+    lib = _C.lib()
+    assert sorted(_C.SIGNATURES) == _declared_symbols() and len(_C.SIGNATURES) == 89
+    for name, params in _C.SIGNATURES.items():
+        fn = getattr(lib, name)
+        assert fn.restype is ctypes.c_int, name
+        assert fn.argtypes == [t for _, t in params], name
+        assert all(p.isidentifier() and p not in ("in", "from", "lambda") for p, _ in params), name
+    assert _C.SIGNATURES["ub2_version"] == []
+    assert _C.SIGNATURES["ub2_seg_stats_blocks"] == [("N", ctypes.c_int), ("HW", ctypes.c_longlong)]
+    assert [t for _, t in _C.SIGNATURES["ub2_bn_finalize"]][3::7] == [ctypes.c_double, ctypes.c_float]
+    assert _C.SIGNATURES["ub2_conv_fwd"][-1] == ("stream", ctypes.c_void_p)
+
+
+def test_wrongly_typed_arguments_raise_before_the_call():
+    """With argtypes from the header a float for an int, or for a pointer, is refused by ctypes (ArgumentError)
+    instead of reaching C as garbage; a refused _C.call counts no launch."""
+    from unet import _C
+    lib = _C.lib()
+    assert lib.ub2_outc_rows(4, 64, 64, 64) > 0
+    with pytest.raises(ctypes.ArgumentError):
+        lib.ub2_outc_rows(4.0, 64, 64, 64)
+    with pytest.raises(ctypes.ArgumentError):
+        lib.ub2_f32_channel_rows(4096, 16.0)
+    with pytest.raises(ctypes.ArgumentError):
+        lib.ub2_resize_planes_fwd(0.5, None, 1, 1, 1, 1, 1, None)
+    with pytest.raises(TypeError):
+        lib.ub2_outc_rows(4, 64, 64)
+    launches = _C.LAUNCHES
+    with pytest.raises(ctypes.ArgumentError):
+        _C.call("ub2_f32_scalar_stats", None, 64.0, None, 1, None)
+    assert _C.LAUNCHES == launches
+
+
+@pytest.mark.parametrize("decl,error", [
+    ("int ub2_f(float* x, short n, void* stream);", "unknown parameter type"),
+    ("int ub2_f(const float*, int n);", "unnamed parameter"),
+    ("int ub2_f(int);", "unnamed parameter"),
+    ("long ub2_f(int n);", "not an int-returning prototype"),
+    ("int ub2_f(int n); int ub2_f(int m);", "declared twice"),
+])
+def test_header_parser_refuses_what_it_cannot_type(tmp_path, decl, error):
+    from unet import _C
+    hdr = tmp_path / "unetb200.h"
+    hdr.write_text("/* int ub2_comment(void); */\nint ub2_ok(const long long* p, long long n, double d);\n" + decl + "\n")
+    with pytest.raises(RuntimeError, match=error):
+        _C._parse_header(str(hdr))
+    hdr.write_text("/* int ub2_comment(void); */\nint ub2_ok(const long long* p, long long n, double d);\n")
+    assert _C._parse_header(str(hdr)) == {"ub2_ok": [("p", ctypes.c_void_p), ("n", ctypes.c_longlong), ("d", ctypes.c_double)]}
+    with pytest.raises(RuntimeError, match="missing.h"):
+        _C._parse_header(str(tmp_path / "missing.h"))
+
+
+def test_only_kernels_py_launches():
+    """Every launch goes through a wrapper of unet/kernels.py: no other module of the package calls _C.call."""
+    import ast
+    pkg = os.path.join(ROOT, "unet-segment-pytorch_b200", "unet")
+    callers = set()
+    for dirpath, _, files in os.walk(pkg):
+        for f in files:
+            if f.endswith(".py"):
+                path = os.path.join(dirpath, f)
+                with open(path) as fh:
+                    tree = ast.parse(fh.read(), path)
+                for node in ast.walk(tree):
+                    if (isinstance(node, ast.Call) and isinstance(node.func, ast.Attribute) and node.func.attr == "call"
+                            and isinstance(node.func.value, ast.Name) and node.func.value.id == "_C"):
+                        callers.add(os.path.relpath(path, pkg))
+    assert callers == {"kernels.py"}
+
+
 def test_state_dict_layout_and_default_init_match_reference():
     from unet.models import AttentionUNet, UNet
     for attention, kw in ((True, {}), (False, {}), (True, {"deep_supervision": True}), (True, {"bilinear": False})):
@@ -149,7 +223,6 @@ def test_workspace_queries_and_argument_errors_on_the_host():
     unsupported arguments before touching the device."""
     from unet import _C
     lib = _C.lib()
-    lib.ub2_seg_stats_blocks.argtypes = [ctypes.c_int, ctypes.c_longlong]
     assert lib.ub2_adamw_chunk_elems() == 16384
     good = (4, 512, 512, 64)
     queries = [lib.ub2_outc_rows, lib.ub2_conv_in_rows, lib.ub2_gate_rows, lib.ub2_gate_strip_rows,
@@ -160,9 +233,8 @@ def test_workspace_queries_and_argument_errors_on_the_host():
             assert q(*bad) == -1, bad
     assert lib.ub2_seg_stats_blocks(4, 512 * 512) > 0
     assert lib.ub2_seg_stats_blocks(0, 512 * 512) == -1 and lib.ub2_seg_stats_blocks(2, 0) == -1
-    f = ctypes.c_float
-    assert lib.ub2_prepare_batch(None, None, None, 1, 8, 8, f(0.5), f(0.5), None, None, None) == -1
-    assert lib.ub2_predict_mask(None, 1, 2, ctypes.c_longlong(64), f(0.5), None, None, None) == -1
+    assert lib.ub2_prepare_batch(None, None, None, 1, 8, 8, 0.5, 0.5, None, None, None) == -1
+    assert lib.ub2_predict_mask(None, 1, 2, 64, 0.5, None, None, None) == -1
     assert lib.ub2_resize_planes_fwd(None, None, 0, 1, 1, 1, 1, None) == -1
     assert lib.ub2_resize_planes_bwd(None, None, 2, 0, 1, 1, 1, None) == -1
 

@@ -13,38 +13,24 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 CHILD = r'''
-import ctypes, re, sys
-root = sys.argv[1]
-sys.path.insert(0, root + "/unet-segment-pytorch_b200")
+import ctypes, sys
+sys.path.insert(0, sys.argv[1] + "/unet-segment-pytorch_b200")
 from unet import _C
 lib = _C.lib()
-hdr = re.sub(r"/\*.*?\*/", "", open(root + "/include/unetb200.h").read(), flags=re.S)
-protos = re.findall(r"\bint\s+(ub2_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", hdr)
-def kind(arg):
-    a = arg.strip()
-    if a in ("void", ""): return None
-    if "*" in a: return "p"
-    if a.startswith("float"): return "f"
-    if a.startswith("double"): return "d"
-    if a.startswith("long long") or a.startswith("size_t"): return "q"
-    return "i"
-def make(k, v):
-    return {"p": ctypes.c_void_p(0), "f": ctypes.c_float(0.5), "d": ctypes.c_double(1.0),
-            "q": ctypes.c_longlong(v), "i": ctypes.c_int(v)}[k]
+FIXED = {ctypes.c_void_p: None, ctypes.c_float: 0.5, ctypes.c_double: 1.0}   # NULL pointers; integers vary
 calls = 0
-for name, args in protos:
-    kinds = [k for k in (kind(a) for a in args.split(",")) if k]
-    if not kinds or name == "ub2_set_conv_mode":
+for name, args in _C.SIGNATURES.items():
+    if not args or name == "ub2_set_conv_mode":
         continue
-    fn = getattr(lib, name); fn.restype = ctypes.c_int
-    ints = [i for i, k in enumerate(kinds) if k in "iq"]
+    fn = getattr(lib, name)
+    ints = [i for i, (_, t) in enumerate(args) if t not in FIXED]
     for base in (8, 16, 64):
         for z in [None] + ints:
             for zv in (0, -3):
-                vals = [base] * len(kinds)
+                vals = [base] * len(args)
                 if z is not None: vals[z] = zv
                 print(name, vals, flush=True)
-                fn(*[make(k, v) for k, v in zip(kinds, vals)])
+                fn(*[FIXED.get(t, v) for (_, t), v in zip(args, vals)])
                 calls += 1
                 if z is None: break
 print("CALLS", calls, flush=True)

@@ -52,20 +52,8 @@ from unet import _C
 lib = _C.lib()
 P = 1 << 20                      # a 16-byte-aligned fake device address: the calls below must never use it
 Q = P + 4                        # 4-byte aligned only
-p, i = "p", "i"
-T = {p: ctypes.c_void_p, i: ctypes.c_int}
-SIG = {
- "ub2_f32_shuffle2x2_fwd": "t:p ld_t:i out:p ld_out:i N:i h:i w:i C:i Ho:i Wo:i s:p",
- "ub2_f32_shuffle2x2_bwd": "dout:p ld_dout:i dt:p ld_dt:i partials:p rows:i dbias:p N:i h:i w:i C:i Ho:i Wo:i s:p",
- "ub2_f32_pack_convt_weight": "w:p bias:p fwd:p scale4:p shift4:p Cin:i Cout:i s:p",
-}
-SIG = {k: [tuple(a.split(":")) for a in v.split()] for k, v in SIG.items()}
-for name, args in SIG.items():
-    fn = getattr(lib, name)
-    fn.restype = ctypes.c_int
-    fn.argtypes = [T[t] for _, t in args]
-lib.ub2_f32_shuffle2x2_rows.restype = ctypes.c_int
-lib.ub2_f32_shuffle2x2_rows.argtypes = [ctypes.c_int] * 6
+# the entry points under test, with their parameters as include/unetb200.h declares them
+SIG = {name: _C.SIGNATURES[name] for name in ("ub2_f32_shuffle2x2_fwd", "ub2_f32_shuffle2x2_bwd", "ub2_f32_pack_convt_weight")}
 rows = lambda N=2, h=4, w=4, C=16, Ho=8, Wo=8: lib.ub2_f32_shuffle2x2_rows(N, h, w, C, Ho, Wo)
 R = rows()
 assert R > 0 and rows(C=1024) > 0 and rows(N=1, h=1, w=1, C=4, Ho=2, Wo=2) > 0
@@ -78,11 +66,11 @@ BASE = {
 def call(name, **kw):
     vals = []
     for a, t in SIG[name]:
-        if a == "s":
+        if a == "stream":
             vals.append(None)
         elif a in kw:
             vals.append(kw[a])
-        elif t == "p":
+        elif t is ctypes.c_void_p:
             vals.append(P)
         else:
             vals.append(BASE[name][a])

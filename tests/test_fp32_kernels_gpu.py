@@ -25,7 +25,6 @@ Not covered on purpose: NaN inputs.  The ReLU and max-pool kernels use ``fmaxf``
 The host-side argument checks (no ``gpu`` mark) run every entry point in a child process without a device: bad
 arguments must come back as their negative UB2_ERR code, valid ones — including every NULL the modules pass — as a
 CUDA error, which proves they got past the checks."""
-import ctypes
 import math
 import os
 import subprocess
@@ -62,10 +61,6 @@ def _p(t):
 
 def _s():
     return _C().stream()
-
-
-def _ll(v):
-    return ctypes.c_longlong(int(v))
 
 
 def _call(name, *args):
@@ -160,44 +155,13 @@ from unet import _C
 lib = _C.lib()
 P = 1 << 20                      # a 16-byte-aligned fake device address: the calls below must never use it
 Q = P + 4                        # 4-byte aligned only
-p, i, q, f, d = "p", "i", "q", "f", "d"
-T = {p: ctypes.c_void_p, i: ctypes.c_int, q: ctypes.c_longlong, f: ctypes.c_float, d: ctypes.c_double}
-SIG = {
- "ub2_f32_channel_stats": "x:p ld:i pixels:q C:i partials:p rows:i s:p",
- "ub2_f32_scalar_stats": "x:p n:q partials:p rows:i s:p",
- "ub2_f32_affine_act": "y:p scale:p shift:p out:p pixels:q C:i relu:i s:p",
- "ub2_f32_maxpool_idx": "a:p p:p idx:p N:i H:i W:i C:i s:p",
- "ub2_f32_act_bwd_reduce": "dA:p ld_da:i dP:p idx:p y:p scale:p shift:p partials:p rows:i N:i H:i W:i C:i relu:i s:p",
- "ub2_f32_act_bwd_apply": "dA:p ld_da:i dP:p idx:p y:p scale:p shift:p coef:p dy:p N:i H:i W:i C:i relu:i s:p",
- "ub2_f32_upsample_bwd": "dout:p ld:i din:p N:i hin:i win:i hu:i wu:i Ho:i Wo:i C:i s:p",
- "ub2_f32_gate_psi": "u:p xp:p sg:p hg:p sx:p hx:p wpsi:p psi:p pixels:q Ci:i s:p",
- "ub2_f32_gate_apply": "psi:p spsi:p hpsi:p x:p out:p a_out:p pixels:q Cx:i s:p",
- "ub2_f32_gate_bwd_a": "dout:p ld:i x:p a:p psi:p dx:p dpsin:p partials:p rows:i pixels:q Cx:i s:p",
- "ub2_f32_gate_bwd_s": "dpsin:p psi:p coef:p u:p xp:p sg:p hg:p sx:p hx:p wpsi:p ds:p partials:p rows:i pixels:q Ci:i s:p",
- "ub2_f32_gate_bwd_xg": "ds:p xp:p u:p coef:p dxp:p du:p pixels:q Ci:i s:p",
- "ub2_f32_outc_bwd": "dl:p a:p w:p da:p partials:p rows:i dw:p db:p N:i H:i W:i C:i K:i s:p",
- "ub2_f32_conv_in_raw": "x:p w:p out:p N:i Cin:i H:i W:i Cout:i s:p",
- "ub2_f32_conv_in_wgrad": "x:p dy:p partials:p rows:i grad:p N:i Cin:i H:i W:i Cout:i s:p",
- "ub2_f32_split_bf16": "x:p hi:p lo:p n:q s:p",
- "ub2_f32_split_tf32": "x0:p ld0:i C0:i x1:p ld1:i C1:i out:p pixels:q s:p",
- "ub2_f32_pack_weight3": "w:p out:p Cout:i Cin:i taps:i dgrad:i s:p",
- "ub2_f32_upsample_fwd": "inp:p out:p N:i hin:i win:i hu:i wu:i Ho:i Wo:i C:i s:p",
- "ub2_f32_pack_weight": "w:p out:p Cout:i Cin:i taps:i s:p",
- "ub2_f32_conv_in": "x:p w:p scale:p shift:p out:p N:i Cin:i H:i W:i Cout:i s:p",
- "ub2_f32_maxpool": "inp:p out:p N:i H:i W:i C:i s:p",
- "ub2_f32_upsample": "inp:p out:p N:i hin:i win:i hu:i wu:i Ho:i Wo:i C:i s:p",
- "ub2_f32_gate": "q:p xp:p x:p sg:p hg:p sx:p hx:p wpsi:p spsi:p hpsi:p out:p N:i hin:i win:i H:i W:i Ci:i Cx:i s:p",
- "ub2_f32_outc": "a:p w:p bias:p logits:p N:i H:i W:i C:i K:i s:p",
-}
-SIG = {k: [tuple(a.split(":")) for a in v.split()] for k, v in SIG.items()}
-for name, args in SIG.items():
-    fn = getattr(lib, name)
-    fn.restype = ctypes.c_int
-    fn.argtypes = [T[t] for _, t in args]
-for name, args in (("ub2_f32_channel_rows", [q, i]), ("ub2_f32_scalar_rows", [q]), ("ub2_f32_gate_rows", [q]),
-                   ("ub2_f32_outc_rows", [i, i, i])):
-    getattr(lib, name).restype = ctypes.c_int
-    getattr(lib, name).argtypes = [T[t] for t in args]
+# the fp32 entry points under test, with their parameters as include/unetb200.h declares them
+SIG = {name: _C.SIGNATURES[name] for name in """
+ub2_f32_channel_stats ub2_f32_scalar_stats ub2_f32_affine_act ub2_f32_maxpool_idx ub2_f32_act_bwd_reduce
+ub2_f32_act_bwd_apply ub2_f32_upsample_bwd ub2_f32_gate_psi ub2_f32_gate_apply ub2_f32_gate_bwd_a
+ub2_f32_gate_bwd_s ub2_f32_gate_bwd_xg ub2_f32_outc_bwd ub2_f32_conv_in_raw ub2_f32_conv_in_wgrad
+ub2_f32_split_bf16 ub2_f32_split_tf32 ub2_f32_pack_weight3 ub2_f32_upsample_fwd ub2_f32_pack_weight
+ub2_f32_conv_in ub2_f32_maxpool ub2_f32_upsample ub2_f32_gate ub2_f32_outc""".split()}
 N, H, W, C = 2, 8, 8, 16
 pix = N * H * W
 chan = lib.ub2_f32_channel_rows(pix, C)
@@ -206,7 +170,7 @@ outcr = lib.ub2_f32_outc_rows(N, H, W)
 scal = lib.ub2_f32_scalar_rows(pix)
 wg4 = lib.ub2_f32_channel_rows(pix, 4)
 assert min(chan, gater, outcr, scal, wg4) > 0
-# every pointer argument defaults to P, `s` (the stream) to NULL
+# every pointer argument defaults to P, the stream to NULL
 BASE = {
  "ub2_f32_channel_stats": dict(ld=C, pixels=pix, C=C, rows=chan),
  "ub2_f32_scalar_stats": dict(n=pix, rows=scal),
@@ -214,10 +178,10 @@ BASE = {
  "ub2_f32_maxpool_idx": dict(N=N, H=H, W=W, C=C),
  "ub2_f32_act_bwd_reduce": dict(ld_da=C, rows=chan, N=N, H=H, W=W, C=C, relu=1),
  "ub2_f32_act_bwd_apply": dict(ld_da=C, N=N, H=H, W=W, C=C, relu=1),
- "ub2_f32_upsample_bwd": dict(ld=C, N=N, hin=4, win=4, hu=8, wu=8, Ho=H, Wo=W, C=C),
+ "ub2_f32_upsample_bwd": dict(ld_dout=C, N=N, hin=4, win=4, hu=8, wu=8, Ho=H, Wo=W, C=C),
  "ub2_f32_gate_psi": dict(pixels=pix, Ci=C),
  "ub2_f32_gate_apply": dict(pixels=pix, Cx=C),
- "ub2_f32_gate_bwd_a": dict(ld=C, rows=gater, pixels=pix, Cx=C),
+ "ub2_f32_gate_bwd_a": dict(ld_do=C, rows=gater, pixels=pix, Cx=C),
  "ub2_f32_gate_bwd_s": dict(rows=gater, pixels=pix, Ci=C),
  "ub2_f32_gate_bwd_xg": dict(pixels=pix, Ci=C),
  "ub2_f32_outc_bwd": dict(rows=outcr, N=N, H=H, W=W, C=C, K=2),
@@ -236,12 +200,13 @@ BASE = {
 }
 def call(name, **kw):
     vals = []
+    assert set(kw) <= {a for a, _ in SIG[name]}, (name, kw)
     for a, t in SIG[name]:
-        if a == "s":
+        if a == "stream":
             vals.append(None)
         elif a in kw:
             vals.append(kw[a])
-        elif t == "p":
+        elif t is ctypes.c_void_p:
             vals.append(P)
         else:
             vals.append(BASE[name][a])
@@ -249,7 +214,7 @@ def call(name, **kw):
 S, A, WS = -1, -2, -3
 BAD = [
  # the cases that reached the device before these checks
- ("ub2_f32_upsample", dict(hin=0), S), ("ub2_f32_upsample", dict(hu=-2, Ho=-2), S), ("ub2_f32_upsample", dict(inp=None), S),
+ ("ub2_f32_upsample", dict(hin=0), S), ("ub2_f32_upsample", dict(hu=-2, Ho=-2), S), ("ub2_f32_upsample", dict(src=None), S),
  ("ub2_f32_gate", dict(hin=0), S), ("ub2_f32_gate", dict(H=0), S), ("ub2_f32_gate", dict(Ci=0), S), ("ub2_f32_gate", dict(q=None), S),
  ("ub2_f32_conv_in", dict(H=-1), S), ("ub2_f32_conv_in", dict(Cout=0), S), ("ub2_f32_conv_in", dict(Cout=-4), S),
  ("ub2_f32_maxpool", dict(C=0), S), ("ub2_f32_maxpool", dict(C=-4), S),
@@ -258,7 +223,7 @@ BAD = [
  ("ub2_f32_act_bwd_apply", dict(dA=None, idx=None), S),
  ("ub2_f32_channel_stats", dict(ld=8), S), ("ub2_f32_split_tf32", dict(ld0=8), S), ("ub2_f32_split_tf32", dict(ld1=8), S),
  ("ub2_f32_act_bwd_reduce", dict(ld_da=8), S), ("ub2_f32_act_bwd_apply", dict(ld_da=8), S),
- ("ub2_f32_gate_bwd_a", dict(ld=8), S), ("ub2_f32_upsample_bwd", dict(ld=8), S),
+ ("ub2_f32_gate_bwd_a", dict(ld_do=8), S), ("ub2_f32_upsample_bwd", dict(ld_dout=8), S),
  # counts
  ("ub2_f32_channel_stats", dict(pixels=0), S), ("ub2_f32_channel_stats", dict(C=6, ld=8), S),
  ("ub2_f32_channel_stats", dict(C=1028, ld=1028), S), ("ub2_f32_scalar_stats", dict(n=0), S),
@@ -276,7 +241,7 @@ BAD = [
  ("ub2_f32_upsample", dict(C=0), S),
  ("ub2_f32_gate_psi", dict(pixels=0), S), ("ub2_f32_gate_psi", dict(Ci=0), S), ("ub2_f32_gate_psi", dict(Ci=6), S),
  ("ub2_f32_gate_apply", dict(pixels=0), S), ("ub2_f32_gate_apply", dict(Cx=0), S),
- ("ub2_f32_gate_bwd_a", dict(Cx=0, ld=0), S), ("ub2_f32_gate_bwd_a", dict(pixels=0), S),
+ ("ub2_f32_gate_bwd_a", dict(Cx=0, ld_do=0), S), ("ub2_f32_gate_bwd_a", dict(pixels=0), S),
  ("ub2_f32_gate_bwd_s", dict(Ci=0), S), ("ub2_f32_gate_bwd_s", dict(Ci=516), S), ("ub2_f32_gate_bwd_s", dict(pixels=0), S),
  ("ub2_f32_gate_bwd_xg", dict(Ci=0), S), ("ub2_f32_gate_bwd_xg", dict(pixels=0), S),
  ("ub2_f32_outc_bwd", dict(K=0), S), ("ub2_f32_outc_bwd", dict(K=9), S), ("ub2_f32_outc_bwd", dict(C=0), S),
@@ -302,7 +267,7 @@ BAD = [
  ("ub2_f32_split_tf32", dict(x1=None), S),
  # strides and alignment
  ("ub2_f32_channel_stats", dict(ld=18), A), ("ub2_f32_act_bwd_reduce", dict(ld_da=18), A), ("ub2_f32_act_bwd_apply", dict(ld_da=18), A),
- ("ub2_f32_upsample_bwd", dict(ld=18), A), ("ub2_f32_gate_bwd_a", dict(ld=18), A), ("ub2_f32_split_tf32", dict(ld0=18), A),
+ ("ub2_f32_upsample_bwd", dict(ld_dout=18), A), ("ub2_f32_gate_bwd_a", dict(ld_do=18), A), ("ub2_f32_split_tf32", dict(ld0=18), A),
  ("ub2_f32_split_tf32", dict(ld1=18), A),
  ("ub2_f32_channel_stats", dict(x=Q), A), ("ub2_f32_affine_act", dict(y=Q), A), ("ub2_f32_affine_act", dict(scale=Q), A),
  ("ub2_f32_affine_act", dict(out=Q), A), ("ub2_f32_maxpool_idx", dict(a=Q), A), ("ub2_f32_maxpool_idx", dict(idx=P + 2), A),
@@ -312,7 +277,7 @@ BAD = [
  ("ub2_f32_gate_bwd_s", dict(ds=Q), A), ("ub2_f32_gate_bwd_xg", dict(coef=Q), A), ("ub2_f32_outc_bwd", dict(a=Q), A),
  ("ub2_f32_outc_bwd", dict(da=Q), A), ("ub2_f32_conv_in_raw", dict(out=Q), A), ("ub2_f32_conv_in_wgrad", dict(dy=Q), A),
  ("ub2_f32_split_bf16", dict(x=Q), A), ("ub2_f32_split_tf32", dict(x1=Q), A), ("ub2_f32_split_tf32", dict(out=Q), A),
- ("ub2_f32_upsample_fwd", dict(inp=Q), A), ("ub2_f32_conv_in", dict(out=Q), A), ("ub2_f32_maxpool", dict(out=Q), A),
+ ("ub2_f32_upsample_fwd", dict(src=Q), A), ("ub2_f32_conv_in", dict(out=Q), A), ("ub2_f32_maxpool", dict(out=Q), A),
  ("ub2_f32_upsample", dict(out=Q), A), ("ub2_f32_gate", dict(q=Q), A), ("ub2_f32_gate", dict(x=Q), A), ("ub2_f32_outc", dict(a=Q), A),
  # workspace rows
  ("ub2_f32_channel_stats", dict(rows=chan + 1), WS), ("ub2_f32_scalar_stats", dict(rows=scal - 1), WS),
@@ -326,7 +291,7 @@ OPTIONAL = {"ub2_f32_act_bwd_reduce": {"dA", "dP"}, "ub2_f32_act_bwd_apply": {"d
             "ub2_f32_outc": {"bias"}}
 for name, args in SIG.items():
     for a, t in args:
-        if t == "p" and a != "s" and a not in OPTIONAL.get(name, ()):
+        if t is ctypes.c_void_p and a != "stream" and a not in OPTIONAL.get(name, ()):
             BAD.append((name, {a: None}, S))
 BAD.append(("ub2_f32_act_bwd_apply", dict(scale=None), S))       # relu = 1 reads scale and shift
 BAD.append(("ub2_f32_act_bwd_apply", dict(shift=None), S))
@@ -341,9 +306,9 @@ GOOD = [(name, {}) for name in SIG] + [
  ("ub2_f32_outc", dict(bias=None)),
  # edges that are valid
  ("ub2_f32_channel_stats", dict(ld=24)), ("ub2_f32_channel_stats", dict(C=1024, ld=1024, rows=lib.ub2_f32_channel_rows(pix, 1024))),
- ("ub2_f32_act_bwd_reduce", dict(ld_da=24)), ("ub2_f32_upsample_bwd", dict(ld=20)), ("ub2_f32_upsample_bwd", dict(hin=1, hu=1, Ho=1)),
+ ("ub2_f32_act_bwd_reduce", dict(ld_da=24)), ("ub2_f32_upsample_bwd", dict(ld_dout=20)), ("ub2_f32_upsample_bwd", dict(hin=1, hu=1, Ho=1)),
  ("ub2_f32_upsample_bwd", dict(Ho=11, Wo=13)), ("ub2_f32_upsample_fwd", dict(hin=7, win=7, hu=16, wu=16, Ho=16, Wo=16)),
- ("ub2_f32_gate_bwd_a", dict(ld=20)), ("ub2_f32_gate_bwd_s", dict(Ci=388)), ("ub2_f32_gate_bwd_s", dict(Ci=512)),
+ ("ub2_f32_gate_bwd_a", dict(ld_do=20)), ("ub2_f32_gate_bwd_s", dict(Ci=388)), ("ub2_f32_gate_bwd_s", dict(Ci=512)),
  ("ub2_f32_outc_bwd", dict(C=188, K=8)), ("ub2_f32_outc_bwd", dict(K=1)),
  ("ub2_f32_conv_in_raw", dict(Cin=7, Cout=1024)), ("ub2_f32_conv_in_wgrad", dict(Cin=7, Cout=4, rows=wg4)),
  ("ub2_f32_split_tf32", dict(ld0=24, ld1=20)), ("ub2_f32_pack_weight3", dict(taps=1, dgrad=1)),
@@ -377,11 +342,11 @@ def _stats_case(pixels, C, ld, seed, far_mean=False):
     if far_mean:
         full[:, 1] = _randn((pixels,), g, 1.0, 100.0)      # mean = 100 std: the one-pass variance's hard case
     x = Guarded((pixels, ld), fill=full.cuda()).t
-    rows = _rows("ub2_f32_channel_rows", _ll(pixels), C)
+    rows = _rows("ub2_f32_channel_rows", pixels, C)
     parts = []
     for _ in range(2):
         pg = Guarded((rows, 2, C), F64)
-        _call("ub2_f32_channel_stats", _p(x), ld, _ll(pixels), C, _p(pg.t), rows, _s())
+        _call("ub2_f32_channel_stats", _p(x), ld, pixels, C, _p(pg.t), rows, _s())
         assert pg.ok(), ("partials bands", pixels, C, ld)
         parts.append(pg.t.clone())
     assert torch.equal(parts[0], parts[1]), ("not repeatable", pixels, C)
@@ -411,8 +376,8 @@ def test_channel_stats_and_bn_finalize(C):
         nbt = torch.tensor([5], dtype=torch.int64, device="cuda")
         mom, eps = 0.1, 1e-5
         out = Guarded((4, C))
-        _call("ub2_bn_finalize", _p(part), part.shape[0], C, ctypes.c_double(float(pixels)), _p(gamma.cuda()),
-              _p(beta.cuda()), _p(rm), _p(rv), _p(nbt), ctypes.c_float(mom), ctypes.c_float(eps), _p(out.t[0]),
+        _call("ub2_bn_finalize", _p(part), part.shape[0], C, pixels, _p(gamma.cuda()),
+              _p(beta.cuda()), _p(rm), _p(rv), _p(nbt), mom, eps, _p(out.t[0]),
               _p(out.t[1]), _p(out.t[2]), _p(out.t[3]), _s())
         assert out.ok()
         s = _folded(part)
@@ -443,7 +408,7 @@ def test_channel_stats_and_bn_finalize(C):
             log[f"variance mean=100std p{pixels} rel"] = float(err[1] / ref_var[1])
         # eval coefficients: 1/sqrtf(rv + eps) (3 roundings), * gamma, beta - rm*g*inv (3 more)
         ec = Guarded((2, C))
-        _call("ub2_bn_eval_coeffs", _p(gamma.cuda()), _p(beta.cuda()), _p(rm), _p(rv), ctypes.c_float(eps), C,
+        _call("ub2_bn_eval_coeffs", _p(gamma.cuda()), _p(beta.cuda()), _p(rm), _p(rv), eps, C,
               _p(ec.t[0]), _p(ec.t[1]), _s())
         assert ec.ok()
         rmd, rvd = rm.cpu().double(), rv.cpu().double()
@@ -460,11 +425,11 @@ def test_scalar_stats():
     for n in (1, 7, 2 * 33 * 17, 300001):
         g = _gen(n)
         x = Guarded((n,), fill=_randn((n,), g, 2.0, 0.5).cuda()).t
-        rows = _rows("ub2_f32_scalar_rows", _ll(n))
+        rows = _rows("ub2_f32_scalar_rows", n)
         parts = []
         for _ in range(2):
             pg = Guarded((rows, 2, 1), F64)
-            _call("ub2_f32_scalar_stats", _p(x), _ll(n), _p(pg.t), rows, _s())
+            _call("ub2_f32_scalar_stats", _p(x), n, _p(pg.t), rows, _s())
             assert pg.ok()
             parts.append(pg.t.clone())
         assert torch.equal(parts[0], parts[1])
@@ -486,7 +451,7 @@ def test_affine_act(C, relu):
     y = _randn((pixels, C), g)
     sc, sh = _randn((C,), g), _randn((C,), g)
     out = Guarded((pixels, C))
-    _call("ub2_f32_affine_act", _p(y.cuda()), _p(sc.cuda()), _p(sh.cuda()), _p(out.t), _ll(pixels), C, relu, _s())
+    _call("ub2_f32_affine_act", _p(y.cuda()), _p(sc.cuda()), _p(sh.cuda()), _p(out.t), pixels, C, relu, _s())
     assert out.ok()
     z = y.double() * sc.double() + sh.double()
     ref = z.clamp_min(0) if relu else z
@@ -547,7 +512,7 @@ def _routed(dA, dP, idx, N, H, W, C):
 def _act_bwd(dA_full, ld_da, dP, idx, y, sc, sh, N, H, W, C, relu, mean, invstd, gamma, frozen, dgamma0, dbeta0):
     pixels = N * H * W
     dA = dA_full[..., :C] if dA_full is not None else None
-    rows = _rows("ub2_f32_channel_rows", _ll(pixels), C)
+    rows = _rows("ub2_f32_channel_rows", pixels, C)
     dev = {k: (v.cuda() if v is not None else None) for k, v in dict(dA=dA_full, dP=dP, idx=idx, y=y, sc=sc, sh=sh).items()}
     dA_ptr = _p(dev["dA"]) if dA is not None else _p(None)
     parts = []
@@ -560,7 +525,7 @@ def _act_bwd(dA_full, ld_da, dP, idx, y, sc, sh, N, H, W, C, relu, mean, invstd,
     assert torch.equal(parts[0], parts[1])
     dgamma, dbeta = dgamma0.clone().cuda(), dbeta0.clone().cuda()
     coef = Guarded((3, C))
-    _call("ub2_bn_bwd_finalize", _p(parts[0]), rows, C, ctypes.c_double(float(pixels)), _p(gamma.cuda()), _p(mean.cuda()),
+    _call("ub2_bn_bwd_finalize", _p(parts[0]), rows, C, pixels, _p(gamma.cuda()), _p(mean.cuda()),
           _p(invstd.cuda()), int(frozen), _p(dgamma), _p(dbeta), _p(coef.t), _s())
     dy = Guarded((N, H, W, C))
     _call("ub2_f32_act_bwd_apply", dA_ptr, ld_da if dA is not None else 0, _p(dev["dP"]), _p(dev["idx"]), _p(dev["y"]),
@@ -763,7 +728,7 @@ def test_gate_training_passes(Ci):
     log = {}
     # psi
     psi = Guarded((pixels,))
-    _call("ub2_f32_gate_psi", _p(ud), _p(xpd), _p(sgd), _p(hgd), _p(sxd), _p(hxd), _p(wd), _p(psi.t), _ll(pixels), Ci, _s())
+    _call("ub2_f32_gate_psi", _p(ud), _p(xpd), _p(sgd), _p(hgd), _p(sxd), _p(hxd), _p(wd), _p(psi.t), pixels, Ci, _s())
     assert psi.ok()
     t32, tt = _gate_t(u, xp, sg, hg, sx, hx)
     psi_ref = (wpsi.double() * t32.double().clamp_min(0)).sum(1)
@@ -772,8 +737,8 @@ def test_gate_training_passes(Ci):
     # apply, with and without a_out
     spsi, hpsi = torch.tensor([0.7]), torch.tensor([-0.2])
     out, a_out, out2 = Guarded((pixels, Cx)), Guarded((pixels,)), Guarded((pixels, Cx))
-    _call("ub2_f32_gate_apply", _p(psi.t), _p(spsi.cuda()), _p(hpsi.cuda()), _p(xd), _p(out.t), _p(a_out.t), _ll(pixels), Cx, _s())
-    _call("ub2_f32_gate_apply", _p(psi.t), _p(spsi.cuda()), _p(hpsi.cuda()), _p(xd), _p(out2.t), _p(None), _ll(pixels), Cx, _s())
+    _call("ub2_f32_gate_apply", _p(psi.t), _p(spsi.cuda()), _p(hpsi.cuda()), _p(xd), _p(out.t), _p(a_out.t), pixels, Cx, _s())
+    _call("ub2_f32_gate_apply", _p(psi.t), _p(spsi.cuda()), _p(hpsi.cuda()), _p(xd), _p(out2.t), _p(None), pixels, Cx, _s())
     assert out.ok() and a_out.ok() and out2.ok()
     assert torch.equal(_bits(out.t), _bits(out2.t))
     psi32 = psi.t.cpu()
@@ -786,13 +751,13 @@ def test_gate_training_passes(Ci):
     a32 = a_out.t.cpu()
     dfull = _randn((pixels, ld_do), g)
     dout = dfull[:, :Cx]
-    rows = _rows("ub2_f32_gate_rows", _ll(pixels))
+    rows = _rows("ub2_f32_gate_rows", pixels)
     dx, dpsin = Guarded((pixels, Cx)), Guarded((pixels,))
     parts = []
     for _ in range(2):
         pg = Guarded((rows, 2, 1), F64)
         _call("ub2_f32_gate_bwd_a", _p(dfull.cuda()), ld_do, _p(xd), _p(a_out.t), _p(psi.t), _p(dx.t), _p(dpsin.t), _p(pg.t), rows,
-              _ll(pixels), Cx, _s())
+              pixels, Cx, _s())
         assert pg.ok()
         parts.append(pg.t.clone())
     assert torch.equal(parts[0], parts[1]) and dx.ok() and dpsin.ok()
@@ -813,7 +778,7 @@ def test_gate_training_passes(Ci):
     mp, ip, gp = torch.tensor([0.1]), torch.tensor([1.3]), torch.tensor([0.7])
     dgp, dbp = torch.tensor([0.25]).cuda(), torch.tensor([-0.5]).cuda()
     coef_p = Guarded((3, 1))
-    _call("ub2_bn_bwd_finalize", _p(parts[0]), rows, 1, ctypes.c_double(float(pixels)), _p(gp.cuda()), _p(mp.cuda()), _p(ip.cuda()), 0,
+    _call("ub2_bn_bwd_finalize", _p(parts[0]), rows, 1, pixels, _p(gp.cuda()), _p(mp.cuda()), _p(ip.cuda()), 0,
           _p(dgp), _p(dbp), _p(coef_p.t), _s())
     assert coef_p.ok()
     dbr, dgr = s[0, 0], ip.double()[0] * (s[1, 0] - mp.double()[0] * s[0, 0])
@@ -832,7 +797,7 @@ def test_gate_training_passes(Ci):
     for _ in range(2):
         pg = Guarded((rows_s, 4, Ci), F64)
         _call("ub2_f32_gate_bwd_s", _p(dpsin.t), _p(psi.t), _p(coef_p.t), _p(ud), _p(xpd), _p(sgd), _p(hgd), _p(sxd), _p(hxd), _p(wd),
-              _p(ds.t), _p(pg.t), rows_s, _ll(pixels), Ci, _s())
+              _p(ds.t), _p(pg.t), rows_s, pixels, Ci, _s())
         assert pg.ok()
         parts2.append(pg.t.clone())
     assert torch.equal(parts2[0], parts2[1]) and ds.ok()
@@ -859,7 +824,7 @@ def test_gate_training_passes(Ci):
     t0 = _randn((5, Ci), g)
     targets = t0.clone().cuda()
     coef = Guarded((6, Ci))
-    _call("ub2_gate_bwd_finalize", _p(parts2[0]), rows_s, Ci, ctypes.c_double(float(pixels)), _p(gx.cuda()), _p(mx.cuda()),
+    _call("ub2_gate_bwd_finalize", _p(parts2[0]), rows_s, Ci, pixels, _p(gx.cuda()), _p(mx.cuda()),
           _p(ix.cuda()), _p(gg.cuda()), _p(mg.cuda()), _p(ig.cuda()), 0, _p(targets[0]), _p(targets[1]), _p(targets[2]),
           _p(targets[3]), _p(targets[4]), _p(coef.t), _s())
     assert coef.ok()
@@ -879,7 +844,7 @@ def test_gate_training_passes(Ci):
     log["gate_bwd_finalize"] = e_fin
     # backward xg
     dxp, du = Guarded((pixels, Ci)), Guarded((pixels, Ci))
-    _call("ub2_f32_gate_bwd_xg", _p(ds.t), _p(xpd), _p(ud), _p(coef.t), _p(dxp.t), _p(du.t), _ll(pixels), Ci, _s())
+    _call("ub2_f32_gate_bwd_xg", _p(ds.t), _p(xpd), _p(ud), _p(coef.t), _p(dxp.t), _p(du.t), pixels, Ci, _s())
     assert dxp.ok() and du.ok()
     c6 = coef.t.cpu().double()
     ds64 = ds.t.cpu().double()
@@ -997,7 +962,7 @@ def test_conv_in(Cin, Cout, N, H, W):
     log["eval"] = _within(ev.t.cpu(), evr, pre_t, 9 * Cin + 1, "conv_in eval", tf32=True)
     dy = _randn((N, H, W, Cout), g)
     g0 = _randn((Cout, Cin, 3, 3), g)
-    rows = _rows("ub2_f32_channel_rows", _ll(N * H * W), Cout)
+    rows = _rows("ub2_f32_channel_rows", N * H * W, Cout)
     grads, parts = [], []
     for _ in range(2):
         grad = Guarded((Cout, Cin, 3, 3), fill=g0.cuda())
@@ -1043,7 +1008,7 @@ def test_split_tf32(C0, ld0, C1, ld1):
     x1f = _with_denormals((pixels, ld1), g) if C1 else None
     C = C0 + C1
     out = Guarded((pixels, 2 * C))
-    _call("ub2_f32_split_tf32", _p(x0f.cuda()), ld0, C0, _p(x1f.cuda() if C1 else None), ld1, C1, _p(out.t), _ll(pixels), _s())
+    _call("ub2_f32_split_tf32", _p(x0f.cuda()), ld0, C0, _p(x1f.cuda() if C1 else None), ld1, C1, _p(out.t), pixels, _s())
     assert out.ok()
     v = torch.cat([x0f[:, :C0]] + ([x1f[:, :C1]] if C1 else []), 1)
     hi = _tf32(v)
@@ -1085,7 +1050,7 @@ def test_split_bf16():
     g = _gen(77)
     x = _with_denormals((4 * 9 * 5 * 12,), g)
     hi, lo = Guarded((x.numel(),), torch.bfloat16), Guarded((x.numel(),), torch.bfloat16)
-    _call("ub2_f32_split_bf16", _p(x.cuda()), _p(hi.t), _p(lo.t), _ll(x.numel()), _s())
+    _call("ub2_f32_split_bf16", _p(x.cuda()), _p(hi.t), _p(lo.t), x.numel(), _s())
     assert hi.ok() and lo.ok()
     rh = x.to(torch.bfloat16)
     rl = (x - rh.float()).to(torch.bfloat16)
@@ -1151,7 +1116,7 @@ def test_offsets_past_2_pow_31():
     sh = torch.randn(C, device="cuda", generator=gen)
     out = torch.empty_like(y)
     pixels = N * H * W
-    _call("ub2_f32_affine_act", _p(y), _p(sc), _p(sh), _p(out), _ll(pixels), C, 1, _s())
+    _call("ub2_f32_affine_act", _p(y), _p(sc), _p(sh), _p(out), pixels, C, 1, _s())
     p = torch.empty((N, H // 2, W // 2, C), device="cuda")
     idx = torch.empty((N, H // 2, W // 2, C), device="cuda", dtype=torch.uint8)
     _call("ub2_f32_maxpool_idx", _p(out), _p(p), _p(idx), N, H, W, C, _s())

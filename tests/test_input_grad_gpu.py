@@ -34,30 +34,30 @@ sys.path.insert(0, sys.argv[1] + "/unet-segment-pytorch_b200")
 from unet import _C
 lib = _C.lib()
 P = 1 << 20                      # a 16-byte-aligned fake device address: the calls below must never use it
-for name in ("ub2_conv_in_dgrad", "ub2_f32_conv_in_dgrad"):
-    getattr(lib, name).restype = ctypes.c_int
-    getattr(lib, name).argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_int] * 5 + [ctypes.c_void_p]
-def call(name, dy=P, ld=64, w=P, dx=P, N=2, Cin=1, H=8, W=8, Cout=64):
-    return getattr(lib, name)(dy, ld, w, dx, N, Cin, H, W, Cout, None)
+BASE = dict(dy=P, ld_dy=64, w=P, dx=P, N=2, Cin=1, H=8, W=8, Cout=64, stream=None)
+def call(name, **kw):
+    assert set(kw) <= set(BASE), kw
+    vals = dict(BASE, **kw)
+    return getattr(lib, name)(*[vals[a] for a, _ in _C.SIGNATURES[name]])
 bad = {
     "N=0": (dict(N=0), -1), "N<0": (dict(N=-3), -1), "H=0": (dict(H=0), -1), "W=0": (dict(W=0), -1),
-    "H<0": (dict(H=-1), -1), "W<0": (dict(W=-8), -1), "Cout=0": (dict(Cout=0, ld=8), -1),
+    "H<0": (dict(H=-1), -1), "W<0": (dict(W=-8), -1), "Cout=0": (dict(Cout=0, ld_dy=8), -1),
     "Cout<0": (dict(Cout=-8), -1), "Cin=0": (dict(Cin=0), -1), "Cin<0": (dict(Cin=-1), -1),
-    "ld<Cout": (dict(ld=32), -1), "dy NULL": (dict(dy=None), -1), "w NULL": (dict(w=None), -1),
+    "ld<Cout": (dict(ld_dy=32), -1), "dy NULL": (dict(dy=None), -1), "w NULL": (dict(w=None), -1),
     "dx NULL": (dict(dx=None), -1), "dx misaligned": (dict(dx=P + 2), -2), "w misaligned": (dict(w=P + 2), -2),
 }
-bf16 = dict(bad, **{"Cin>4": (dict(Cin=5), -1), "Cout%8": (dict(Cout=12, ld=16), -1), "ld%8": (dict(ld=68), -2),
-                    "Cout/8>256": (dict(Cout=2056, ld=2056), -1), "dy odd": (dict(dy=P + 1), -2),
+bf16 = dict(bad, **{"Cin>4": (dict(Cin=5), -1), "Cout%8": (dict(Cout=12, ld_dy=16), -1), "ld%8": (dict(ld_dy=68), -2),
+                    "Cout/8>256": (dict(Cout=2056, ld_dy=2056), -1), "dy odd": (dict(dy=P + 1), -2),
                     "N*H*W*Cin>=2e9": (dict(N=8000, H=512, W=512), -1),
-                    "smem>48KB": (dict(Cin=4, Cout=512, ld=512), -1)})
-f32 = dict(bad, **{"Cout%4": (dict(Cout=6, ld=8), -1), "ld%4": (dict(ld=66), -2), "dy misaligned": (dict(dy=P + 2), -2),
-                   "smem>48KB": (dict(Cin=15, Cout=128, ld=128), -1)})
+                    "smem>48KB": (dict(Cin=4, Cout=512, ld_dy=512), -1)})
+f32 = dict(bad, **{"Cout%4": (dict(Cout=6, ld_dy=8), -1), "ld%4": (dict(ld_dy=66), -2), "dy misaligned": (dict(dy=P + 2), -2),
+                   "smem>48KB": (dict(Cin=15, Cout=128, ld_dy=128), -1)})
 for name, cases in (("ub2_conv_in_dgrad", bf16), ("ub2_f32_conv_in_dgrad", f32)):
     for what, (kw, want) in cases.items():
         rc = call(name, **kw)
         print(name, what, rc, want, "OK" if rc == want else "WRONG", flush=True)
     # valid arguments pass the checks and only then fail for want of a device (a CUDA error code, > 0)
-    for kw in (dict(), dict(Cin=3, W=9), dict(Cin=4, Cout=16, ld=16) if name == "ub2_conv_in_dgrad" else dict(Cin=7, Cout=20, ld=20)):
+    for kw in (dict(), dict(Cin=3, W=9), dict(Cin=4, Cout=16, ld_dy=16) if name == "ub2_conv_in_dgrad" else dict(Cin=7, Cout=20, ld_dy=20)):
         rc = call(name, **kw)
         print(name, "valid", kw, rc, "positive", "OK" if rc > 0 else "WRONG", flush=True)
 print("DONE", flush=True)

@@ -3,8 +3,8 @@
     python tools/bench_fp32_convt.py [--out profiles/r04_bench_fp32_convt.json]     (on a B200)
 
 * kernel times of ub2_f32_shuffle2x2_fwd / _bwd (the latter with its bias gradient) at the four decoder levels of
-  AttentionUNet(1, 2, bilinear=False, 64) at 4 x 1 x 512^2: CUDA events over 200 back-to-back launches after
-  warm-up.  Bytes from shapes: t (N,h,w,4C) read + out (N,2h,2w,C) written, and the reverse; the bound is those
+  AttentionUNet(1, 2, bilinear=False, 64) at 4 x 1 x 512^2: CUDA events over 200 back-to-back calls of the
+  kernels.py wrappers the layer uses (so the backward includes the zero fill of its bias gradient) after warm-up.  Bytes from shapes: t (N,h,w,4C) read + out (N,2h,2w,C) written, and the reverse; the bound is those
   bytes at 6.55 TB/s (the copy bandwidth this project measured on a B200).  A level whose operands (in + out) fit
   the 126 MB L2 is marked L2-resident: back-to-back launches then read it from L2, not HBM;
 * the fp32-mode layer forward + backward (fp32.conv_transpose2x2 in training) against F.conv_transpose2d + F.pad
@@ -36,26 +36,19 @@ LEVELS = [("up1", 16 * BASE, HW // 16), ("up2", 8 * BASE, HW // 8), ("up3", 4 * 
 
 
 def shuffle_kernels():
-    from unet import _C
     from unet import kernels as K
-    from unet._C import ptr, stream
     out = []
     g = torch.Generator(device="cuda").manual_seed(0)
     for name, cin, h in LEVELS:
         c = cin // 2
         t = torch.randn((N, h, h, 4 * c), device="cuda", generator=g)
-        o = torch.empty((N, 2 * h, 2 * h, c), device="cuda")
-        dt = torch.empty_like(t)
-        rows = K._rows("ub2_f32_shuffle2x2_rows", N, h, h, c, 2 * h, 2 * h)
-        part = torch.empty((rows, c), device="cuda", dtype=torch.float64)
-        db = torch.zeros((c,), device="cuda")
+        o = K.f32_shuffle2x2(t, c, 2 * h, 2 * h)
 
         def fwd():
-            _C.call("ub2_f32_shuffle2x2_fwd", ptr(t), 4 * c, ptr(o), c, N, h, h, c, 2 * h, 2 * h, stream())
+            K.f32_shuffle2x2(t, c, 2 * h, 2 * h)
 
         def bwd():
-            _C.call("ub2_f32_shuffle2x2_bwd", ptr(o), c, ptr(dt), 4 * c, ptr(part), rows, ptr(db), N, h, h, c, 2 * h, 2 * h,
-                    stream())
+            K.f32_shuffle2x2_bwd(o, h, h)
 
         nbytes = (t.numel() + o.numel()) * 4
         bound_us = nbytes / (HBM_TBPS * 1e12) * 1e6
@@ -64,8 +57,8 @@ def shuffle_kernels():
             out.append({"level": name, "direction": direction, "shape_in": list(t.shape if direction == "fwd" else o.shape),
                         "us": us, "bytes": nbytes, "GBps": nbytes / us / 1e3, "hbm_bound_us": bound_us,
                         "frac_of_hbm_bound": bound_us / us, "l2_resident": nbytes <= L2_BYTES})
-        assert torch.equal(dt, t), "shuffle backward did not invert the forward"
-        del t, o, dt, part
+        assert torch.equal(K.f32_shuffle2x2_bwd(o, h, h)[0], t), "shuffle backward did not invert the forward"
+        del t, o
         torch.cuda.empty_cache()
     return out
 

@@ -5,6 +5,7 @@ Usage: python tools/step_profile.py [batch] [--unet] [--detail] [--out FILE.md]
 """
 import argparse
 import collections
+import ctypes
 import os
 import sys
 
@@ -43,13 +44,12 @@ def main():
     records = []
     orig_call = _C.call
 
-    def timed_call(name, *a):
+    def timed_call(name, *a, **kw):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        orig_call(name, *a)
+        orig_call(name, *a, **kw)
         e1.record()
-        dims = tuple(int(v) if isinstance(v, int) else int(v.value) for v in a
-                     if isinstance(v, int) or isinstance(v, (_C.c_int,)))
+        dims = tuple(v for (_, t), v in zip(_C.SIGNATURES[name], a) if t is not ctypes.c_void_p)   # sizes, not pointers
         records.append((name, dims, e0, e1))
 
     _C.call = timed_call

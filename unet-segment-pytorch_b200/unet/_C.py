@@ -1,12 +1,15 @@
 """ctypes binding of libunetb200.so (the C ABI declared in include/unetb200.h).
 
-There is no CPU or eager-PyTorch fallback: if the library is missing, or a
-tensor is not on a CUDA device, the ops raise.
+The header is the only declaration of the ABI: ``lib()`` parses its prototypes and sets every entry
+point's ``restype`` / ``argtypes`` from them, so a wrongly typed argument raises ``ctypes.ArgumentError``
+instead of reaching C as garbage.  There is no CPU or eager-PyTorch fallback: if the library is missing,
+or a tensor is not on a CUDA device, the ops raise.
 """
 from __future__ import annotations
 
 import ctypes
 import os
+import re
 import threading
 
 import torch
@@ -15,8 +18,11 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _PKG = os.path.dirname(_HERE)
 # UB2_LIB: another build of the same library (same-box A/B runs of a kernel change, tools/ab_lib.sh)
 LIB_PATH = os.environ.get("UB2_LIB") or os.path.join(_PKG, "lib", "libunetb200.so")
+HEADER = os.path.normpath(os.path.join(_PKG, os.pardir, "include", "unetb200.h"))
 
 _lib = None
+# {entry point: [(parameter name, ctypes type), ...]} in header order; filled by lib()
+SIGNATURES: dict = {}
 _lock = threading.Lock()
 
 ERRORS = {
@@ -28,9 +34,44 @@ ERRORS = {
 }
 
 
+_SCALARS = {"int": ctypes.c_int, "long long": ctypes.c_longlong, "float": ctypes.c_float, "double": ctypes.c_double}
+_TYPE_WORDS = {"const", "void", "char", "short", "int", "long", "float", "double", "signed", "unsigned"}
+
+
+def _parse_header(path: str = HEADER) -> dict:
+    """``int ub2_name(...);`` prototypes of the header -> SIGNATURES.  Any pointer is c_void_p; a ub2_ name
+    that is not such a prototype, an unnamed parameter or an unknown scalar type raises."""
+    if not os.path.exists(path):
+        raise RuntimeError(f"C ABI header not found at {path}")
+    with open(path) as f:
+        text = re.sub(r"/\*.*?\*/", " ", f.read(), flags=re.S)
+    sigs = {}
+    for m in re.finditer(r"\bint\s+(ub2_\w+)\s*\(([^()]*)\)\s*;", text):
+        name, params = m.group(1), " ".join(m.group(2).split())
+        if name in sigs:
+            raise RuntimeError(f"{path}: {name} is declared twice")
+        args = []
+        for p in ([] if params == "void" else params.split(",")):
+            words = re.findall(r"\w+|\*", p)
+            if len(words) < 2 or words[-1] in _TYPE_WORDS or words[-1] == "*":
+                raise RuntimeError(f"{path}: {name}: unnamed parameter '{p.strip()}'")
+            if "*" in words:
+                ctype = ctypes.c_void_p
+            else:
+                ctype = _SCALARS.get(" ".join(w for w in words[:-1] if w != "const"))
+                if ctype is None:
+                    raise RuntimeError(f"{path}: {name}: unknown parameter type in '{p.strip()}'")
+            args.append((words[-1], ctype))
+        sigs[name] = args
+    stray = sorted(set(re.findall(r"\bub2_\w+", text)) - set(sigs))
+    if stray:
+        raise RuntimeError(f"{path}: not an int-returning prototype: {', '.join(stray)}")
+    return sigs
+
+
 def lib() -> ctypes.CDLL:
-    """Load (once) and return the shared library; build it in-tree if it is absent."""
-    global _lib
+    """Load (once) and return the shared library, typed from the header; build it in-tree if it is absent."""
+    global _lib, SIGNATURES
     if _lib is not None:
         return _lib
     with _lock:
@@ -44,7 +85,14 @@ def lib() -> ctypes.CDLL:
                 mod.build()
             if not os.path.exists(LIB_PATH):
                 raise RuntimeError(f"libunetb200.so not found at {LIB_PATH} and could not be built")
-            _lib = ctypes.CDLL(LIB_PATH)
+            sigs = _parse_header()
+            handle = ctypes.CDLL(LIB_PATH)
+            for name, args in sigs.items():
+                fn = getattr(handle, name)
+                fn.restype = ctypes.c_int
+                fn.argtypes = [t for _, t in args]
+            SIGNATURES = sigs
+            _lib = handle
     return _lib
 
 
@@ -65,9 +113,9 @@ _tls = threading.local()
 
 
 def ptr(t):
-    """Device pointer of a CUDA tensor (None -> NULL)."""
+    """Device pointer of a CUDA tensor as an int (None -> NULL)."""
     if t is None:
-        return ctypes.c_void_p(0)
+        return None
     if not t.is_cuda:
         raise RuntimeError("unet-b200 ops need CUDA tensors: there is no CPU fallback")
     idx = t.device.index
@@ -77,12 +125,12 @@ def ptr(t):
     elif prev != idx:
         _tls.device = None
         raise RuntimeError(f"unet-b200 op received tensors on cuda:{prev} and cuda:{idx}")
-    return ctypes.c_void_p(t.data_ptr())
+    return t.data_ptr()
 
 
-def stream() -> ctypes.c_void_p:
+def stream() -> int:
     idx = getattr(_tls, "device", None)
-    return ctypes.c_void_p(torch.cuda.current_stream(idx).cuda_stream)
+    return torch.cuda.current_stream(idx).cuda_stream
 
 
 # kernels launched per entry point (default 1); used for the bench's `gpu_launches` claim
@@ -100,7 +148,6 @@ PROFILE = None
 def call(name: str, *args, work=None) -> None:
     global LAUNCHES
     fn = getattr(lib(), name)
-    fn.restype = ctypes.c_int
     idx = getattr(_tls, "device", None)
     _tls.device = None
     prof = PROFILE
@@ -120,7 +167,4 @@ def call(name: str, *args, work=None) -> None:
 
 
 c_int = ctypes.c_int
-c_float = ctypes.c_float
-c_double = ctypes.c_double
-c_longlong = ctypes.c_longlong
 byref = ctypes.byref

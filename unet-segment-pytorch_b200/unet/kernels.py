@@ -1,7 +1,8 @@
-"""Typed Python wrappers over the C ABI (one function per entry point family).
+"""Typed Python wrappers over the C ABI (one function per entry point family): the only module of
+the package that launches (``_C.call``).
 
-All tensors are CUDA tensors; activations are NHWC bf16 ``(N, H, W, C)`` views
-that are dense in their last dimension.  These wrappers only allocate outputs /
+All tensors are CUDA tensors; activations are NHWC bf16 ``(N, H, W, C)`` views (fp32 in the fp32 /
+TF32 section at the end) that are dense in their last dimension.  These wrappers only allocate outputs /
 workspaces with torch and pass raw pointers through ctypes; nothing here
 computes on the host and nothing synchronises the device, so a whole training
 step can be captured into a CUDA graph.
@@ -13,7 +14,7 @@ import ctypes
 import torch
 
 from . import _C
-from ._C import byref, c_double, c_float, c_int, c_longlong, ptr, stream
+from ._C import byref, c_int, ptr, stream
 
 BF16 = torch.bfloat16
 F32 = torch.float32
@@ -50,9 +51,11 @@ def _nhwc(t: torch.Tensor):
     return n, h, w, c, ld
 
 
-def _nhwc32(t: torch.Tensor):
-    """fp32 / TF32 mode: (N,H,W,C) fp32 whose channel stride may exceed C (a channel slice)."""
+def _nhwc32(t: torch.Tensor, dense=False):
+    """fp32 / TF32 mode: (N,H,W,C) fp32 whose channel stride may exceed C (a channel slice); ``dense``: the
+    entry point takes no channel stride, so the stride must be C."""
     assert t.dim() == 4 and t.dtype == F32 and t.stride(3) == 1, "expected NHWC fp32"
+    assert not dense or t.is_contiguous(), "expected dense NHWC fp32"
     n, h, w, c = t.shape
     # the stride between consecutive pixels: across a row, or (W = 1) down the rows, or (H = W = 1) across images
     ld = t.stride(2) if w > 1 else t.stride(1) if h > 1 else t.stride(0) if n > 1 else c
@@ -210,8 +213,8 @@ def bn_finalize(partials, count, gamma, beta, running_mean, running_var, nbt, mo
     rows, _, c = partials.shape
     dev = partials.device
     out = torch.empty((4, c), device=dev, dtype=F32)
-    _C.call("ub2_bn_finalize", ptr(partials), rows, c, c_double(float(count)), ptr(gamma), ptr(beta),
-            ptr(running_mean), ptr(running_var), ptr(nbt), c_float(momentum), c_float(eps),
+    _C.call("ub2_bn_finalize", ptr(partials), rows, c, count, ptr(gamma), ptr(beta),
+            ptr(running_mean), ptr(running_var), ptr(nbt), momentum, eps,
             ptr(out[0]), ptr(out[1]), ptr(out[2]), ptr(out[3]), stream())
     return out[0], out[1], out[2], out[3]
 
@@ -220,7 +223,7 @@ def bn_eval_coeffs(gamma, beta, running_mean, running_var, eps):
     c = running_mean.numel()
     out = torch.empty((2, c), device=running_mean.device, dtype=F32)
     _C.call("ub2_bn_eval_coeffs", ptr(gamma), ptr(beta), ptr(running_mean), ptr(running_var),
-            c_float(eps), c, ptr(out[0]), ptr(out[1]), stream())
+            eps, c, ptr(out[0]), ptr(out[1]), stream())
     return out[0], out[1]
 
 
@@ -269,7 +272,7 @@ def bn_bwd_finalize(partials, count, gamma, mean, invstd, frozen=False, dgamma=N
         grads = torch.zeros((2, c), device=partials.device, dtype=F32)
         dgamma, dbeta = grads[0], grads[1]
     coef = torch.empty((3, c), device=partials.device, dtype=F32)
-    _C.call("ub2_bn_bwd_finalize", ptr(partials), rows, c, c_double(float(count)), ptr(gamma), ptr(mean),
+    _C.call("ub2_bn_bwd_finalize", ptr(partials), rows, c, count, ptr(gamma), ptr(mean),
             ptr(invstd), int(frozen), ptr(dgamma), ptr(dbeta), ptr(coef), stream())
     if direct:
         return None, None, coef
@@ -387,7 +390,7 @@ def gate_bwd_finalize(partials, count, gamma_x, mean_x, invstd_x, gamma_g, mean_
     rows, _, ci = partials.shape
     grads = targets if targets is not None else torch.zeros((5, ci), device=partials.device, dtype=F32)
     coef = torch.empty((6, ci), device=partials.device, dtype=F32)
-    _C.call("ub2_gate_bwd_finalize", ptr(partials), rows, ci, c_double(float(count)), ptr(gamma_x),
+    _C.call("ub2_gate_bwd_finalize", ptr(partials), rows, ci, count, ptr(gamma_x),
             ptr(mean_x), ptr(invstd_x), ptr(gamma_g), ptr(mean_g), ptr(invstd_g), int(frozen), ptr(grads[0]),
             ptr(grads[1]),
             ptr(grads[2]), ptr(grads[3]), ptr(grads[4]), ptr(coef), stream())
@@ -479,10 +482,10 @@ def seg_stats(logits, targets):
     assert logits.dtype == F32 and logits.is_contiguous() and targets.dtype == torch.int64
     n, c, h, w = logits.shape
     targets = targets.contiguous()
-    blocks = _rows("ub2_seg_stats_blocks", n, c_longlong(h * w))
+    blocks = _rows("ub2_seg_stats_blocks", n, h * w)
     partials = torch.empty((n, blocks, c, 4), device=logits.device, dtype=F64)
     stats = torch.empty((n, 4, c), device=logits.device, dtype=F32)
-    _C.call("ub2_seg_stats", ptr(logits), ptr(targets), n, c, c_longlong(h * w), ptr(partials), blocks,
+    _C.call("ub2_seg_stats", ptr(logits), ptr(targets), n, c, h * w, ptr(partials), blocks,
             ptr(stats), stream(), work=(0.0, _nbytes(logits, targets)))
     return stats
 
@@ -496,7 +499,7 @@ def seg_stats_bwd(logits, targets, coef, gscale=None):
     assert gscale is None or (gscale.dtype == F32 and gscale.numel() == 1)
     dl = torch.empty_like(logits)
     _C.call("ub2_seg_stats_bwd", ptr(logits), ptr(targets.contiguous()), ptr(coef), ptr(gscale), n, c,
-            c_longlong(h * w), ptr(dl), stream(), work=(0.0, _nbytes(logits, targets, dl)))
+            h * w, ptr(dl), stream(), work=(0.0, _nbytes(logits, targets, dl)))
     return dl
 
 
@@ -505,8 +508,8 @@ def dice_bce_head(stats, ce_weight, dice_weight, class_weight, ce_smooth, dice_s
     n, _, c = stats.shape
     loss = torch.empty((1,), device=stats.device, dtype=F32)
     coef = torch.empty((n, 3, c), device=stats.device, dtype=F32)
-    _C.call("ub2_dice_bce_head", ptr(stats), n, c, c_float(ce_weight), c_float(dice_weight), c_float(class_weight),
-            c_float(ce_smooth), c_float(dice_smooth), int(ignore_background), ptr(loss), ptr(coef), stream())
+    _C.call("ub2_dice_bce_head", ptr(stats), n, c, ce_weight, dice_weight, class_weight,
+            ce_smooth, dice_smooth, int(ignore_background), ptr(loss), ptr(coef), stream())
     return loss[0], coef
 
 
@@ -524,9 +527,9 @@ def confusion(pred, target, num_classes, cm, ignore_index=None, threshold=None, 
         assert pred.dtype == torch.int64
         n, h, w = pred.shape
         mode = 1
-    _C.call("ub2_confusion", ptr(pred), ptr(target), mode, n, num_classes, c_longlong(h * w),
-            c_longlong(ignore_index if ignore_index is not None else 0),
-            int(ignore_index is not None), c_float(threshold if threshold is not None else 0.5), ptr(cm),
+    _C.call("ub2_confusion", ptr(pred), ptr(target), mode, n, num_classes, h * w,
+            ignore_index if ignore_index is not None else 0,
+            int(ignore_index is not None), threshold if threshold is not None else 0.5, ptr(cm),
             ptr(mask_out), stream(), work=(0.0, _nbytes(pred, target, mask_out)))
     return cm
 
@@ -549,7 +552,7 @@ def prepare_batch(images, labels=None, flags=None, mean=0.5, std=0.5, x=None, ta
         targets = None
     if flags is not None:
         assert flags.dtype == torch.uint8 and flags.numel() == n and flags.is_contiguous()
-    _C.call("ub2_prepare_batch", ptr(images), ptr(labels), ptr(flags), n, h, w, c_float(mean), c_float(std),
+    _C.call("ub2_prepare_batch", ptr(images), ptr(labels), ptr(flags), n, h, w, mean, std,
             ptr(x), ptr(targets), stream())
     return x, targets
 
@@ -564,9 +567,26 @@ def predict_mask(logits, threshold=0.5, mask=None, positives=None):
         positives = torch.empty((n,), device=logits.device, dtype=torch.int32)
     assert mask.dtype == torch.uint8 and mask.is_contiguous() and mask.numel() == n * h * w
     assert positives.dtype == torch.int32 and positives.numel() == n
-    _C.call("ub2_predict_mask", ptr(logits), n, c, c_longlong(h * w), c_float(threshold), ptr(mask), ptr(positives),
+    _C.call("ub2_predict_mask", ptr(logits), n, c, h * w, threshold, ptr(mask), ptr(positives),
             stream())
     return mask, positives
+
+
+# --------------------------------------------------------------------------- optimizer tail
+def grad_sumsq(ptrs, numel, chunks, nchunks, t, partial, step):
+    """Per-chunk fp64 sums of squared gradients (FusedAdamW's device tables, see unetb200.h); step += 1."""
+    _C.call("ub2_grad_sumsq", ptr(ptrs), ptr(numel), ptr(chunks), nchunks, t, ptr(partial), ptr(step), stream())
+
+
+def adamw_step(ptrs, numel, group, chunks, nchunks, t, partial, hyper, step, total_norm, write_grads):
+    """Gradient-norm clipping + AdamW update in place from grad_sumsq's partials."""
+    _C.call("ub2_adamw_step", ptr(ptrs), ptr(numel), ptr(group), ptr(chunks), nchunks, t, ptr(partial), ptr(hyper),
+            ptr(step), ptr(total_norm), int(write_grads), stream())
+
+
+def ema_update(desc, chunks, nchunks, decay):
+    """ModelEMA.update over the (T,4) int64 table ``desc`` with the device scalar ``decay``."""
+    _C.call("ub2_ema_update", ptr(desc), ptr(chunks), nchunks, ptr(decay), stream())
 
 
 # --------------------------------------------------------------------------- ConvTranspose2d(k = 2, s = 2)
@@ -630,3 +650,331 @@ def resize_planes_bwd(dout, h, w):
     din = torch.empty((n, c, h, w), device=dout.device, dtype=F32)
     _C.call("ub2_resize_planes_bwd", ptr(dout), ptr(din), n * c, h, w, ho, wo, stream())
     return din
+
+
+# --------------------------------------------------------------------------- fp32 / TF32 mode
+# fp32 NHWC activations and gradients (unet/fp32.py); reductions write the fp64 rows that bn_finalize,
+# bn_bwd_finalize and gate_bwd_finalize above fold.
+def conv_fwd_tf32(x0, x1, pack, cout, taps, scale=None, shift=None, relu=False, exact=False):
+    """x0 / x1: NHWC fp32 (channel stride may exceed the channel count); ``pack``: (Cout, taps, Cin) fp32."""
+    n, h, w, c0, ld0 = _nhwc32(x0)
+    c1, ld1 = 0, 0
+    if x1 is not None:
+        _, _, _, c1, ld1 = _nhwc32(x1)
+    assert pack.is_contiguous() and pack.numel() == cout * taps * (c0 + c1)
+    out = torch.empty((n, h, w, cout), device=x0.device, dtype=F32)
+    _C.call("ub2_conv_fwd_tf32", ptr(x0), ld0, c0, ptr(x1), ld1, c1, ptr(pack), ptr(out), cout, n, h, w,
+            cout, taps, ptr(scale), ptr(shift), int(relu), int(exact), stream(),
+            work=(2.0 * n * h * w * cout * taps * (c0 + c1), _nbytes(x0, x1, pack, out)))
+    return out
+
+
+def f32_pack_weight(w):
+    """OIHW fp32 -> the TF32 pack (Cout, taps, Cin)."""
+    cout, cin, kh, kw = w.shape
+    out = torch.empty((cout, kh * kw, cin), device=w.device, dtype=F32)
+    _C.call("ub2_f32_pack_weight", ptr(w.contiguous()), ptr(out), cout, cin, kh * kw, stream())
+    return out
+
+
+def f32_pack_weight3(w, dgrad=False):
+    """OIHW fp32 -> the 3xTF32 pack (rows, taps, 3*K) = per tap [w_hi | w_hi | w_lo]; ``dgrad``: rows = Cin,
+    K = Cout, taps flipped (the data gradient is the same kernel)."""
+    cout, cin, kh, kw = w.shape
+    rows, k = (cin, cout) if dgrad else (cout, cin)
+    out = torch.empty((rows, kh * kw, 3 * k), device=w.device, dtype=F32)
+    _C.call("ub2_f32_pack_weight3", ptr(w.contiguous()), ptr(out), cout, cin, kh * kw, int(dgrad), stream())
+    return out
+
+
+def f32_split_tf32(x0, x1=None):
+    """(N,H,W,C0 [+C1]) fp32 -> (N,H,W,2*(C0+C1)) = [hi(x0) | hi(x1) | lo(x0) | lo(x1)], two TF32 numbers per value."""
+    n, h, w, c0, ld0 = _nhwc32(x0)
+    c1, ld1 = 0, 0
+    if x1 is not None:
+        _, _, _, c1, ld1 = _nhwc32(x1)
+    out = torch.empty((n, h, w, 2 * (c0 + c1)), device=x0.device, dtype=F32)
+    _C.call("ub2_f32_split_tf32", ptr(x0), ld0, c0, ptr(x1), ld1, c1, ptr(out), n * h * w, stream(),
+            work=(0.0, _nbytes(x0, x1, out)))
+    return out
+
+
+def f32_split_bf16(x):
+    """dense fp32 NHWC -> (hi, lo) bf16 NHWC with x = hi + lo to 2^-16 relative."""
+    _nhwc32(x, dense=True)
+    hi = torch.empty(x.shape, device=x.device, dtype=BF16)
+    lo = torch.empty(x.shape, device=x.device, dtype=BF16)
+    _C.call("ub2_f32_split_bf16", ptr(x), ptr(hi), ptr(lo), x.numel(), stream(), work=(0.0, _nbytes(x, hi, lo)))
+    return hi, lo
+
+
+def f32_conv_in(x, w, scale, shift):
+    """Inference: first conv + folded BN + ReLU, x (N,Cin,H,W) fp32 NCHW -> (N,H,W,Cout) fp32."""
+    assert x.dtype == F32 and x.is_contiguous()
+    n, cin, h, wd = x.shape
+    cout = w.shape[0]
+    out = torch.empty((n, h, wd, cout), device=x.device, dtype=F32)
+    _C.call("ub2_f32_conv_in", ptr(x), ptr(w.contiguous()), ptr(scale), ptr(shift), ptr(out), n, cin, h, wd, cout,
+            stream())
+    return out
+
+
+def f32_conv_in_raw(x, w):
+    """First conv without BatchNorm (training): x (N,Cin,H,W) fp32 NCHW -> y (N,H,W,Cout) fp32."""
+    assert x.dtype == F32 and x.is_contiguous()
+    n, cin, h, wd = x.shape
+    cout = w.shape[0]
+    y = torch.empty((n, h, wd, cout), device=x.device, dtype=F32)
+    _C.call("ub2_f32_conv_in_raw", ptr(x), ptr(w.contiguous()), ptr(y), n, cin, h, wd, cout, stream())
+    return y
+
+
+def f32_conv_in_wgrad(x, dy, wshape):
+    """Weight gradient (Cout,Cin,3,3) fp32 of f32_conv_in_raw from x NCHW and dy (N,H,W,Cout) fp32."""
+    assert x.dtype == F32 and x.is_contiguous()
+    _nhwc32(dy, dense=True)
+    n, cin, h, wd = x.shape
+    cout = wshape[0]
+    rows = _rows("ub2_f32_channel_rows", n * h * wd, cout)
+    part = torch.empty((rows, cin, 9, cout), device=x.device, dtype=F64)
+    gw = torch.zeros(wshape, device=x.device, dtype=F32)
+    _C.call("ub2_f32_conv_in_wgrad", ptr(x), ptr(dy), ptr(part), rows, ptr(gw), n, cin, h, wd, cout, stream())
+    return gw
+
+
+def f32_maxpool(a):
+    """Inference: 2x2 max-pool of a dense NHWC fp32 tensor."""
+    n, h, w, c, _ = _nhwc32(a, dense=True)
+    out = torch.empty((n, h // 2, w // 2, c), device=a.device, dtype=F32)
+    _C.call("ub2_f32_maxpool", ptr(a), ptr(out), n, h, w, c, stream())
+    return out
+
+
+def f32_maxpool_idx(a):
+    """2x2 max-pool of a dense NHWC fp32 tensor and the uint8 window position of each maximum."""
+    n, h, w, c, _ = _nhwc32(a, dense=True)
+    p = torch.empty((n, h // 2, w // 2, c), device=a.device, dtype=F32)
+    idx = torch.empty((n, h // 2, w // 2, c), device=a.device, dtype=torch.uint8)
+    _C.call("ub2_f32_maxpool_idx", ptr(a), ptr(p), ptr(idx), n, h, w, c, stream(), work=(0.0, _nbytes(a, p, idx)))
+    return p, idx
+
+
+def f32_maxpool_bwd(dP, idx, shape):
+    """Route the pooled gradient to the saved window positions: the act_bwd apply pass with identity coefficients
+    (dy = routed gradient) onto an (N,H,W,C) = ``shape`` fp32 tensor."""
+    n, h, w, c = shape
+    _nhwc32(dP, dense=True)
+    dev = idx.device
+    ones, zeros = torch.ones(c, device=dev), torch.zeros(c, device=dev)
+    coef = torch.stack([ones, zeros, zeros])
+    dummy_y = torch.zeros((n, h, w, c), device=dev, dtype=F32)
+    dy = torch.empty((n, h, w, c), device=dev, dtype=F32)
+    _C.call("ub2_f32_act_bwd_apply", None, 0, ptr(dP), ptr(idx), ptr(dummy_y), ptr(ones), ptr(zeros),
+            ptr(coef), ptr(dy), n, h, w, c, 0, stream())
+    return dy
+
+
+def f32_upsample(a, out_h, out_w):
+    """Inference: bilinear 2x (align_corners=True) of a dense NHWC fp32 tensor, centred in (out_h, out_w)."""
+    n, h, w, c, _ = _nhwc32(a, dense=True)
+    out = torch.empty((n, out_h, out_w, c), device=a.device, dtype=F32)
+    _C.call("ub2_f32_upsample", ptr(a), ptr(out), n, h, w, 2 * h, 2 * w, out_h, out_w, c, stream())
+    return out
+
+
+def f32_upsample_fwd(a, out_h, out_w, hu=None, wu=None):
+    """bilinear (h,w) -> (hu,wu) (default 2x), centred in a zero (out_h,out_w) canvas (F.pad of layers.py:98-102)."""
+    n, h, w, c, _ = _nhwc32(a, dense=True)
+    hu, wu = (2 * h if hu is None else hu), (2 * w if wu is None else wu)
+    out = torch.empty((n, out_h, out_w, c), device=a.device, dtype=F32)
+    _C.call("ub2_f32_upsample_fwd", ptr(a), ptr(out), n, h, w, hu, wu, out_h, out_w, c, stream(),
+            work=(0.0, _nbytes(a, out)))
+    return out
+
+
+def f32_upsample_bwd(dout, hin, win, hu, wu):
+    n, ho, wo, c, ld = _nhwc32(dout)
+    din = torch.empty((n, hin, win, c), device=dout.device, dtype=F32)
+    _C.call("ub2_f32_upsample_bwd", ptr(dout), ld, ptr(din), n, hin, win, hu, wu, ho, wo, c, stream(),
+            work=(0.0, _nbytes(dout, din)))
+    return din
+
+
+def f32_channel_stats(x):
+    """(rows, 2, C) fp64 per-block sums / sums of squares over the pixels of an NHWC fp32 tensor."""
+    n, h, w, c, ld = _nhwc32(x)
+    rows = _rows("ub2_f32_channel_rows", n * h * w, c)
+    part = torch.empty((rows, 2, c), device=x.device, dtype=F64)
+    _C.call("ub2_f32_channel_stats", ptr(x), ld, n * h * w, c, ptr(part), rows, stream(), work=(0.0, _nbytes(x)))
+    return part
+
+
+def f32_scalar_stats(x):
+    """(rows, 2, 1) fp64 per-block sum / sum of squares of a dense fp32 tensor."""
+    assert x.dtype == F32 and x.is_contiguous()
+    n = x.numel()
+    rows = _rows("ub2_f32_scalar_rows", n)
+    part = torch.empty((rows, 2, 1), device=x.device, dtype=F64)
+    _C.call("ub2_f32_scalar_stats", ptr(x), n, ptr(part), rows, stream(), work=(0.0, _nbytes(x)))
+    return part
+
+
+def f32_affine_act(y, scale, shift, relu=True):
+    """relu?(scale*y + shift) per channel of a dense NHWC fp32 tensor."""
+    n, h, w, c, _ = _nhwc32(y, dense=True)
+    out = torch.empty_like(y)
+    _C.call("ub2_f32_affine_act", ptr(y), ptr(scale), ptr(shift), ptr(out), n * h * w, c, int(relu), stream(),
+            work=(0.0, _nbytes(y, out)))
+    return out
+
+
+def f32_act_bwd(dA, dP, idx, y, scale, shift, mean, invstd, gamma, batch, relu=True):
+    """BatchNorm (+ReLU, + max-pool routing) backward: (dy, dgamma, dbeta).  dA may be a channel slice; dP, y dense."""
+    n, h, w, c, _ = _nhwc32(y, dense=True)
+    ld_da = _nhwc32(dA)[4] if dA is not None else 0
+    if dP is not None:
+        _nhwc32(dP, dense=True)
+    rows = _rows("ub2_f32_channel_rows", n * h * w, c)
+    part = torch.empty((rows, 2, c), device=y.device, dtype=F64)
+    _C.call("ub2_f32_act_bwd_reduce", ptr(dA), ld_da, ptr(dP), ptr(idx), ptr(y), ptr(scale), ptr(shift), ptr(part),
+            rows, n, h, w, c, int(relu), stream(), work=(0.0, _nbytes(dA, dP, idx, y)))
+    dgamma, dbeta, coef = bn_bwd_finalize(part, n * h * w, gamma, mean, invstd, frozen=not batch)
+    dy = torch.empty_like(y)
+    _C.call("ub2_f32_act_bwd_apply", ptr(dA), ld_da, ptr(dP), ptr(idx), ptr(y), ptr(scale), ptr(shift), ptr(coef),
+            ptr(dy), n, h, w, c, int(relu), stream(), work=(0.0, _nbytes(dA, dP, idx, y, dy)))
+    return dy, dgamma, dbeta
+
+
+def f32_gate(q, xp, x, sg, hg, sx, hx, wpsi, spsi, hpsi):
+    """Inference: out = x * sigmoid(BN_psi(w_psi . relu(BN_g(up q) + BN_x(xp)))), q at the gating resolution."""
+    _, hin, win, ci, _ = _nhwc32(q, dense=True)
+    _nhwc32(xp, dense=True)
+    n, h, w, cx, _ = _nhwc32(x, dense=True)
+    out = torch.empty_like(x)
+    _C.call("ub2_f32_gate", ptr(q), ptr(xp), ptr(x), ptr(sg), ptr(hg), ptr(sx), ptr(hx), ptr(wpsi), ptr(spsi),
+            ptr(hpsi), ptr(out), n, hin, win, h, w, ci, cx, stream())
+    return out
+
+
+def f32_gate_psi(u, xp, sg, hg, sx, hx, wpsi):
+    """psi_raw (N,H,W) = w_psi . relu(BN_g(u) + BN_x(xp)), u = up(q) and xp dense NHWC fp32."""
+    n, h, w, ci, _ = _nhwc32(u, dense=True)
+    _nhwc32(xp, dense=True)
+    psi = torch.empty((n, h, w), device=u.device, dtype=F32)
+    _C.call("ub2_f32_gate_psi", ptr(u), ptr(xp), ptr(sg), ptr(hg), ptr(sx), ptr(hx), ptr(wpsi), ptr(psi),
+            n * h * w, ci, stream(), work=(0.0, _nbytes(u, xp, psi)))
+    return psi
+
+
+def f32_gate_apply(psi, spsi, hpsi, x):
+    """a = sigmoid(BN_psi(psi_raw)), out = x * a: returns (out, a)."""
+    n, h, w, cx, _ = _nhwc32(x, dense=True)
+    assert psi.is_contiguous()
+    out = torch.empty_like(x)
+    a = torch.empty((n, h, w), device=x.device, dtype=F32)
+    _C.call("ub2_f32_gate_apply", ptr(psi), ptr(spsi), ptr(hpsi), ptr(x), ptr(out), ptr(a), n * h * w, cx, stream(),
+            work=(0.0, _nbytes(psi, x, out, a)))
+    return out, a
+
+
+def f32_gate_bwd_a(dout, x, a, psi):
+    """(dx, dpsin, (rows, 2, 1) partials); dout may be a channel slice."""
+    ld_do = _nhwc32(dout)[4]
+    n, h, w, cx, _ = _nhwc32(x, dense=True)
+    assert a.is_contiguous() and psi.is_contiguous()
+    rows = _rows("ub2_f32_gate_rows", n * h * w)
+    dx = torch.empty_like(x)
+    dpsin = torch.empty((n, h, w), device=x.device, dtype=F32)
+    part = torch.empty((rows, 2, 1), device=x.device, dtype=F64)
+    _C.call("ub2_f32_gate_bwd_a", ptr(dout), ld_do, ptr(x), ptr(a), ptr(psi), ptr(dx), ptr(dpsin), ptr(part), rows,
+            n * h * w, cx, stream(), work=(0.0, _nbytes(dout, x, a, psi, dx, dpsin)))
+    return dx, dpsin, part
+
+
+def f32_gate_bwd_s(dpsin, psi, coef_psi, u, xp, sg, hg, sx, hx, wpsi):
+    """(ds, (rows, 4, Ci) partials)."""
+    n, h, w, ci, _ = _nhwc32(u, dense=True)
+    _nhwc32(xp, dense=True)
+    assert dpsin.is_contiguous() and psi.is_contiguous()
+    rows = _rows("ub2_f32_gate_rows", n * h * w)
+    ds = torch.empty_like(xp)
+    part = torch.empty((rows, 4, ci), device=u.device, dtype=F64)
+    _C.call("ub2_f32_gate_bwd_s", ptr(dpsin), ptr(psi), ptr(coef_psi), ptr(u), ptr(xp), ptr(sg), ptr(hg), ptr(sx),
+            ptr(hx), ptr(wpsi), ptr(ds), ptr(part), rows, n * h * w, ci, stream(),
+            work=(0.0, _nbytes(dpsin, psi, u, xp, ds)))
+    return ds, part
+
+
+def f32_gate_bwd_xg(ds, xp, u, coef):
+    """(dxp, du): the gradients of BN_x(xp) and BN_g(u)."""
+    n, h, w, ci, _ = _nhwc32(u, dense=True)
+    _nhwc32(ds, dense=True)
+    _nhwc32(xp, dense=True)
+    dxp = torch.empty_like(xp)
+    du = torch.empty_like(xp)
+    _C.call("ub2_f32_gate_bwd_xg", ptr(ds), ptr(xp), ptr(u), ptr(coef), ptr(dxp), ptr(du), n * h * w, ci, stream(),
+            work=(0.0, _nbytes(ds, xp, u, dxp, du)))
+    return dxp, du
+
+
+def f32_outc(a, w, bias, claim_work=True):
+    """OutConv: dense NHWC fp32 a, w (K,C,1,1) -> fp32 NCHW logits.  ``claim_work=False``: no roofline claim (the
+    inference path)."""
+    n, h, wd, c, _ = _nhwc32(a, dense=True)
+    k = w.shape[0]
+    logits = torch.empty((n, k, h, wd), device=a.device, dtype=F32)
+    _C.call("ub2_f32_outc", ptr(a), ptr(w.reshape(k, -1).contiguous()), ptr(bias), ptr(logits), n, h, wd, c, k,
+            stream(), work=(0.0, _nbytes(a, logits)) if claim_work else None)
+    return logits
+
+
+def f32_outc_bwd(dlogits, a, w, need_da=True):
+    """(da or None, dw (K,C,1,1), db (K,)) from dense fp32 NCHW dlogits."""
+    n, h, wd, c, _ = _nhwc32(a, dense=True)
+    assert dlogits.dtype == F32 and dlogits.is_contiguous()
+    k = w.shape[0]
+    rows = _rows("ub2_f32_outc_rows", n, h, wd)
+    part = torch.empty((rows, k * c + k), device=a.device, dtype=F64)
+    da = torch.empty_like(a) if need_da else None
+    dw = torch.zeros(w.shape, device=a.device, dtype=F32)
+    db = torch.zeros((k,), device=a.device, dtype=F32)
+    _C.call("ub2_f32_outc_bwd", ptr(dlogits), ptr(a), ptr(w.reshape(k, -1).contiguous()), ptr(da), ptr(part), rows,
+            ptr(dw), ptr(db), n, h, wd, c, k, stream(), work=(0.0, _nbytes(dlogits, a, da)))
+    return da, dw, db
+
+
+def f32_pack_convt_weight(weight, bias):
+    """(Cin, Cout, 2, 2) fp32 parameter -> (the exact 1x1 weight (4*Cout, Cin, 1, 1) OIHW, row (i*2+j)*Cout + co;
+    scale4 = ones, shift4 = bias tiled four times)."""
+    cin, cout = weight.shape[0], weight.shape[1]
+    w1 = torch.empty((4 * cout, cin, 1, 1), device=weight.device, dtype=F32)
+    ss = torch.empty((2, 4 * cout), device=weight.device, dtype=F32)
+    _C.call("ub2_f32_pack_convt_weight", ptr(weight.contiguous()), ptr(bias), ptr(w1), ptr(ss[0]), ptr(ss[1]), cin,
+            cout, stream())
+    return w1, ss[0], ss[1]
+
+
+def f32_shuffle2x2(t, cout, out_h, out_w):
+    """t (N,h,w,4*Cout) fp32 -> (N,out_h,out_w,Cout): pixel shuffle of the transposed convolution + F.pad (zeros)."""
+    n, h, w, c4, ld = _nhwc32(t)
+    assert c4 == 4 * cout
+    out = torch.empty((n, out_h, out_w, cout), device=t.device, dtype=F32)
+    _C.call("ub2_f32_shuffle2x2_fwd", ptr(t), ld, ptr(out), cout, n, h, w, cout, out_h, out_w, stream(),
+            work=(0.0, _nbytes(t, out)))
+    return out
+
+
+def f32_shuffle2x2_bwd(dout, h, w, want_bias=True):
+    """Transpose of f32_shuffle2x2: dout (N,Ho,Wo,Cout), channel stride may exceed Cout -> (dt (N,h,w,4*Cout),
+    bias gradient (Cout,) or None)."""
+    n, ho, wo, cout, ld = _nhwc32(dout)
+    dt = torch.empty((n, h, w, 4 * cout), device=dout.device, dtype=F32)
+    partials = db = None
+    rows = 0
+    if want_bias:
+        rows = _rows("ub2_f32_shuffle2x2_rows", n, h, w, cout, ho, wo)
+        partials = torch.empty((rows, cout), device=dout.device, dtype=F64)
+        db = torch.zeros((cout,), device=dout.device, dtype=F32)
+    _C.call("ub2_f32_shuffle2x2_bwd", ptr(dout), ld, ptr(dt), 4 * cout, ptr(partials), rows, ptr(db), n, h, w, cout,
+            ho, wo, stream(), work=(0.0, _nbytes(dout, dt)))
+    return dt, db

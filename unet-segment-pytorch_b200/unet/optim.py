@@ -14,7 +14,7 @@ from __future__ import annotations
 import torch
 
 from . import _C
-from ._C import ptr, stream
+from . import kernels as K
 
 
 class FusedAdamW(torch.optim.AdamW):
@@ -177,11 +177,9 @@ class FusedAdamW(torch.optim.AdamW):
             raise RuntimeError("FusedAdamW: run at least one eager step before capturing a CUDA graph")
         fz = self._fz
         t = len(fz["params"])
-        _C.call("ub2_grad_sumsq", ptr(fz["ptrs"]), ptr(fz["numel"]), ptr(fz["chunks"]), fz["nchunks"], t,
-                ptr(fz["partial"]), ptr(fz["step"]), stream())
-        _C.call("ub2_adamw_step", ptr(fz["ptrs"]), ptr(fz["numel"]), ptr(fz["group"]), ptr(fz["chunks"]),
-                fz["nchunks"], t, ptr(fz["partial"]), ptr(fz["hyper"]), ptr(fz["step"]), ptr(fz["total_norm"]),
-                int(self.write_clipped_grads), stream())
+        K.grad_sumsq(fz["ptrs"], fz["numel"], fz["chunks"], fz["nchunks"], t, fz["partial"], fz["step"])
+        K.adamw_step(fz["ptrs"], fz["numel"], fz["group"], fz["chunks"], fz["nchunks"], t, fz["partial"], fz["hyper"],
+                     fz["step"], fz["total_norm"], self.write_clipped_grads)
         return loss
 
     @property

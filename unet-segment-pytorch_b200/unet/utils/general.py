@@ -14,7 +14,7 @@ import copy
 import torch
 
 from .. import _C
-from .._C import ptr, stream
+from .. import kernels as K
 
 
 class ModelEMA:
@@ -88,7 +88,7 @@ class ModelEMA:
         elif self._tables is None:
             raise RuntimeError("ModelEMA: call prepare(model) before update(model, _advance=False)")
         _, desc, chunks, nchunks, decay = self._tables
-        _C.call("ub2_ema_update", ptr(desc), ptr(chunks), nchunks, ptr(decay), stream())
+        K.ema_update(desc, chunks, nchunks, decay)
 
     def state_dict(self) -> dict:
         return {'ema_state_dict': self.ema_model.state_dict(), 'decay': self.decay, 'updates': self.updates}
