@@ -55,6 +55,11 @@ int ub2_last_conv_variant(void);
  * out1), and per-CTA rows of per-channel sum / sum-of-squares (stats: (stats_rows,2,Cout)
  * doubles; *stats_rows_used rows are written) for train-mode BatchNorm.  With the
  * flipped/transposed weight pack it is the data-gradient pass autograd runs for the same conv.
+ * Channels: C0, C1 and Cout multiples of 8, not necessarily of 16 (the K chunks past a source's end
+ * read zeros through the tensor map, never memory); ld_in0 / ld_in1 / ld0 / ld1 and split multiples
+ * of 8.  A C0 or C1 that is not a multiple of 8 returns UB2_ERR_ALIGN: each source's columns of the
+ * weight pack must start on 16 bytes.  Only output channels < Cout are written: channels between
+ * Cout and ld0 keep their contents.
  */
 int ub2_conv_fwd(const void* in0, int ld_in0, int C0, const void* in1, int ld_in1, int C1,
                  const void* wgt, void* out0, int ld0, void* out1, int ld1, int split, int N, int H,
@@ -63,7 +68,8 @@ int ub2_conv_fwd(const void* in0, int ld_in0, int C0, const void* in1, int ld_in
                  int bn_override, int grid_override, void* stream);
 
 /* Weight-gradient pass of the same nn.Conv2d (autograd of layers.py:32,35,152,158): split-K
- * partial tiles (splits, taps*(C0+C1), Cout) fp32; *splits_used <= max_splits are written. */
+ * partial tiles (splits, taps*(C0+C1), Cout) fp32; *splits_used <= max_splits are written.
+ * Channels: C0 >= 1 and C1 >= 0 of any count, Cout a multiple of 8, channel strides multiples of 8. */
 int ub2_conv_wgrad(const void* in0, int ld_in0, int C0, const void* in1, int ld_in1, int C1,
                    const void* dy, int ld_dy, float* partial, int max_splits, int* splits_used,
                    int N, int H, int W, int Cout, int taps, int splits_override, void* stream);
@@ -89,8 +95,9 @@ int ub2_wgrad_reduce_multi(const Ub2ReduceItem* items, int n, int accumulate, vo
 int ub2_pack_conv_weight(const float* w, void* fwd, void* dgrad, int Cout, int Cin, int taps,
                          const float* out_scale, void* stream);
 /* The same for many weights in one launch (once per optimizer step): desc (T,6) int64 =
- * {w, fwd, dgrad, Cout, Cin, taps} with Cout and Cin multiples of 16; blocks (nblocks,4) int32 =
- * {tensor, Cin tile, Cout tile, 0}, one per 16x16 channel tile. */
+ * {w, fwd, dgrad, Cout, Cin, taps}; blocks (nblocks,4) int32 = {tensor, Cin tile, Cout tile, edge},
+ * one per 16x16 channel tile.  edge = 0 only for a whole tile (16 channels of each) of a weight whose
+ * Cout and Cin are multiples of 8; any other tile (partial, or other channel counts) needs edge = 1. */
 int ub2_pack_conv_weights_multi(const long long* desc, const int* blocks, int nblocks, void* stream);
 
 /* ======================= BatchNorm / ReLU / MaxPool passes ============================== */
@@ -271,7 +278,9 @@ int ub2_confusion(const void* pred, const long long* target, int mode, int N, in
 /* nn.Conv2d (+ folded BN + ReLU) of layers.py:32-37,152,158: in0/in1 fp32 NHWC (virtual concat),
  * wgt = ub2_f32_pack_weight output (Cout,taps,C0+C1) fp32, out fp32 NHWC; out = relu?(scale*acc+shift).
  * exact_out = 0: the result is rounded to TF32 (it feeds the next single-pass convolution: inference);
- * exact_out = 1: the fp32 accumulator is stored as is (the 3xTF32 launches of the training mode). */
+ * exact_out = 1: the fp32 accumulator is stored as is (the 3xTF32 launches of the training mode).
+ * Channels as for ub2_conv_fwd, with C0 and C1 multiples of 4 (16 bytes of fp32): Cout and the channel
+ * strides multiples of 8. */
 int ub2_conv_fwd_tf32(const float* in0, int ld_in0, int C0, const float* in1, int ld_in1, int C1,
                       const float* wgt, float* out, int ld_out, int N, int H, int W, int Cout, int taps,
                       const float* scale, const float* shift, int relu, int exact_out, void* stream);

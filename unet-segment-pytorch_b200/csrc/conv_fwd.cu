@@ -60,7 +60,11 @@ conv_fwd_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
   const int C0 = p.C0;
   const int Ctot = p.C0 + p.C1;
   const int kc = p.kc;
-  const int kchunks = Ctot / kc;
+  // each source is walked in whole kc chunks (C0p, C1p: its channel count rounded up to kc); channels past a
+  // source's end are zero-filled by its tensor map, so the weight columns they meet contribute nothing
+  const int C0p = (C0 + kc - 1) & -kc;
+  const int Ckp = C0p + ((p.C1 + kc - 1) & -kc);
+  const int kchunks = Ckp / kc;
   const int tiles_m = p.tiles_w * p.tiles_h * p.tiles_n;
   const int n_tiles = p.n_tiles;
   const int total_tiles = tiles_m * n_tiles;
@@ -111,17 +115,18 @@ conv_fwd_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
       for (int tap = 0; tap < TAPS; ++tap) {
         const int dr = (TAPS == 9) ? tap / 3 - 1 : 0;
         const int ds = (TAPS == 9) ? tap % 3 - 1 : 0;
-        int kb = tap * Ctot;
-        for (int c = 0; c < Ctot; c += kc, ++kb) {
+        for (int c = 0; c < Ckp; c += kc) {
           mbar_wait(&hdr->empty[stage], phase ^ 1);
           if (elect_one()) {
             uint8_t* sa = tiles + stage * stage_bytes;
             mbar_expect_tx(&hdr->full[stage], tx_bytes);
-            if (c < C0)
+            if (c < C0p) {
               tma_load_4d(sa, &tmA0, &hdr->full[stage], c, w0 + ds, h0 + dr, i0);
-            else
-              tma_load_4d(sa, &tmA1, &hdr->full[stage], c - C0, w0 + ds, h0 + dr, i0);
-            tma_load_2d(sa + kATileBytes, &tmB, &hdr->full[stage], tap * Ctot + c, n0);
+              tma_load_2d(sa + kATileBytes, &tmB, &hdr->full[stage], tap * Ctot + c, n0);
+            } else {
+              tma_load_4d(sa, &tmA1, &hdr->full[stage], c - C0p, w0 + ds, h0 + dr, i0);
+              tma_load_2d(sa + kATileBytes, &tmB, &hdr->full[stage], tap * Ctot + C0 + (c - C0p), n0);
+            }
           }
           if (++stage == stages) {
             stage = 0;
@@ -247,11 +252,16 @@ int conv_fwd_launch(const ConvFwdArgs& a, cudaStream_t stream) {
   const int esz = a.tf32 ? 4 : 2;
   if (a.taps != 1 && a.taps != 9) return UB2_ERR_SHAPE;
   if (a.N <= 0 || a.H <= 0 || a.W <= 0 || a.C0 <= 0 || a.C1 < 0) return UB2_ERR_SHAPE;
-  if (Ctot % 16 != 0 || a.C0 % 16 != 0 || a.Cout % 16 != 0) return UB2_ERR_SHAPE;
+  // output channels in multiples of 8 (one 16-byte store); each source's weight-pack columns start on 16 bytes
+  // (a TMA box may not start inside a 16-byte unit): C0 and C1 multiples of 8 bf16 / 4 fp32 channels
+  if (a.Cout % 8 != 0) return UB2_ERR_SHAPE;
   if (a.ld_in0 % 8 != 0 || (a.C1 > 0 && a.ld_in1 % 8 != 0) || a.ld0 % 8 != 0) return UB2_ERR_ALIGN;
+  if ((a.C0 * esz) % 16 != 0 || (a.C1 * esz) % 16 != 0) return UB2_ERR_ALIGN;
   if (a.tf32 && (a.stats != nullptr || a.accumulate || a.out1 != nullptr)) return UB2_ERR_SHAPE;  // eval only
-  int kc = 128 / esz;   // channels per 128-byte K chunk
-  while (a.C0 % kc != 0 || Ctot % kc != 0) kc /= 2;
+  // channels per K chunk: 128 bytes, halved while it does not divide both sources, down to 32 bytes (the MMA K);
+  // sources that are not a multiple of the chunk are padded to it (zero fill of the activation tensor maps)
+  int kc = 128 / esz;
+  while (kc > 32 / esz && (a.C0 % kc != 0 || Ctot % kc != 0)) kc /= 2;
 
   ConvFwdParams p{};
   p.N = a.N; p.H = a.H; p.W = a.W;
@@ -263,8 +273,9 @@ int conv_fwd_launch(const ConvFwdArgs& a, cudaStream_t stream) {
   p.tiles_w = (a.W + p.BW - 1) / p.BW;
   p.tiles_h = (a.H + p.BH - 1) / p.BH;
   p.tiles_n = (a.N + p.BI - 1) / p.BI;
-  // N tile: whole Cout when it fits one accumulator buffer; must divide the split point.
-  int BN = a.Cout <= 256 ? a.Cout : 256;
+  // N tile: whole Cout (rounded up to the MMA's multiple of 16; the weight tensor map zero-fills the rows past
+  // Cout) when it fits one accumulator buffer; must divide the split point.
+  int BN = a.Cout <= 256 ? (a.Cout + 15) & ~15 : 256;
   const int split = (a.out1 != nullptr) ? a.split : (1 << 30);
   if (a.out1 != nullptr) {
     if (a.split % 8 != 0 || a.ld1 % 8 != 0) return UB2_ERR_ALIGN;

@@ -3,7 +3,9 @@
 //   dW[tap, c, co] = sum_{n,h,w} in[n, h+r-1, w+s-1, c] * dy[n,h,w,co]
 //
 // GEMM view: M = taps*(C0+C1) (im2col rows, tile 128), N = Cout (tile BN <= 256),
-// K = pixels, walked in chunks of 64 (one TMA box BW x BH x BI).  Both operands
+// K = pixels, walked in chunks of 64 (one TMA box BW x BH x BI).  A source whose channel count is
+// not a multiple of the mc-channel A sub-box is padded to whole sub-boxes per tap (M rows that the
+// tensor map zero-fills and the epilogue drops), so the partial layout keeps the real rows only.  Both operands
 // are read exactly as the activations lie in HBM (NHWC: channels contiguous), i.e.
 // MN-major shared-memory tiles — no transposed copies.  Split-K over pixels: each
 // work item (m tile, n tile, split) writes an fp32 partial tile; a second kernel
@@ -41,6 +43,9 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
   const int lane = threadIdx.x & 31;
   const int Ctot = p.C0 + p.C1;
   const int Mtot = p.taps * Ctot;
+  const int C0p = (p.C0 + p.mc - 1) & -p.mc;                 // sources padded to whole A sub-boxes
+  const int Ctp = C0p + ((p.C1 + p.mc - 1) & -p.mc);
+  const int Mp = p.taps * Ctp;                              // padded M rows
   const int total_chunks = p.chunks_w * p.chunks_h * p.chunks_n;
   const int per_split = (total_chunks + p.splits - 1) / p.splits;
   const int total_items = p.m_tiles * p.n_tiles * p.splits;
@@ -87,9 +92,9 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
       int sub_c = 0, sub_ds = 0, sub_dr = 0;
       if (lane < a_subs) {
         int m = mt * 128 + lane * p.mc;
-        if (m >= Mtot) m = Mtot - p.mc;  // rows past the end are discarded by the epilogue
-        const int tap = m / Ctot;
-        sub_c = m % Ctot;
+        if (m >= Mp) m = Mp - p.mc;  // rows past the end are discarded by the epilogue
+        const int tap = m / Ctp;
+        sub_c = m % Ctp;
         sub_dr = (p.taps == 9) ? tap / 3 - 1 : 0;
         sub_ds = (p.taps == 9) ? tap % 3 - 1 : 0;
       }
@@ -103,11 +108,11 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
         if (lane == 0) mbar_expect_tx(&hdr->full[stage], tx_bytes);
         __syncwarp();
         if (lane < a_subs) {
-          if (sub_c < p.C0)
+          if (sub_c < C0p)
             tma_load_4d(sa + lane * p.a_sub_bytes, &tmA0, &hdr->full[stage], sub_c, w0 + sub_ds,
                         h0 + sub_dr, i0);
           else
-            tma_load_4d(sa + lane * p.a_sub_bytes, &tmA1, &hdr->full[stage], sub_c - p.C0, w0 + sub_ds,
+            tma_load_4d(sa + lane * p.a_sub_bytes, &tmA1, &hdr->full[stage], sub_c - C0p, w0 + sub_ds,
                         h0 + sub_dr, i0);
         } else if (lane - a_subs < b_subs) {
           const int j = lane - a_subs;
@@ -183,7 +188,12 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
       const int sp = it / (p.m_tiles * p.n_tiles);
       const int ch_begin = sp * per_split;
       const int as = n & 1;
-      const int m = mt * 128 + row;
+      // padded row -> (tap, source channel) -> row of the partial tile; padding rows are not stored
+      const int mp = mt * 128 + row;
+      const int cp = mp % Ctp;
+      const int cs = cp < C0p ? cp : cp - C0p;
+      const int m = (mp / Ctp) * Ctot + (cp < C0p ? cp : p.C0 + cs);
+      const bool real = mp < Mp && cs < (cp < C0p ? p.C0 : p.C1);
       const bool empty_split = ch_begin >= total_chunks;  // host never creates one; be safe
       mbar_wait(&hdr->tmem_full[as], (n >> 1) & 1);
       tc_fence_after();
@@ -193,7 +203,7 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
         tmem_ld32(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * bn_cols + j * 32, raw);
         tmem_ld_wait();
         const int cbase = nt * p.BN + j * 32;
-        if (m < Mtot) {
+        if (real) {
 #pragma unroll
           for (int g = 0; g < 8; ++g) {
             const int c = cbase + g * 4;
@@ -240,14 +250,18 @@ int conv_wgrad_launch(const ConvWgradArgs& a, cudaStream_t stream) {
   const int Ctot = a.C0 + a.C1;
   if (a.taps != 1 && a.taps != 9) return UB2_ERR_SHAPE;
   if (a.N <= 0 || a.H <= 0 || a.W <= 0 || a.C0 <= 0 || a.C1 < 0) return UB2_ERR_SHAPE;
-  if (Ctot % 16 != 0 || a.C0 % 16 != 0 || a.Cout % 16 != 0) return UB2_ERR_SHAPE;
+  if (a.Cout % 8 != 0) return UB2_ERR_SHAPE;   // any source channel count; Cout in 16-byte rows of dy
   if (g_conv_mode_wgrad != 1) {   // deep layers: two-CTA kernel sharing dy (conv_wgrad2.cu)
     const int rc2 = conv_wgrad2_launch(a, stream);
     if (rc2 != 1) return rc2;
   }
   if (a.ld_in0 % 8 != 0 || (a.C1 > 0 && a.ld_in1 % 8 != 0) || a.ld_dy % 8 != 0) return UB2_ERR_ALIGN;
+  // channels per A sub-box: 64, halved while it does not divide both sources, down to 16 (32 bytes: there is no
+  // 16-byte swizzle); sources that are not a multiple of it are padded to whole sub-boxes
   int mc = 64;
-  while (a.C0 % mc != 0 || Ctot % mc != 0) mc /= 2;
+  while (mc > 16 && (a.C0 % mc != 0 || Ctot % mc != 0)) mc /= 2;
+  const int C0p = (a.C0 + mc - 1) / mc * mc;
+  const int Mp = a.taps * (C0p + (a.C1 + mc - 1) / mc * mc);
 
   ConvWgradParams p{};
   p.N = a.N; p.H = a.H; p.W = a.W; p.C0 = a.C0; p.C1 = a.C1; p.Cout = a.Cout; p.taps = a.taps;
@@ -259,9 +273,9 @@ int conv_wgrad_launch(const ConvWgradArgs& a, cudaStream_t stream) {
   p.chunks_h = (a.H + p.BH - 1) / p.BH;
   p.chunks_n = (a.N + p.BI - 1) / p.BI;
   const int total_chunks = p.chunks_w * p.chunks_h * p.chunks_n;
-  const int Mtot = a.taps * Ctot;
-  p.m_tiles = (Mtot + 127) / 128;
-  const int BN = a.Cout <= 256 ? a.Cout : 256;
+  p.m_tiles = (Mp + 127) / 128;
+  // N tile rounded up to the MMA's multiple of 16: dy's tensor map zero-fills the channels past Cout
+  const int BN = a.Cout <= 256 ? (a.Cout + 15) & ~15 : 256;
   p.BN = BN;
   p.n_tiles = (a.Cout + BN - 1) / BN;
   const int bn_cols = (BN + 31) & ~31;

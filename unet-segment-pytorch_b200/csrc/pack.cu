@@ -116,8 +116,11 @@ pack_weight_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ fwd,
 }
 
 // Every conv weight of the network in one launch (the packs are rebuilt once per optimizer step):
-// desc[t] = {w, fwd, dgrad, Cout, Cin, taps} as int64, blocks[b] = {tensor, ci tile, co tile, -}.
-__global__ void __launch_bounds__(256)
+// desc[t] = {w, fwd, dgrad, Cout, Cin, taps} as int64, blocks[b] = {tensor, ci tile, co tile, edge}.
+// edge = 0: a whole 16x16 tile with Cin and Cout multiples of 8 (16-byte stores); otherwise the
+// generic tile (partial extents, element stores).
+// (min 8 blocks per SM: the register budget of the whole tiles alone; the edge path may spill)
+__global__ void __launch_bounds__(256, 8)
 pack_weights_multi_kernel(const long long* __restrict__ desc, const int4* __restrict__ blocks) {
   pdl_trigger();
   pdl_wait();
@@ -128,8 +131,14 @@ pack_weights_multi_kernel(const long long* __restrict__ desc, const int4* __rest
   __nv_bfloat16* fwd = reinterpret_cast<__nv_bfloat16*>(d[1]);
   __nv_bfloat16* dgrad = reinterpret_cast<__nv_bfloat16*>(d[2]);
   const int Cout = static_cast<int>(d[3]), Cin = static_cast<int>(d[4]);
-  if (d[5] == 9) pack_tile<9, true>(w, fwd, dgrad, Cout, Cin, nullptr, b.y, b.z, tile);
-  else pack_tile<1, true>(w, fwd, dgrad, Cout, Cin, nullptr, b.y, b.z, tile);
+  if (b.w != 0) {
+    if (d[5] == 9) pack_tile<9, false>(w, fwd, dgrad, Cout, Cin, nullptr, b.y, b.z, tile);
+    else pack_tile<1, false>(w, fwd, dgrad, Cout, Cin, nullptr, b.y, b.z, tile);
+  } else if (d[5] == 9) {
+    pack_tile<9, true>(w, fwd, dgrad, Cout, Cin, nullptr, b.y, b.z, tile);
+  } else {
+    pack_tile<1, true>(w, fwd, dgrad, Cout, Cin, nullptr, b.y, b.z, tile);
+  }
 }
 
 // Stage 1 of the split-K fold when there are many splits: partial[0][i] = sum_s partial[s][i],

@@ -86,20 +86,19 @@ def double_conv(module, x0, x1=None, pool_out=False):
     """DoubleConv (layers.py:16-41) on logical-NCHW inputs; returns (activation, pooled or None)."""
     _check(module, x0, x1)
     seq = module.double_conv
+    cin = x0.shape[1] + (x1.shape[1] if x1 is not None else 0)
+    # direct fp32 convolution (any Cin, e.g. the network stem) wherever its data gradient is not needed or fits
+    # (head.cu: Cin * 9 * Cout <= 12288 for 8 and more input channels); the rest on the tensor cores
+    needs_dx = torch.is_grad_enabled() and x0.requires_grad
+    stem = x1 is None and cin % 16 != 0 and (cin % 8 != 0 or not needs_dx or cin * 9 * seq[0].out_channels <= 12288)
     if _training_path(module, x0, x1):
-        cin = x0.shape[1] + (x1.shape[1] if x1 is not None else 0)
-        if cin % 16 != 0:
-            if x1 is not None:
-                raise RuntimeError("concatenated inputs need channel counts that are multiples of 16")
+        if stem:
             a = ConvInBnReluF32.apply(x0, seq[0].weight, seq[1].weight, seq[1].bias, seq[1])
         else:
             a, _ = ConvBnReluF32.apply(x0, x1, seq[0].weight, seq[1].weight, seq[1].bias, seq[1], False)
         return ConvBnReluF32.apply(a, None, seq[3].weight, seq[4].weight, seq[4].bias, seq[4], bool(pool_out))
-    cin = x0.shape[1] + (x1.shape[1] if x1 is not None else 0)
     s1, h1 = _bn_coeffs(seq[1])
-    if cin % 16 != 0:
-        if x1 is not None:
-            raise RuntimeError("concatenated inputs need channel counts that are multiples of 16")
+    if stem:
         a = K.f32_conv_in(x0.contiguous().float(), seq[0].weight, s1, h1)
     else:
         a = conv(nhwc(x0), nhwc(x1) if x1 is not None else None, seq[0].weight, s1, h1, relu=True)

@@ -181,14 +181,16 @@ class WeightPacker:
         for w in weights:
             cout, cin, kh, kw = w.shape
             taps = kh * kw
-            if not (w.is_cuda and w.dtype == F32 and w.is_contiguous() and cout % 16 == 0 and cin % 16 == 0
+            if not (w.is_cuda and w.dtype == F32 and w.is_contiguous() and cout % 8 == 0 and cin % 8 == 0
                     and taps in (1, 9)) or id(w) in self.entries:
                 continue
             fwd = torch.empty((cout, taps, cin), device=w.device, dtype=BF16)
             dg = torch.empty((cin, taps, cout), device=w.device, dtype=BF16)
             t = len(desc)
             desc.append([w.data_ptr(), fwd.data_ptr(), dg.data_ptr(), cout, cin, taps])
-            blocks += [[t, ci, co, 0] for co in range(cout // 16) for ci in range(cin // 16)]
+            # 4th field: a tile that reaches past Cin or Cout (channel counts not multiples of 16) -> edge path
+            blocks += [[t, ci, co, int(16 * ci + 16 > cin or 16 * co + 16 > cout)]
+                       for co in range((cout + 15) // 16) for ci in range((cin + 15) // 16)]
             self.entries[id(w)] = (w, w.data_ptr(), fwd, dg)
         self.nblocks = len(blocks)
         if self.nblocks:

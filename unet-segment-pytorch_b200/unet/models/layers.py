@@ -41,15 +41,23 @@ class DoubleConv(nn.Module):
         )
 
     def _run(self, x0, x1=None, pool_out: bool = False):
+        seq = self.double_conv
+        for c in (seq[0].out_channels, seq[3].out_channels) + ((x0.shape[1], x1.shape[1]) if x1 is not None else ()):
+            if c % 8 != 0:
+                raise RuntimeError(f"DoubleConv: {c} channels; unet-b200 needs every layer's channel count to be a "
+                                   "multiple of 8 (base_features a multiple of 8; any n_channels)")
         if fp32.active():
             return fp32.double_conv(self, x0, x1, pool_out)
-        seq = self.double_conv
         cin = x0.shape[1] + (x1.shape[1] if x1 is not None else 0)
-        if cin % 16 != 0:
+        if x1 is None and cin <= 4:
             # network stem: a handful of input channels, direct fp32 convolution
-            if x1 is not None:
-                raise RuntimeError("concatenated inputs need channel counts that are multiples of 16")
             a = ops.ConvInBnRelu.apply(x0, seq[0].weight, seq[1].weight, seq[1].bias, seq[1])
+        elif x1 is None and cin % 8 != 0:
+            # network input with more channels: zero channels up to a multiple of 8 (the activations' channel
+            # stride) in the input and the weight; autograd slices both gradients back
+            pad = -cin % 8
+            a, _ = ops.ConvBnRelu.apply(F.pad(x0, (0, 0, 0, 0, 0, pad)), None, F.pad(seq[0].weight, (0, 0, 0, 0, 0, pad)),
+                                        seq[1].weight, seq[1].bias, seq[1], False)
         else:
             a, _ = _stage(x0, x1, seq[0], seq[1])
         return _stage(a, None, seq[3], seq[4], pool=pool_out)
@@ -145,8 +153,8 @@ class _W:
 
 
 class _PaddedGate:
-    """An AttentionGate whose inter-channel count is not a multiple of 16 (base_features=16: 8 channels), seen
-    through padding: the tensor-core kernels need K and N in multiples of 16, so W_g / W_x get zero output rows,
+    """An AttentionGate whose inter-channel count is not a multiple of 16 (base_features=16: 8 channels, 24: 12),
+    seen through padding: the gate kernels need Ci in multiples of 16, so W_g / W_x get zero output rows,
     psi zero input columns and the two BatchNorms neutral channels.  The padded channels stay exactly zero through
     the gate (zero projection -> BatchNorm of a zero channel -> ReLU(0) -> zero psi weight), gradients reach the real
     parameters through the padding's own autograd, and the module's parameters / state_dict are untouched."""
@@ -183,8 +191,6 @@ class AttentionGate(nn.Module):
     def forward(self, g: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
         inter = self.W_g[0].weight.shape[0]
         if inter % 16 != 0:
-            if inter % 8 != 0:
-                raise RuntimeError("AttentionGate needs an inter-channel count that is a multiple of 8")
             view = _PaddedGate(self, 16 - inter % 16)
             out = self._gate(view, g, x)
             view.write_back()
