@@ -101,6 +101,13 @@ int ub2_pack_conv_weight(const float* w, void* fwd, void* dgrad, int Cout, int C
 int ub2_pack_conv_weights_multi(const long long* desc, const int* blocks, int nblocks, void* stream);
 
 /* ======================= BatchNorm / ReLU / MaxPool passes ============================== */
+/* The bf16 entry points below (BatchNorm, max-pool, attention gate, network ends, ConvTranspose2d pieces) check their
+ * arguments before the device is touched.  UB2_ERR_SHAPE: a count <= 0 (N, H, W, C, Ci, Cx, Cin, Cout, K, h, w, hin,
+ * win, splits), a channel count that is not a multiple of 8 or above the kernel's limit (named per entry point), a
+ * channel stride below its channel count, or a NULL pointer other than the optional ones named per entry point.
+ * UB2_ERR_ALIGN: a channel stride that is not a multiple of 8, a pointer read or written with 16-byte vectors (the
+ * NHWC bf16 tensors) that is not 16-byte aligned, pidx not 8-byte aligned, partials not 8-byte aligned, or an fp32
+ * pointer not 4-byte aligned.  UB2_ERR_WORKSPACE: rows other than the matching *_rows query. */
 
 /* nn.BatchNorm2d in train mode (layers.py:33,36,153,159,165): per-CTA sums -> batch mean and
  * biased variance; running_mean/var momentum update with the unbiased variance and
@@ -110,13 +117,14 @@ int ub2_bn_finalize(const double* partials, int rows, int C, double count, const
                     const float* beta, float* running_mean, float* running_var, long long* nbt,
                     float momentum, float eps, float* scale, float* shift, float* mean, float* invstd,
                     void* stream);
-/* nn.BatchNorm2d in eval mode: scale/shift from the running statistics. */
+/* nn.BatchNorm2d in eval mode: scale/shift from the running statistics; gamma / beta may be NULL (1 / 0). */
 int ub2_bn_eval_coeffs(const float* gamma, const float* beta, const float* running_mean,
                        const float* running_var, float eps, int C, float* scale, float* shift,
                        void* stream);
 /* a = relu(scale*y + shift) (nn.ReLU, layers.py:34,37) and, optionally, its 2x2 max-pooled copy
  * (nn.MaxPool2d(2) of Down, layers.py:56) with pidx (N,H/2,W/2,C) uint8 = window position of each
- * maximum (first maximum wins, as ATen); a, pooled, pidx may be NULL; scale/shift NULL = identity. */
+ * maximum (first maximum wins, as ATen); a, pooled, pidx may be NULL; scale/shift NULL = identity.
+ * C <= 2048; y, ld_y required; ld_a / ld_p are checked only with a / pooled. */
 int ub2_bn_act(const void* y, int ld_y, const float* scale, const float* shift, void* a, int ld_a,
                void* pooled, int ld_p, unsigned char* pidx, int N, int H, int W, int C, int relu,
                void* stream);
@@ -125,7 +133,8 @@ int ub2_bn_act(const void* y, int ld_y, const float* scale, const float* shift, 
  *   reduce  : rows of (sum g, sum g*y);  rows = ub2_bn_bwd_rows(...)
  *   finalize: dgamma/dbeta (+= into the fp32 .grad) and coef (3,C): dy = c0*g + c1*y + c2
  *             (frozen != 0: eval-mode statistics, c1 = c2 = 0)
- *   apply   : dy bf16.  dA or dP may be NULL. */
+ *   apply   : dy bf16.  dA or dP may be NULL (not both; dP needs pidx; ld_da / ld_dp are then ignored);
+ *             y, scale, shift, partials / coef and dY are required.  C <= 2048. */
 int ub2_bn_bwd_rows(int N, int H, int W, int C, int pool);
 int ub2_bn_bwd_reduce(const void* dA, int ld_da, const void* dP, int ld_dp, const unsigned char* pidx,
                       const void* y, int ld_y, const float* scale, const float* shift, double* partials,
@@ -151,7 +160,8 @@ int ub2_upsample_bwd(const void* dout, int ld_dout, void* din, int ld_din, int a
  * convolution itself is ub2_conv_fwd with the (4*Cout, Cin) reshaped weight (row (i,j,co)) and the bias in its
  * epilogue; these are the pixel shuffle out[n, 2y+i+py, 2x+j+px, co] = t[n, y, x, (i*2+j)*C + co] with the
  * padding of F.pad (zeros), its transpose, and the bias gradient: dbias[co] += sum of the gathered dout.
- * `partials`: (rows, C) doubles with rows = ub2_shuffle2x2_rows(...); pass NULL to skip the bias gradient. */
+ * `partials`: (rows, C) doubles with rows = ub2_shuffle2x2_rows(...); pass NULL (and dbias NULL) to skip the bias
+ * gradient.  t / dt have channel strides >= 4*C, out / dout >= C; C <= 2048 for the backward. */
 int ub2_shuffle2x2_fwd(const void* t, int ld_t, void* out, int ld_out, int N, int h, int w, int C, int Ho, int Wo,
                        void* stream);
 int ub2_shuffle2x2_rows(int N, int h, int w, int C, int Ho, int Wo);
@@ -159,7 +169,7 @@ int ub2_shuffle2x2_bwd(const void* dout, int ld_dout, void* dt, int ld_dt, doubl
                        int N, int h, int w, int C, int Ho, int Wo, void* stream);
 /* The (Cin, Cout, 2, 2) fp32 ConvTranspose2d parameter as 1x1-convolution packs: fwd (4*Cout, Cin) bf16 with row
  * (i*2+j)*Cout + co, dg (Cin, 4*Cout) bf16, and the epilogue vectors scale4 = 1, shift4 = bias tiled four times
- * (each 4*Cout floats; bias may be NULL).  Any output pointer may be NULL. */
+ * (each 4*Cout floats; bias may be NULL).  Any output pointer may be NULL, but scale4 and shift4 only together. */
 int ub2_pack_convt_weight(const float* w, const float* bias, void* fwd, void* dg, float* scale4, float* shift4,
                           int Cin, int Cout, void* stream);
 /* grad (Cin, Cout, 2, 2) fp32 = (or +=) the split-K partials (splits, Cin, 4*Cout) of ub2_conv_wgrad(taps = 1) on
@@ -183,6 +193,10 @@ int ub2_gate_strip_rows(int N, int H, int W, int C);
  * (layers.py:183,186) without materialising the up-sampled tensor. */
 int ub2_gate_upstats(const void* q, int ld_q, int N, int hin, int win, int H, int W, int Ci,
                      double* partials, int rows, void* stream);
+/* The strip passes (upstats, psi, fused_eval, bwd_s, bwd_xg) take Ci <= 512 and (hin - 1) < 2 (H - 1) (a ring of at
+ * most 8 low-resolution rows; a stronger down-sampling is UB2_ERR_SHAPE);
+ * gate_bwd_a takes Cx <= 512, gate_apply any Cx.  Every pointer is required except partials of ub2_gate_psi (no
+ * statistics) and a_out of ub2_gate_apply. */
 /* psi_raw = w_psi . relu(BN_g(up q) + BN_x(xp)) (layers.py:188, :164) + rows of (sum, sum sq). */
 int ub2_gate_psi(const void* q, int ld_q, const void* xp, int ld_xp, const float* scale_g,
                  const float* shift_g, const float* scale_x, const float* shift_x, const float* wpsi,
@@ -190,8 +204,10 @@ int ub2_gate_psi(const void* q, int ld_q, const void* xp, int ld_xp, const float
                  int Ci, void* stream);
 /* a = sigmoid(BN_psi(psi_raw)); out = x * a (layers.py:165-166, :192). */
 /* Inference only (BatchNorm frozen, nothing saved): psi, sigmoid and out = x * a in ONE pass over q, xp and x
- * (north_star (3)); needs Cx == 2 * Ci (layers.py:147-148's default inter-channel count), else UB2_ERR_SHAPE and the
- * caller runs ub2_gate_psi + ub2_gate_apply. */
+ * (north_star (3)); needs Cx == 2 * Ci (layers.py:147-148's default inter-channel count) and, for Ci > 256, a
+ * 4-row ring, 3 (hin - 1) < 2 (H - 1) (the U-Net's 2x up-sampling): its 8-row ring would not fit a block's shared
+ * memory.  Else UB2_ERR_SHAPE, and the caller runs ub2_gate_psi + ub2_gate_apply.  ub2_gate_bwd_xg likewise needs
+ * the 4-row ring for Ci > 336. */
 int ub2_gate_fused_eval(const void* q, int ld_q, const void* xp, int ld_xp, const void* x, int ld_x, const float* scale_g,
                         const float* shift_g, const float* scale_x, const float* shift_x, const float* wpsi,
                         const float* scale_psi, const float* shift_psi, void* out, int ld_out, int N, int hin, int win,
@@ -220,7 +236,10 @@ int ub2_gate_bwd_xg(const void* ds, int ld_ds, const void* xp, int ld_xp, const 
 /* ======================= network ends =================================================== */
 
 /* inc.double_conv.0 (layers.py:32 with in_channels = n_channels <= 4): direct fp32 conv of the
- * fp32 NCHW input, NHWC bf16 output + BatchNorm statistic rows; and its weight gradient. */
+ * fp32 NCHW input, NHWC bf16 output + BatchNorm statistic rows (partials may be NULL); and its weight gradient
+ * (grad +=).  1 <= Cin <= 4, Cout <= 2048; partials and grad 8- / 4-byte aligned.  Outside the register-window
+ * variant (Cin == 1, W % 4 == 0, x 16-byte aligned) the forward keeps the Cin * 9 * Cout weights and 16 floats per
+ * thread of its (at most 256-thread) block in 48 KB of shared memory; a larger product is UB2_ERR_SHAPE. */
 int ub2_conv_in_rows(int N, int H, int W, int Cout);
 int ub2_conv_in_fwd(const float* x, const float* w, void* y, int ld_y, double* partials, int rows, int N,
                     int Cin, int H, int W, int Cout, void* stream);
@@ -232,7 +251,8 @@ int ub2_conv_in_wgrad(const float* x, const void* dy, int ld_dy, double* partial
  * for Cin > 1, W % 4 != 0 or pointers not 16-byte aligned also Cin * 9 * Cout <= 12288. */
 int ub2_conv_in_dgrad(const void* dy, int ld_dy, const float* w, float* dx, int N, int Cin, int H, int W, int Cout,
                       void* stream);
-/* OutConv (layers.py:120-123): 1x1 conv with bias to fp32 NCHW logits, and its backward. */
+/* OutConv (layers.py:120-123): 1x1 conv with bias to fp32 NCHW logits, and its backward.  1 <= K <= 8; the backward
+ * takes C <= 512.  bias, da, dw and db may be NULL (dw and db accumulate: +=); a and w are 16-byte aligned. */
 int ub2_outc_rows(int N, int H, int W, int C);
 int ub2_outc_fwd(const void* a, int ld_a, const float* w, const float* bias, float* logits, int N, int H,
                  int W, int C, int K, void* stream);

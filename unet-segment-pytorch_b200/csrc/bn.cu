@@ -347,6 +347,7 @@ __global__ void bn_bwd_finalize_kernel(const double* __restrict__ partials, int 
 }
 
 static int bn_block(int cgs) { return cgs * (kBnThreads / cgs); }
+static bool al16(const void* p) { return aligned_to(p, 16); }
 
 }  // namespace ub2
 
@@ -366,7 +367,8 @@ int ub2_bn_finalize(const double* partials, int rows, int C, double count, const
 int ub2_bn_eval_coeffs(const float* gamma, const float* beta, const float* running_mean,
                        const float* running_var, float eps, int C, float* scale, float* shift,
                        void* stream) {
-  if (C <= 0) return UB2_ERR_SHAPE;
+  if (C <= 0 || running_mean == nullptr || running_var == nullptr || scale == nullptr || shift == nullptr)
+    return UB2_ERR_SHAPE;
   launch(bn_eval_coeffs_kernel, (C + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream), gamma, beta, running_mean, running_var, eps, C, scale, shift);
   return static_cast<int>(cudaGetLastError());
 }
@@ -376,7 +378,9 @@ int ub2_bn_act(const void* y, int ld_y, const float* scale, const float* shift, 
                void* stream) {
   if (C <= 0 || C % 8 != 0 || C / 8 > kBnThreads || N <= 0 || H <= 0 || W <= 0 || !fits32(N, H, W, C))
     return UB2_ERR_SHAPE;
+  if (y == nullptr || ld_y < C || (a && ld_a < C) || (pooled && ld_p < C)) return UB2_ERR_SHAPE;
   if (ld_y % 8 || (a && ld_a % 8) || (pooled && ld_p % 8)) return UB2_ERR_ALIGN;
+  if (!al16(y) || !al16(a) || !al16(pooled) || !aligned_to(pidx, 8)) return UB2_ERR_ALIGN;
   WinGeom g = make_geom(N, H, W, C);
   const int block = bn_block(g.cgs);
   const int lanes = block / g.cgs;
@@ -395,6 +399,20 @@ int ub2_bn_act(const void* y, int ld_y, const float* scale, const float* shift, 
   return static_cast<int>(cudaGetLastError());
 }
 
+// Arguments shared by the reduce and apply passes: dA and dP optional (not both; dP needs pidx), every other
+// pointer required, channel strides >= C and multiples of 8, 128-bit-accessed pointers 16-byte aligned.
+static int bwd_check(const void* dA, int ld_da, const void* dP, int ld_dp, const unsigned char* pidx, const void* y,
+                     int ld_y, const float* scale, const float* shift, int N, int H, int W, int C) {
+  if (C <= 0 || C % 8 != 0 || C / 8 > kBnThreads || N <= 0 || H <= 0 || W <= 0 || !fits32(N, H, W, C))
+    return UB2_ERR_SHAPE;
+  if ((dA == nullptr && dP == nullptr) || (dP != nullptr && pidx == nullptr)) return UB2_ERR_SHAPE;
+  if (y == nullptr || scale == nullptr || shift == nullptr) return UB2_ERR_SHAPE;
+  if (ld_y < C || (dA && ld_da < C) || (dP && ld_dp < C)) return UB2_ERR_SHAPE;
+  if (ld_y % 8 || (dA && ld_da % 8) || (dP && ld_dp % 8)) return UB2_ERR_ALIGN;
+  if (!al16(y) || !al16(dA) || !al16(dP) || !aligned_to(pidx, 8)) return UB2_ERR_ALIGN;
+  return 0;
+}
+
 static int bwd_items(const WinGeom& g, bool pool) {
   return pool ? g.windows : static_cast<int>(g.N) * g.H * g.W;
 }
@@ -409,9 +427,10 @@ int ub2_bn_bwd_rows(int N, int H, int W, int C, int pool) {
 int ub2_bn_bwd_reduce(const void* dA, int ld_da, const void* dP, int ld_dp, const unsigned char* pidx,
                       const void* y, int ld_y, const float* scale, const float* shift, double* partials,
                       int rows, int N, int H, int W, int C, int relu, void* stream) {
-  if (C <= 0 || C % 8 != 0 || C / 8 > kBnThreads || N <= 0 || H <= 0 || W <= 0 || !fits32(N, H, W, C))
-    return UB2_ERR_SHAPE;
-  if ((dA == nullptr && dP == nullptr) || (dP != nullptr && pidx == nullptr)) return UB2_ERR_SHAPE;
+  const int rc = bwd_check(dA, ld_da, dP, ld_dp, pidx, y, ld_y, scale, shift, N, H, W, C);
+  if (rc) return rc;
+  if (partials == nullptr) return UB2_ERR_SHAPE;
+  if (!aligned_to(partials, 8)) return UB2_ERR_ALIGN;
   WinGeom g = make_geom(N, H, W, C);
   const bool pool = dP != nullptr;
   const int block = bn_block(g.cgs);
@@ -438,9 +457,10 @@ int ub2_bn_bwd_finalize(const double* partials, int rows, int C, double count, c
 int ub2_bn_bwd_apply(const void* dA, int ld_da, const void* dP, int ld_dp, const unsigned char* pidx,
                      const void* y, int ld_y, const float* scale, const float* shift, const float* coef,
                      void* dY, int ld_dy, int N, int H, int W, int C, int relu, void* stream) {
-  if (C <= 0 || C % 8 != 0 || C / 8 > kBnThreads || N <= 0 || H <= 0 || W <= 0 || !fits32(N, H, W, C))
-    return UB2_ERR_SHAPE;
-  if ((dA == nullptr && dP == nullptr) || (dP != nullptr && pidx == nullptr)) return UB2_ERR_SHAPE;
+  const int rc = bwd_check(dA, ld_da, dP, ld_dp, pidx, y, ld_y, scale, shift, N, H, W, C);
+  if (rc) return rc;
+  if (coef == nullptr || dY == nullptr || ld_dy < C) return UB2_ERR_SHAPE;
+  if (ld_dy % 8 || !al16(dY)) return UB2_ERR_ALIGN;
   WinGeom g = make_geom(N, H, W, C);
   const bool pool = dP != nullptr;
   const int block = bn_block(g.cgs);

@@ -44,7 +44,7 @@ static int gate_tpp(int cgs) {
   return t;
 }
 static int make_gate_geom(GateGeom* g, int N, int H, int W, int C, int hin, int win) {
-  if (C <= 0 || C % 8 != 0 || N <= 0 || H <= 0 || W <= 0) return UB2_ERR_SHAPE;
+  if (C <= 0 || C % 8 != 0 || N <= 0 || H <= 0 || W <= 0 || hin <= 0 || win <= 0) return UB2_ERR_SHAPE;
   if (static_cast<double>(N) * H * W * (C / 8) >= 2.0e9) return UB2_ERR_SHAPE;  // 32-bit pixel indices
   g->N = N; g->H = H; g->W = W; g->C = C; g->cgs = C / 8;
   g->tpp = gate_tpp(g->cgs);
@@ -53,10 +53,17 @@ static int make_gate_geom(GateGeom* g, int N, int H, int W, int C, int hin, int 
   g->pixels = static_cast<int>(N) * H * W;
   g->wt = (W + g->slots - 1) / g->slots;
   g->ht = (H + kGateStrip - 1) / kGateStrip;
-  g->lr = make_lowres(hin > 0 ? hin : 1, win > 0 ? win : 1, H, W);
+  g->lr = make_lowres(hin, win, H, W);
   return 0;
 }
 static int gate_strip_grid(const GateGeom& g) { return g.wt * g.ht * g.N; }
+static bool al16(const void* p) { return aligned_to(p, 16); }
+// A bf16 NHWC operand of C channels read or written with 16-byte vectors: UB2_ERR_SHAPE for a NULL pointer or a
+// channel stride below C, UB2_ERR_ALIGN for a stride that is not a multiple of 8 or a pointer off 16 bytes.
+static int vec_operand(const void* p, int ld, int C) {
+  if (p == nullptr || ld < C) return UB2_ERR_SHAPE;
+  return (ld % 8 || !al16(p)) ? UB2_ERR_ALIGN : 0;
+}
 static int gate_grid(const GateGeom& g, int per_sm) {
   return stream_grid(g.pixels, g.slots, num_sms(), per_sm);
 }
@@ -782,6 +789,11 @@ static int strip_qr(const GateGeom& g) {
   if (alive <= 8) return 8;
   return 0;
 }
+// Dynamic shared memory the strip kernels opt in to (their static shared memory stays within the 227 KB of a block).
+// A <G, QR> ring plus its coefficient vectors above it cannot launch, so the entry point refuses the shape: at two
+// channel groups per thread (Ci > 256) with the 8-row ring, gate_fused_eval (its caller runs gate_psi + gate_apply
+// instead) and gate_bwd_xg (Ci > 336).
+static constexpr size_t kStripSmemMax = 200 * 1024;
 // Opt in to > 48 KB of dynamic shared memory once per (kernel, device).
 static int strip_smem_attr(const void* fn, size_t bytes) {
   if (bytes <= 48 * 1024) return 0;
@@ -791,7 +803,7 @@ static int strip_smem_attr(const void* fn, size_t bytes) {
   std::lock_guard<std::mutex> lock(mu);
   for (const auto& d : done)
     if (d.first == fn && d.second == dev) return 0;
-  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kStripSmemMax));
   if (e != cudaSuccess) return static_cast<int>(e);
   done.emplace_back(fn, dev);
   return 0;
@@ -806,18 +818,22 @@ static int strip_smem_attr(const void* fn, size_t bytes) {
     int rc_ = 0;                                                                                            \
     if (!g2_ && qr_ == 4) {                                                                                 \
       const size_t sm_ = Strip<1, 4, NV, NS>::kBytes + coef_;                                               \
+      if (sm_ > kStripSmemMax) return UB2_ERR_SHAPE;                                                        \
       rc_ = strip_smem_attr(reinterpret_cast<const void*>(&KERNEL<1, 4>), sm_);                            \
       if (!rc_) launch(KERNEL<1, 4>, grid, kGateThreads, sm_, s, __VA_ARGS__);                              \
     } else if (!g2_) {                                                                                      \
       const size_t sm_ = Strip<1, 8, NV, NS>::kBytes + coef_;                                               \
+      if (sm_ > kStripSmemMax) return UB2_ERR_SHAPE;                                                        \
       rc_ = strip_smem_attr(reinterpret_cast<const void*>(&KERNEL<1, 8>), sm_);                            \
       if (!rc_) launch(KERNEL<1, 8>, grid, kGateThreads, sm_, s, __VA_ARGS__);                              \
     } else if (qr_ == 4) {                                                                                  \
       const size_t sm_ = Strip<2, 4, NV, NS>::kBytes + coef_;                                               \
+      if (sm_ > kStripSmemMax) return UB2_ERR_SHAPE;                                                        \
       rc_ = strip_smem_attr(reinterpret_cast<const void*>(&KERNEL<2, 4>), sm_);                            \
       if (!rc_) launch(KERNEL<2, 4>, grid, kGateThreads, sm_, s, __VA_ARGS__);                              \
     } else {                                                                                                \
       const size_t sm_ = Strip<2, 8, NV, NS>::kBytes + coef_;                                               \
+      if (sm_ > kStripSmemMax) return UB2_ERR_SHAPE;                                                        \
       rc_ = strip_smem_attr(reinterpret_cast<const void*>(&KERNEL<2, 8>), sm_);                            \
       if (!rc_) launch(KERNEL<2, 8>, grid, kGateThreads, sm_, s, __VA_ARGS__);                              \
     }                                                                                                       \
@@ -851,6 +867,9 @@ int ub2_gate_upstats(const void* q, int ld_q, int N, int hin, int win, int H, in
   GateGeom g;
   int rc = make_gate_geom(&g, N, H, W, Ci, hin, win);
   if (rc) return rc;
+  if (partials == nullptr) return UB2_ERR_SHAPE;
+  if ((rc = vec_operand(q, ld_q, Ci))) return rc;
+  if (!aligned_to(partials, 8)) return UB2_ERR_ALIGN;
   const int grid = gate_strip_grid(g);
   if (grid != rows) return UB2_ERR_WORKSPACE;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -873,6 +892,9 @@ int ub2_gate_psi(const void* q, int ld_q, const void* xp, int ld_xp, const float
   GateGeom g;
   int rc = make_gate_geom(&g, N, H, W, Ci, hin, win);
   if (rc) return rc;
+  if (!scale_g || !shift_g || !scale_x || !shift_x || !wpsi || !psi_raw) return UB2_ERR_SHAPE;
+  if ((rc = vec_operand(q, ld_q, Ci)) || (rc = vec_operand(xp, ld_xp, Ci))) return rc;
+  if (!aligned_to(psi_raw, 4) || !aligned_to(partials, 8)) return UB2_ERR_ALIGN;
   const int grid = gate_strip_grid(g);
   if (partials != nullptr && grid != rows) return UB2_ERR_WORKSPACE;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -889,7 +911,10 @@ int ub2_gate_fused_eval(const void* q, int ld_q, const void* xp, int ld_xp, cons
   GateGeom g;
   int rc = make_gate_geom(&g, N, H, W, Ci, hin, win);
   if (rc) return rc;
-  if (ld_x % 8 || ld_out % 8 || ld_xp % 8 || ld_q % 8) return UB2_ERR_ALIGN;
+  if (!scale_g || !shift_g || !scale_x || !shift_x || !wpsi || !scale_psi || !shift_psi) return UB2_ERR_SHAPE;
+  if ((rc = vec_operand(q, ld_q, Ci)) || (rc = vec_operand(xp, ld_xp, Ci)) || (rc = vec_operand(x, ld_x, Cx)) ||
+      (rc = vec_operand(out, ld_out, Cx)))
+    return rc;
   const int grid = gate_strip_grid(g);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   GATE_STRIP_DISPATCH(gate_fused_eval_kernel, 3, 0, 4 * Ci, static_cast<cbf>(q), ld_q, static_cast<cbf>(xp), ld_xp, static_cast<cbf>(x),
@@ -900,7 +925,12 @@ int ub2_gate_fused_eval(const void* q, int ld_q, const void* xp, int ld_xp, cons
 int ub2_gate_apply(const float* psi_raw, const float* scale_psi, const float* shift_psi, const void* x,
                    int ld_x, void* out, int ld_out, float* a_out, int N, int H, int W, int Cx,
                    void* stream) {
-  if (Cx % 8 != 0 || N <= 0 || static_cast<double>(N) * H * W * (Cx / 8) >= 2.0e9) return UB2_ERR_SHAPE;
+  if (Cx <= 0 || Cx % 8 != 0 || N <= 0 || H <= 0 || W <= 0 || static_cast<double>(N) * H * W * (Cx / 8) >= 2.0e9)
+    return UB2_ERR_SHAPE;
+  if (!psi_raw || !scale_psi || !shift_psi) return UB2_ERR_SHAPE;
+  int rc;
+  if ((rc = vec_operand(x, ld_x, Cx)) || (rc = vec_operand(out, ld_out, Cx))) return rc;
+  if (!aligned_to(psi_raw, 4) || !aligned_to(a_out, 4)) return UB2_ERR_ALIGN;
   const int pixels = static_cast<int>(N) * H * W;
   launch(gate_apply_kernel, stream_grid(pixels * (Cx / 8), 256, num_sms()), 256, 0, static_cast<cudaStream_t>(stream), psi_raw, scale_psi, shift_psi, static_cast<cbf>(x), ld_x, static_cast<bf>(out), ld_out, a_out, pixels, Cx / 8);
   return static_cast<int>(cudaGetLastError());
@@ -912,6 +942,9 @@ int ub2_gate_bwd_a(const void* dout, int ld_do, const void* x, int ld_x, const f
   GateGeom g;
   int rc = make_gate_geom(&g, N, H, W, Cx, 1, 1);
   if (rc) return rc;
+  if (!a || !psi_raw || !dpsin || !partials) return UB2_ERR_SHAPE;
+  if ((rc = vec_operand(dout, ld_do, Cx)) || (rc = vec_operand(x, ld_x, Cx)) || (rc = vec_operand(dx, ld_dx, Cx))) return rc;
+  if (!aligned_to(a, 4) || !aligned_to(psi_raw, 4) || !aligned_to(dpsin, 4) || !aligned_to(partials, 8)) return UB2_ERR_ALIGN;
   const int grid = gate_grid(g, 8);
   if (grid != rows) return UB2_ERR_WORKSPACE;
   if (g.cgs > g.tpp)
@@ -929,6 +962,10 @@ int ub2_gate_bwd_s(const float* dpsin, const float* psi_raw, const float* coef_p
   GateGeom g;
   int rc = make_gate_geom(&g, N, H, W, Ci, hin, win);
   if (rc) return rc;
+  if (!dpsin || !psi_raw || !coef_psi || !scale_g || !shift_g || !scale_x || !shift_x || !wpsi || !partials)
+    return UB2_ERR_SHAPE;
+  if ((rc = vec_operand(q, ld_q, Ci)) || (rc = vec_operand(xp, ld_xp, Ci)) || (rc = vec_operand(ds, ld_ds, Ci))) return rc;
+  if (!aligned_to(dpsin, 4) || !aligned_to(psi_raw, 4) || !aligned_to(partials, 8)) return UB2_ERR_ALIGN;
   const int grid = gate_strip_grid(g);
   if (grid != rows) return UB2_ERR_WORKSPACE;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -953,6 +990,10 @@ int ub2_gate_bwd_xg(const void* ds, int ld_ds, const void* xp, int ld_xp, const 
   GateGeom g;
   int rc = make_gate_geom(&g, N, H, W, Ci, hin, win);
   if (rc) return rc;
+  if (coef == nullptr) return UB2_ERR_SHAPE;
+  if ((rc = vec_operand(ds, ld_ds, Ci)) || (rc = vec_operand(xp, ld_xp, Ci)) || (rc = vec_operand(q, ld_q, Ci)) ||
+      (rc = vec_operand(dxp, ld_dxp, Ci)) || (rc = vec_operand(dgup, ld_dg, Ci)))
+    return rc;
   const int grid = gate_strip_grid(g);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   GATE_STRIP_DISPATCH(gate_bwd_xg_kernel, 2, 0, 6 * Ci, static_cast<cbf>(ds), ld_ds, static_cast<cbf>(xp), ld_xp, static_cast<cbf>(q),

@@ -727,6 +727,21 @@ __global__ void outc_bwd_finalize_kernel(const double* __restrict__ partials, in
   }
 }
 
+static bool al16(const void* p) { return aligned_to(p, 16); }
+
+// The stem convolution's arguments (forward and weight gradient): counts > 0, 1 <= Cin <= kMaxCin, Cout a multiple of
+// 8 with at most kHeadThreads groups of 8, x and w required, the NHWC bf16 side (y or dy) with a channel stride
+// >= Cout that is a multiple of 8 and a 16-byte-aligned pointer.
+static int conv_in_check(const float* x, const float* w, const void* nhwc, int ld, int N, int Cin, int H, int W,
+                         int Cout) {
+  if (N <= 0 || H <= 0 || W <= 0 || Cout <= 0 || Cout % 8 != 0 || Cout / 8 > kHeadThreads || Cin < 1 || Cin > kMaxCin)
+    return UB2_ERR_SHAPE;
+  if (static_cast<double>(N) * H * W * Cin >= 2.0e9) return UB2_ERR_SHAPE;  // 32-bit pixel indices
+  if (x == nullptr || w == nullptr || nhwc == nullptr || ld < Cout) return UB2_ERR_SHAPE;
+  if (ld % 8 || !al16(nhwc) || !aligned_to(x, 4) || !aligned_to(w, 4)) return UB2_ERR_ALIGN;
+  return 0;
+}
+
 static int head_geom(HeadGeom* g, int N, int H, int W, int C, int K) {
   if (C <= 0 || C % 8 != 0 || K < 1 || K > kMaxClasses || N <= 0 || H <= 0 || W <= 0) return UB2_ERR_SHAPE;
   if (static_cast<double>(N) * H * W * K >= 2.0e9) return UB2_ERR_SHAPE;  // 32-bit pixel indices
@@ -754,15 +769,20 @@ int ub2_conv_in_rows(int N, int H, int W, int Cout) {
 
 int ub2_conv_in_fwd(const float* x, const float* w, void* y, int ld_y, double* partials, int rows, int N,
                     int Cin, int H, int W, int Cout, void* stream) {
-  if (Cout % 8 != 0 || Cout / 8 > kHeadThreads || Cin < 1 || Cin > kMaxCin) return UB2_ERR_SHAPE;
-  if (static_cast<double>(N) * H * W * Cin >= 2.0e9) return UB2_ERR_SHAPE;  // 32-bit pixel indices
+  const int rc = conv_in_check(x, w, y, ld_y, N, Cin, H, W, Cout);
+  if (rc) return rc;
+  if (!aligned_to(partials, 8)) return UB2_ERR_ALIGN;
   const int cgs = Cout / 8;
   const int block = cgs * (kHeadThreads / cgs);
   const int lanes = block / cgs;
+  // the general variant keeps the weights and the statistics lanes in the 48 KB of dynamic shared memory that
+  // needs no opt-in; the register-window variant (Cin == 1, W % 4 == 0, x 16-byte aligned) only the lanes
+  const bool four = Cin == 1 && W % 4 == 0 && al16(x);
+  const size_t smem = (static_cast<size_t>(Cin) * 9 * Cout + static_cast<size_t>(lanes) * cgs * 16) * sizeof(float);
+  if (!four && smem > 48 * 1024) return UB2_ERR_SHAPE;
   const int grid = stream_grid(static_cast<int>(N) * H * W, lanes, num_sms(), 4);
   if (partials != nullptr && grid != rows) return UB2_ERR_WORKSPACE;
-  const size_t smem = (static_cast<size_t>(Cin) * 9 * Cout + static_cast<size_t>(lanes) * cgs * 16) * sizeof(float);
-  if (Cin == 1 && W % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0)
+  if (four)
     launch(conv_in_fwd4_kernel, grid, block, static_cast<size_t>(lanes) * cgs * 16 * sizeof(float), static_cast<cudaStream_t>(stream), x, w, static_cast<__nv_bfloat16*>(y), ld_y, partials, N, H, W, Cout);
   else if (Cin == 1)
     launch(conv_in_fwd_kernel<true>, grid, block, smem, static_cast<cudaStream_t>(stream), x, w, static_cast<__nv_bfloat16*>(y), ld_y, partials, N, Cin, H, W, Cout);
@@ -773,8 +793,10 @@ int ub2_conv_in_fwd(const float* x, const float* w, void* y, int ld_y, double* p
 
 int ub2_conv_in_wgrad(const float* x, const void* dy, int ld_dy, double* partials, int rows, float* grad,
                       int N, int Cin, int H, int W, int Cout, void* stream) {
-  if (Cout % 8 != 0 || Cout / 8 > kHeadThreads || Cin < 1 || Cin > kMaxCin) return UB2_ERR_SHAPE;
-  if (static_cast<double>(N) * H * W * Cin >= 2.0e9) return UB2_ERR_SHAPE;  // 32-bit pixel indices
+  const int rc = conv_in_check(x, grad, dy, ld_dy, N, Cin, H, W, Cout);
+  if (rc) return rc;
+  if (partials == nullptr) return UB2_ERR_SHAPE;
+  if (!aligned_to(partials, 8)) return UB2_ERR_ALIGN;
   const int cgs = Cout / 8;
   const int block = cgs * (kHeadThreads / cgs);
   const int lanes = block / cgs;
@@ -782,8 +804,7 @@ int ub2_conv_in_wgrad(const float* x, const void* dy, int ld_dy, double* partial
   if (grid != rows) return UB2_ERR_WORKSPACE;
   const size_t smem = static_cast<size_t>(lanes) * cgs * 8 * sizeof(float);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (Cin == 1 && W % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
-      static_cast<double>(N) * H * W < 4.0e9)
+  if (Cin == 1 && W % 4 == 0 && al16(x) && static_cast<double>(N) * H * W < 4.0e9)
     launch(conv_in_wgrad4_kernel, grid, block, smem, s, x, static_cast<const __nv_bfloat16*>(dy), ld_dy, partials, N, H, W, Cout);
   else
     launch(conv_in_wgrad_kernel, dim3(grid, Cin), block, smem, s, x, static_cast<const __nv_bfloat16*>(dy), ld_dy, partials, N, Cin, H, W, Cout);
@@ -824,6 +845,8 @@ int ub2_outc_fwd(const void* a, int ld_a, const float* w, const float* bias, flo
   HeadGeom g;
   int rc = head_geom(&g, N, H, W, C, K);
   if (rc) return rc;
+  if (a == nullptr || w == nullptr || logits == nullptr || ld_a < C) return UB2_ERR_SHAPE;
+  if (ld_a % 8 || !al16(a) || !al16(w) || !aligned_to(bias, 4) || !aligned_to(logits, 4)) return UB2_ERR_ALIGN;
   const int grid = stream_grid((g.pixels + 3) / 4, g.slots, num_sms(), 8);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const __nv_bfloat16* ap = static_cast<const __nv_bfloat16*>(a);
@@ -840,6 +863,11 @@ int ub2_outc_bwd(const float* dlogits, const void* a, int ld_a, const float* w, 
   int rc = head_geom(&g, N, H, W, C, K);
   if (rc) return rc;
   if (g.cgs > 2 * g.tpp) return UB2_ERR_SHAPE;
+  if (dlogits == nullptr || a == nullptr || w == nullptr || partials == nullptr || ld_a < C || (da && ld_da < C))
+    return UB2_ERR_SHAPE;
+  if (ld_a % 8 || (da && ld_da % 8) || !al16(a) || !al16(da) || !al16(w) || !aligned_to(dlogits, 4) ||
+      !aligned_to(partials, 8) || !aligned_to(dw, 4) || !aligned_to(db, 4))
+    return UB2_ERR_ALIGN;
   const int grid = stream_grid(g.pixels, g.slots, num_sms(), 4);
   if (grid != rows) return UB2_ERR_WORKSPACE;
   cudaStream_t s = static_cast<cudaStream_t>(stream);

@@ -189,7 +189,8 @@ int ub2_shuffle2x2_fwd(const void* t, int ld_t, void* out, int ld_out, int N, in
   ShufGeom g;
   int rc = shuf_geom(&g, N, h, w, C, Ho, Wo);
   if (rc) return rc;
-  if (ld_t % 8 || ld_out % 8) return UB2_ERR_ALIGN;
+  if (t == nullptr || out == nullptr || ld_t < 4 * C || ld_out < C) return UB2_ERR_SHAPE;
+  if (ld_t % 8 || ld_out % 8 || !al16(t) || !al16(out)) return UB2_ERR_ALIGN;
   const long long total = static_cast<long long>(N) * Ho * Wo * g.cgs;
   launch(shuffle2x2_fwd_kernel<__nv_bfloat16>, stream_grid(total, 256, num_sms(), 8), 256, 0, static_cast<cudaStream_t>(stream),
          static_cast<const __nv_bfloat16*>(t), ld_t, static_cast<__nv_bfloat16*>(out), ld_out, g);
@@ -210,21 +211,27 @@ int ub2_shuffle2x2_bwd(const void* dout, int ld_dout, void* dt, int ld_dt, doubl
   int rc = shuf_geom(&g, N, h, w, C, Ho, Wo);
   if (rc) return rc;
   if (g.cgs > 256) return UB2_ERR_SHAPE;
-  if (ld_dout % 8 || ld_dt % 8) return UB2_ERR_ALIGN;
+  if (dout == nullptr || dt == nullptr || (partials != nullptr && dbias == nullptr) || ld_dout < C || ld_dt < 4 * C)
+    return UB2_ERR_SHAPE;
+  if (ld_dout % 8 || ld_dt % 8 || !al16(dout) || !al16(dt) || !aligned_to(partials, 8) || !aligned_to(dbias, 4))
+    return UB2_ERR_ALIGN;
   const int grid = shuf_bwd_grid(g);
   if (partials != nullptr && rows != grid) return UB2_ERR_WORKSPACE;
   const int lanes = 256 / g.cgs;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   launch(shuffle2x2_bwd_kernel<__nv_bfloat16>, grid, lanes * g.cgs, 0, s, static_cast<const __nv_bfloat16*>(dout), ld_dout,
          static_cast<__nv_bfloat16*>(dt), ld_dt, partials, g);
-  if (partials != nullptr && dbias != nullptr)
+  if (partials != nullptr)
     launch(shuffle_bias_finalize_kernel, (C + 7) / 8, dim3(8, 128), 0, s, static_cast<const double*>(partials), grid, C, dbias);
   return static_cast<int>(cudaGetLastError());
 }
 
 int ub2_pack_convt_weight(const float* w, const float* bias, void* fwd, void* dg, float* scale4, float* shift4,
                           int Cin, int Cout, void* stream) {
-  if (Cin <= 0 || Cout <= 0) return UB2_ERR_SHAPE;
+  if (w == nullptr || (scale4 == nullptr) != (shift4 == nullptr) || Cin <= 0 || Cout <= 0) return UB2_ERR_SHAPE;
+  if (!aligned_to(w, 4) || !aligned_to(bias, 4) || !aligned_to(fwd, 2) || !aligned_to(dg, 2) || !aligned_to(scale4, 4) ||
+      !aligned_to(shift4, 4))
+    return UB2_ERR_ALIGN;
   const long long total = static_cast<long long>(Cin) * Cout * 4;
   launch(pack_convt_weight_kernel<__nv_bfloat16>, stream_grid(total, 256, num_sms(), 8), 256, 0, static_cast<cudaStream_t>(stream), w, bias,
          static_cast<__nv_bfloat16*>(fwd), static_cast<__nv_bfloat16*>(dg), scale4, shift4, Cin, Cout);
@@ -233,7 +240,8 @@ int ub2_pack_convt_weight(const float* w, const float* bias, void* fwd, void* dg
 
 int ub2_convt_wgrad_reduce(const float* partial, int splits, int Cin, int Cout, float* grad, int accumulate,
                            void* stream) {
-  if (Cin <= 0 || Cout <= 0 || splits <= 0) return UB2_ERR_SHAPE;
+  if (partial == nullptr || grad == nullptr || Cin <= 0 || Cout <= 0 || splits <= 0) return UB2_ERR_SHAPE;
+  if (!aligned_to(partial, 4) || !aligned_to(grad, 4)) return UB2_ERR_ALIGN;
   const long long total = static_cast<long long>(Cin) * Cout * 4;
   launch(convt_wgrad_reduce_kernel, stream_grid(total, 256, num_sms(), 8), 256, 0, static_cast<cudaStream_t>(stream), partial, splits,
          Cin, Cout, grad, accumulate);
