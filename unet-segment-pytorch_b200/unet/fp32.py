@@ -21,6 +21,7 @@ from __future__ import annotations
 import torch
 
 from . import kernels as K
+from . import syncbn
 
 F32 = torch.float32
 PRECISION = "bf16"
@@ -241,6 +242,7 @@ class ConvBnReluF32(torch.autograd.Function):
         p, pidx = K.f32_maxpool_idx(a) if pool else (None, None)
         ctx.save_for_backward(a0, a1, y, scale, shift, mean, invstd, gamma, weight, pidx)
         ctx.batch = batch
+        ctx.group = syncbn.group_of(bn) if batch else None
         return nchw(a), (nchw(p) if pool else None)
 
     @staticmethod
@@ -249,7 +251,8 @@ class ConvBnReluF32(torch.autograd.Function):
         cout, cin, kh, kw = weight.shape
         dA_n = nhwc_view(dA) if dA is not None else None
         dP_n = _dense(nhwc_view(dP)) if dP is not None else None
-        dy, dgamma, dbeta = K.f32_act_bwd(dA_n, dP_n, pidx, y, scale, shift, mean, invstd, gamma, ctx.batch)
+        dy, dgamma, dbeta = K.f32_act_bwd(dA_n, dP_n, pidx, y, scale, shift, mean, invstd, gamma, ctx.batch,
+                                          exchange=syncbn.exchanger(ctx.group))
         gw = weight_grad(a0, a1, dy, weight.shape) if ctx.needs_input_grad[2] else None
         d0 = d1 = None
         if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
@@ -274,14 +277,15 @@ class ConvInBnReluF32(torch.autograd.Function):
         a = K.f32_affine_act(y, scale, shift, relu=True)
         ctx.save_for_backward(x, y, scale, shift, mean, invstd, gamma,
                               weight if ctx.needs_input_grad[0] else None)
-        ctx.meta = (weight.shape, batch, x_dtype)
+        ctx.meta = (weight.shape, batch, x_dtype, syncbn.group_of(bn) if batch else None)
         return nchw(a)
 
     @staticmethod
     def backward(ctx, dA):
         x, y, scale, shift, mean, invstd, gamma, weight = ctx.saved_tensors
-        wshape, batch, x_dtype = ctx.meta
-        dy, dgamma, dbeta = K.f32_act_bwd(nhwc_view(dA), None, None, y, scale, shift, mean, invstd, gamma, batch)
+        wshape, batch, x_dtype, group = ctx.meta
+        dy, dgamma, dbeta = K.f32_act_bwd(nhwc_view(dA), None, None, y, scale, shift, mean, invstd, gamma, batch,
+                                          exchange=syncbn.exchanger(group))
         dx = K.conv_in_dgrad(dy, weight.contiguous(), wshape[1]).to(x_dtype) if ctx.needs_input_grad[0] else None
         gw = K.f32_conv_in_wgrad(x, dy, wshape) if ctx.needs_input_grad[1] else None
         return dx, gw, dgamma, dbeta, None
@@ -366,21 +370,24 @@ class AttentionGateF32(torch.autograd.Function):
         out, a = K.f32_gate_apply(psi, sp, hp, xn)
         ctx.save_for_backward(gn, xn, u, xp, psi, a, sg, hg, mg, ig, sx, hx, mx, ix, mp, ip, wpsi, gam_g, gam_x, gam_p,
                               w_g, w_x)
-        ctx.meta = (w_psi.shape, batch)
+        ctx.meta = (w_psi.shape, batch) + (ops.gate_groups(bn_g, bn_x, bn_p) if batch else (None, None))
         return nchw(out)
 
     @staticmethod
     def backward(ctx, dout):
         (gn, xn, u, xp, psi, a, sg, hg, mg, ig, sx, hx, mx, ix, mp, ip, wpsi, gam_g, gam_x, gam_p, w_g,
          w_x) = ctx.saved_tensors
-        sh_p, batch = ctx.meta
+        sh_p, batch, group_xg, group_p = ctx.meta
         n, h, w, cx = xn.shape
         _, hin, win, cg = gn.shape
         count = n * h * w
         dx, dpsin, part = K.f32_gate_bwd_a(nhwc_view(dout), xn, a, psi)
         dgam_p, dbet_p, coef_p = K.bn_bwd_finalize(part, count, gam_p, mp, ip, frozen=not batch)
+        if group_p is not None:
+            coef_p = K.synced_coef(part, count, syncbn.exchanger(group_p), gam_p, mp, ip)
         ds, part2 = K.f32_gate_bwd_s(dpsin, psi, coef_p, u, xp, sg, hg, sx, hx, wpsi)
-        grads, coef = K.gate_bwd_finalize(part2, count, gam_x, mx, ix, gam_g, mg, ig, frozen=not batch)
+        grads, coef = K.gate_bwd_finalize(part2, count, gam_x, mx, ix, gam_g, mg, ig, frozen=not batch,
+                                          exchange=syncbn.exchanger(group_xg))
         dxp, du = K.f32_gate_bwd_xg(ds, xp, u, coef)
         dq = K.f32_upsample_bwd(du, hin, win, h, w)
         gw_x = weight_grad(xn, None, dxp, w_x.shape)

@@ -244,11 +244,11 @@ def bn_act(y, scale, shift, relu=True, pool=False, write_act=True, want_idx=Fals
 
 
 def bn_backward(dA, dP, pidx, y, scale, shift, mean, invstd, gamma, relu=True, frozen=False,
-                dgamma=None, dbeta=None):
+                dgamma=None, dbeta=None, exchange=None):
     """BatchNorm(+ReLU, + max-pool routing) backward: returns (dy bf16, dgamma, dbeta).
     ``frozen``: statistics were the running buffers (eval-mode backward), no mean terms.
     ``dgamma`` / ``dbeta``: existing fp32 gradient buffers to accumulate into (then None is
-    returned in their place)."""
+    returned in their place).  ``exchange``: SyncBatchNorm (see ``synced_coef``)."""
     n, h, w, c, ld_y = _nhwc(y)
     ld_da = _nhwc(dA)[4] if dA is not None else 0
     ld_dp = _nhwc(dP)[4] if dP is not None else 0
@@ -258,6 +258,8 @@ def bn_backward(dA, dP, pidx, y, scale, shift, mean, invstd, gamma, relu=True, f
     _C.call("ub2_bn_bwd_reduce", ptr(dA), ld_da, ptr(dP), ld_dp, ptr(pidx), ptr(y), ld_y, ptr(scale),
             ptr(shift), ptr(partials), rows, n, h, w, c, int(relu), stream(), work=(0.0, _nbytes(dA, dP, pidx, y)))
     dgamma, dbeta, coef = bn_bwd_finalize(partials, n * h * w, gamma, mean, invstd, frozen, dgamma, dbeta)
+    if exchange is not None:
+        coef = synced_coef(partials, n * h * w, exchange, gamma, mean, invstd, frozen)
     dy = empty_nhwc(n, h, w, c, dev)
     _C.call("ub2_bn_bwd_apply", ptr(dA), ld_da, ptr(dP), ld_dp, ptr(pidx), ptr(y), ld_y, ptr(scale),
             ptr(shift), ptr(coef), ptr(dy), c, n, h, w, c, int(relu), stream(),
@@ -265,12 +267,16 @@ def bn_backward(dA, dP, pidx, y, scale, shift, mean, invstd, gamma, relu=True, f
     return dy, dgamma, dbeta
 
 
-def bn_bwd_finalize(partials, count, gamma, mean, invstd, frozen=False, dgamma=None, dbeta=None):
+def bn_bwd_finalize(partials, count, gamma, mean, invstd, frozen=False, dgamma=None, dbeta=None, grads=True):
     """(sum g, sum g*y) rows -> (dgamma, dbeta, coef[3,C]) with dy = coef0*g + coef1*y + coef2.
-    The kernel accumulates (+=): into fresh zeros, or into the given ``dgamma`` / ``dbeta``."""
+    The kernel accumulates (+=): into fresh zeros, or into the given ``dgamma`` / ``dbeta``;
+    ``grads=False``: coefficients only (no gradient is written, None is returned for both)."""
     rows, _, c = partials.shape
     direct = dgamma is not None and dbeta is not None
-    if not direct:
+    if not grads:
+        dgamma = dbeta = None
+        direct = True
+    elif not direct:
         grads = torch.zeros((2, c), device=partials.device, dtype=F32)
         dgamma, dbeta = grads[0], grads[1]
     coef = torch.empty((3, c), device=partials.device, dtype=F32)
@@ -279,6 +285,16 @@ def bn_bwd_finalize(partials, count, gamma, mean, invstd, frozen=False, dgamma=N
     if direct:
         return None, None, coef
     return dgamma, dbeta, coef
+
+
+def synced_coef(partials, count, exchange, gamma, mean, invstd, frozen=False):
+    """SyncBatchNorm backward: the apply coefficients of one BatchNorm from the (sum g, sum g*y) rows of every
+    rank.  ``exchange(partials, count)`` returns the rows summed over the ranks and the pixel count over the
+    ranks (unet.syncbn.exchange); it sums ``partials`` in place when the ranks' row counts agree.  The caller has
+    already finalized ``partials`` into dgamma / dbeta: those stay the LOCAL sums, which the trainer's gradient
+    all-reduce then adds up over the ranks (as DDP does with nn.SyncBatchNorm)."""
+    partials, count = exchange(partials, count)
+    return bn_bwd_finalize(partials, count, gamma, mean, invstd, frozen, grads=False)[2]
 
 
 def maxpool_bwd(dP, pidx, a):
@@ -386,9 +402,10 @@ def gate_bwd_s(dpsin, psi, coef_psi, q, xp, sg, hg, sx, hx, wpsi):
 
 
 def gate_bwd_finalize(partials, count, gamma_x, mean_x, invstd_x, gamma_g, mean_g, invstd_g, frozen=False,
-                      targets=None):
+                      targets=None, exchange=None):
     """``targets``: five existing fp32 buffers (dgamma_x, dbeta_x, dgamma_g, dbeta_g, dwpsi) to
-    accumulate into instead of fresh zeros."""
+    accumulate into instead of fresh zeros.  ``exchange``: SyncBatchNorm — the gradients come from this
+    rank's rows, the coefficients from the rows of every rank (see ``synced_coef``)."""
     rows, _, ci = partials.shape
     grads = targets if targets is not None else torch.zeros((5, ci), device=partials.device, dtype=F32)
     coef = torch.empty((6, ci), device=partials.device, dtype=F32)
@@ -396,6 +413,12 @@ def gate_bwd_finalize(partials, count, gamma_x, mean_x, invstd_x, gamma_g, mean_
             ptr(mean_x), ptr(invstd_x), ptr(gamma_g), ptr(mean_g), ptr(invstd_g), int(frozen), ptr(grads[0]),
             ptr(grads[1]),
             ptr(grads[2]), ptr(grads[3]), ptr(grads[4]), ptr(coef), stream())
+    if exchange is not None:
+        partials, count = exchange(partials, count)
+        rows = partials.shape[0]
+        _C.call("ub2_gate_bwd_finalize", ptr(partials), rows, ci, count, ptr(gamma_x),
+                ptr(mean_x), ptr(invstd_x), ptr(gamma_g), ptr(mean_g), ptr(invstd_g), int(frozen), ptr(None),
+                ptr(None), ptr(None), ptr(None), ptr(None), ptr(coef), stream())
     # dgamma_x, dbeta_x, dgamma_g, dbeta_g, dwpsi
     return grads, coef
 
@@ -830,8 +853,9 @@ def f32_affine_act(y, scale, shift, relu=True):
     return out
 
 
-def f32_act_bwd(dA, dP, idx, y, scale, shift, mean, invstd, gamma, batch, relu=True):
-    """BatchNorm (+ReLU, + max-pool routing) backward: (dy, dgamma, dbeta).  dA may be a channel slice; dP, y dense."""
+def f32_act_bwd(dA, dP, idx, y, scale, shift, mean, invstd, gamma, batch, relu=True, exchange=None):
+    """BatchNorm (+ReLU, + max-pool routing) backward: (dy, dgamma, dbeta).  dA may be a channel slice; dP, y dense.
+    ``exchange``: SyncBatchNorm (see ``synced_coef``)."""
     n, h, w, c, _ = _nhwc32(y, dense=True)
     ld_da = _nhwc32(dA)[4] if dA is not None else 0
     if dP is not None:
@@ -841,6 +865,8 @@ def f32_act_bwd(dA, dP, idx, y, scale, shift, mean, invstd, gamma, batch, relu=T
     _C.call("ub2_f32_act_bwd_reduce", ptr(dA), ld_da, ptr(dP), ptr(idx), ptr(y), ptr(scale), ptr(shift), ptr(part),
             rows, n, h, w, c, int(relu), stream(), work=(0.0, _nbytes(dA, dP, idx, y)))
     dgamma, dbeta, coef = bn_bwd_finalize(part, n * h * w, gamma, mean, invstd, frozen=not batch)
+    if exchange is not None:
+        coef = synced_coef(part, n * h * w, exchange, gamma, mean, invstd, frozen=not batch)
     dy = torch.empty_like(y)
     _C.call("ub2_f32_act_bwd_apply", ptr(dA), ld_da, ptr(dP), ptr(idx), ptr(y), ptr(scale), ptr(shift), ptr(coef),
             ptr(dy), n, h, w, c, int(relu), stream(), work=(0.0, _nbytes(dA, dP, idx, y, dy)))

@@ -18,7 +18,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from .. import fp32, ops
+from .. import fp32, ops, syncbn
 
 
 def _stage(x0, x1, conv: nn.Conv2d, bn: nn.BatchNorm2d, pool: bool = False):
@@ -128,10 +128,13 @@ class OutConv(nn.Module):
 class _BnView:
     """What unet.ops / unet.fp32 read from a BatchNorm2d, with the channel vectors padded by `pad` neutral
     channels (gamma 1, beta 0, running statistics 0 / 1); ``write_back`` returns the real channels' running
-    statistics to the module (``num_batches_tracked`` is shared and advanced in place)."""
+    statistics to the module (``num_batches_tracked`` is shared and advanced in place).  An nn.SyncBatchNorm's
+    decision to synchronise travels with the view (``sync_group``, read by unet.syncbn): the neutral channels sum to
+    zero on every rank and change nothing."""
 
     def __init__(self, bn: nn.BatchNorm2d, pad: int):
         self._bn, self._c = bn, bn.num_features
+        self.sync_group = syncbn.group_of(bn)
         self.training, self.momentum, self.eps = bn.training, bn.momentum, bn.eps
         self.track_running_stats = bn.track_running_stats
         self.weight = F.pad(bn.weight, (0, pad), value=1.0)

@@ -11,6 +11,7 @@ from __future__ import annotations
 import torch
 
 from . import kernels as K
+from . import syncbn
 
 BF16 = torch.bfloat16
 
@@ -125,9 +126,13 @@ def from_nhwc(t: torch.Tensor) -> torch.Tensor:
 
 def _bn_train_coeffs(partials, count, bn):
     """Batch statistics -> (scale, shift, mean, invstd); running buffers updated like
-    nn.BatchNorm2d in train mode (layers.py:33)."""
+    nn.BatchNorm2d in train mode (layers.py:33).  An nn.SyncBatchNorm that synchronises sums
+    the statistics and pixel counts of every rank of its group first (unet.syncbn)."""
     if bn.momentum is None:
         raise NotImplementedError("BatchNorm momentum=None (cumulative average) is not supported")
+    group = syncbn.group_of(bn)
+    if group is not None:
+        partials, count = syncbn.exchange(partials, count, group)
     track = bn.track_running_stats and bn.running_mean is not None
     return K.bn_finalize(partials, count, bn.weight, bn.bias,
                          bn.running_mean if track else None, bn.running_var if track else None,
@@ -178,14 +183,14 @@ class ConvBnRelu(torch.autograd.Function):
         else:
             a, p = K.bn_act(y, scale, shift, relu=True, pool=False)
         ctx.save_for_backward(a0, a1, y, scale, shift, mean, invstd, gamma, wd, pidx)
-        ctx.meta = (weight.shape, batch)
+        ctx.meta = (weight.shape, batch, syncbn.group_of(bn) if batch else None)
         ctx.params = (weight, gamma, beta)
         return from_nhwc(a), (from_nhwc(p) if pool else None)
 
     @staticmethod
     def backward(ctx, dA, dP):
         a0, a1, y, scale, shift, mean, invstd, gamma, wd, pidx = ctx.saved_tensors
-        wshape, batch = ctx.meta
+        wshape, batch, group = ctx.meta
         cout, cin, kh, kw = wshape
         taps = kh * kw
         dA_n = to_nhwc(dA) if dA is not None else None
@@ -193,7 +198,7 @@ class ConvBnRelu(torch.autograd.Function):
         p_w, p_gamma, p_beta = ctx.params
         bn_t = _grad_targets(p_gamma, p_beta) if ctx.needs_input_grad[3] and ctx.needs_input_grad[4] else None
         dy, dgamma, dbeta = _bn_backward(dA_n, dP_n, pidx, y, scale, shift, mean, invstd, gamma, batch,
-                                         targets=bn_t)
+                                         targets=bn_t, group=group)
         if bn_t is not None:
             _grads_done(p_gamma, p_beta)
         # data gradient first: it is what the next layer's backward waits for
@@ -221,10 +226,10 @@ class ConvBnRelu(torch.autograd.Function):
         return d0, d1, gw, dgamma, dbeta, None, None
 
 
-def _bn_backward(dA, dP, pidx, y, scale, shift, mean, invstd, gamma, batch, relu=True, targets=None):
+def _bn_backward(dA, dP, pidx, y, scale, shift, mean, invstd, gamma, batch, relu=True, targets=None, group=None):
     dg, db = targets if targets is not None else (None, None)
     return K.bn_backward(dA, dP, pidx, y, scale, shift, mean, invstd, gamma, relu=relu, frozen=not batch,
-                         dgamma=dg, dbeta=db)
+                         dgamma=dg, dbeta=db, exchange=syncbn.exchanger(group))
 
 
 class ConvInBnRelu(torch.autograd.Function):
@@ -247,18 +252,18 @@ class ConvInBnRelu(torch.autograd.Function):
         if any(ctx.needs_input_grad):
             ctx.save_for_backward(x, y, scale, shift, mean, invstd, gamma,
                                   weight if ctx.needs_input_grad[0] else None)
-            ctx.meta = (weight.shape, batch, x_dtype)
+            ctx.meta = (weight.shape, batch, x_dtype, syncbn.group_of(bn) if batch else None)
             ctx.params = (weight, gamma, beta)
         return from_nhwc(a)
 
     @staticmethod
     def backward(ctx, dA):
         x, y, scale, shift, mean, invstd, gamma, weight = ctx.saved_tensors
-        wshape, batch, x_dtype = ctx.meta
+        wshape, batch, x_dtype, group = ctx.meta
         p_w, p_gamma, p_beta = ctx.params
         bn_t = _grad_targets(p_gamma, p_beta) if ctx.needs_input_grad[2] and ctx.needs_input_grad[3] else None
         dy, dgamma, dbeta = _bn_backward(to_nhwc(dA), None, None, y, scale, shift, mean, invstd, gamma, batch,
-                                         targets=bn_t)
+                                         targets=bn_t, group=group)
         if bn_t is not None:
             _grads_done(p_gamma, p_beta)
         dx = K.conv_in_dgrad(dy, weight.contiguous(), wshape[1]).to(x_dtype) if ctx.needs_input_grad[0] else None
@@ -312,6 +317,16 @@ def resize_logits(x, size):
     return ResizeLogits.apply(x.float(), int(size[0]), int(size[1]))
 
 
+def gate_groups(bn_g, bn_x, bn_p):
+    """The groups the gate's BatchNorms synchronise over: (W_g and W_x together, psi).  The backward folds the
+    statistics of W_g and W_x in one table, so the two must agree."""
+    group_g, group_x = syncbn.group_of(bn_g), syncbn.group_of(bn_x)
+    if group_g is not group_x:
+        raise NotImplementedError("AttentionGate: W_g and W_x BatchNorms must both synchronise over the same "
+                                  "process group or both not (convert them together with convert_sync_batchnorm)")
+    return group_x, syncbn.group_of(bn_p)
+
+
 class AttentionGateFn(torch.autograd.Function):
     """AttentionGate.forward (layers.py:171-192) as two tensor-core 1x1 projections plus three
     bandwidth-bound passes; see csrc/gate.cu."""
@@ -348,7 +363,7 @@ class AttentionGateFn(torch.autograd.Function):
         if need_grad:
             ctx.save_for_backward(gn, xn, q, xp, psi, a, sg, hg, mg, ig, sx, hx, mx, ix, mp, ip, wgd, wxd,
                                   wpsi, gam_g, gam_x, gam_p)
-            ctx.meta = (w_g.shape, w_x.shape, w_psi.shape, batch)
+            ctx.meta = (w_g.shape, w_x.shape, w_psi.shape, batch) + (gate_groups(bn_g, bn_x, bn_p) if batch else (None, None))
             ctx.params = (w_g, w_x, w_psi, gam_g, bet_g, gam_x, bet_x, gam_p, bet_p)
         return from_nhwc(out)
 
@@ -356,7 +371,7 @@ class AttentionGateFn(torch.autograd.Function):
     def backward(ctx, dout):
         (gn, xn, q, xp, psi, a, sg, hg, mg, ig, sx, hx, mx, ix, mp, ip, wgd, wxd, wpsi, gam_g, gam_x,
          gam_p) = ctx.saved_tensors
-        sh_g, sh_x, sh_p, batch = ctx.meta
+        sh_g, sh_x, sh_p, batch, group_xg, group_p = ctx.meta
         n, h, w, cx = xn.shape
         _, hin, win, cg = gn.shape
         ci = q.shape[3]
@@ -370,9 +385,12 @@ class AttentionGateFn(torch.autograd.Function):
             _, _, coef_p = K.bn_bwd_finalize(part, count, gam_p, mp, ip, frozen=not batch, dgamma=t_gp, dbeta=t_bp)
         else:
             dgam_p, dbet_p, coef_p = K.bn_bwd_finalize(part, count, gam_p, mp, ip, frozen=not batch)
+        if group_p is not None:
+            coef_p = K.synced_coef(part, count, syncbn.exchanger(group_p), gam_p, mp, ip)
         ds, part2 = K.gate_bwd_s(dpsin, psi, coef_p, q, xp, sg, hg, sx, hx, wpsi)
         grads, coef = K.gate_bwd_finalize(part2, count, gam_x, mx, ix, gam_g, mg, ig, frozen=not batch,
-                                          targets=[t_gx, t_bx, t_gg, t_bg, t_wpsi] if direct is not None else None)
+                                          targets=[t_gx, t_bx, t_gg, t_bg, t_wpsi] if direct is not None else None,
+                                          exchange=syncbn.exchanger(group_xg))
         dxp, dgup = K.gate_bwd_xg(ds, xp, q, coef)
         dq = K.upsample_bwd(dgup, hin, win, h, w)
         if direct is not None:

@@ -8,7 +8,8 @@ clip + optimizer step follows (train.py:139-143).  Here the micro-batches run at
 one per GPU (one process per GPU): rank r computes forward/backward on its shard with the loss
 divided by ``world_size``, gradients are summed with NCCL all-reduce over NVLink, and every
 rank then applies the identical clip + optimizer step.  Up to summation order this is the same
-arithmetic (no SyncBN: statistics stay per micro-batch, exactly as in the reference).
+arithmetic (statistics stay per micro-batch, exactly as in the reference, unless the model's
+BatchNorms were converted with ``nn.SyncBatchNorm.convert_sync_batchnorm``: see unet/syncbn.py).
 
 Gradients live in a few flat fp32 buckets cut in backward order; a bucket's all-reduce is
 launched from an autograd hook as soon as its last gradient has been accumulated, on NCCL's
